@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- window-graphs/s, forward+backward, of the detector's message-passing path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -52,6 +52,7 @@ GOLDEN = REPO / "tests" / "golden"
 METRIC = "window_graphs_per_sec_fwd_bwd"
 UNIT = "window-graphs/s"
 SENSORS = 29
+DUMP_LIMIT = 64_000_000   # bytes that --dump-outputs writes at most
 
 WORKLOADS = {
     "lta4096": dict(net="LTA", batch=4096, l_det=288, pipes=764, hidden=64, full_step=False, cpu_sample=32,
@@ -138,6 +139,26 @@ def network(net: str, n_pipes: int):
     return dict(inp=inp, sensors=sensors, pipe_ids=classes, n_nodes=len(names), n_edges=2 * len(links),
                 nnz=2 * len(links) + len(names), edge_index=ei, pipe_ends=lk[[pidx[p] for p in classes]],
                 sensor_idx=np.asarray([int(s[1:]) for s in sensors], dtype=np.int64))
+
+
+def dump_outputs(out_dir, arrays: dict, limit: int = DUMP_LIMIT) -> None:
+    """Write every array as out_dir/<name>.npy in float32.  If they add up to more than `limit` bytes, each array above
+    1/64 of the limit keeps the same share of its first-axis rows, drawn by a fixed seed and kept in order.  The sample
+    depends on the shapes alone: arrays with as many rows keep the same rows, and two builds keep the same sample."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        big = [k for k, a in arrays.items() if a.ndim > 0 and a.shape[0] > 1 and a.nbytes > limit // 64]
+        rest = total - sum(arrays[k].nbytes for k in big)
+        share = (limit - rest) / (total - rest)
+        for k in big:
+            n = arrays[k].shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(n, int(n * share), replace=False))
+            arrays[k] = arrays[k][rows]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", a)
 
 
 class ClockSampler:
@@ -425,11 +446,14 @@ def run_ours(args, wl: dict) -> None:
     bucket = FlatGradBucket(params)
     unit_bytes = net["n_nodes"] * hidden * 4 * args.batch
     flush = torch.empty(64 * 1024 * 1024, device=dev) if unit_bytes * 8 < 400e6 else None  # 256 MB > L2
+    last = {}   # the logits and loss of the latest step (graph replays: their static tensors), for --dump-outputs
 
     def detector_step(residual, tfeat):
         """reference train_detector.py:310-317 from the detector call on"""
         bucket.zero()
-        loss = torch.nn.functional.cross_entropy(model(residual, tfeat), label)
+        logits = model(residual, tfeat)
+        loss = torch.nn.functional.cross_entropy(logits, label)
+        last.update(logits=logits.detach(), loss=loss.detach())
         loss.backward()
         bucket.allreduce()
         if full_step:
@@ -453,8 +477,13 @@ def run_ours(args, wl: dict) -> None:
         # CUDA-graph replay of the whole step (leak_det_gnn_b200/graphed.py); --eager times the call-by-call form
         from leak_det_gnn_b200.graphed import GraphedStep, GraphedTrainStep
 
+        def recorded_ce(logits, target):
+            last["logits"] = logits.detach()
+            return torch.nn.functional.cross_entropy(logits, target)
+
         g_e2e = GraphedTrainStep(model, opt, bucket, args.batch, args.l_det, predictor=predictor,
-                                 l_pred=l_pred if full_step else 0, grad_clip=1.0 if full_step else 0.0)
+                                 l_pred=l_pred if full_step else 0, grad_clip=1.0 if full_step else 0.0,
+                                 loss_fn=recorded_ce)
         g_e2e.label.copy_(label)
     if full_step:
         def eager_value_step():
@@ -471,7 +500,9 @@ def run_ours(args, wl: dict) -> None:
                 flush.fill_(0.0)
             bucket.zero()
             h_s.grad = None
-            loss = torch.nn.functional.cross_entropy(model.gnn_stack(h_s), label)
+            logits = model.gnn_stack(h_s)
+            loss = torch.nn.functional.cross_entropy(logits, label)
+            last.update(logits=logits.detach(), loss=loss.detach(), h_s=h_s)
             loss.backward()
             bucket.allreduce()
 
@@ -483,7 +514,10 @@ def run_ours(args, wl: dict) -> None:
         else:
             def stack_fwd_bwd():
                 bucket.zero()
-                loss = torch.nn.functional.cross_entropy(model.gnn_stack(h_s.detach().requires_grad_(True)), label)
+                leaf = h_s.detach().requires_grad_(True)
+                logits = model.gnn_stack(leaf)
+                loss = torch.nn.functional.cross_entropy(logits, label)
+                last.update(logits=logits.detach(), h_s=leaf)   # captured: every replay rewrites them and leaf.grad
                 loss.backward()
                 return loss
             g_value = GraphedStep(model, stack_fwd_bwd, None, bucket)
@@ -565,6 +599,19 @@ def run_ours(args, wl: dict) -> None:
     else:
         ms_stack, launches, ksum = timed(value_step, args.steps, args.warmup)
         clocks = None
+    if rank == 0 and args.dump_outputs:
+        # what the last timed step of `value` handed its caller, before the passes below overwrite it: the logits and
+        # loss, the gradient of every parameter and (GNN stack) of the sensor embeddings, the parameters after the update
+        if graphed:
+            last["loss"] = g_value.loss
+        outs = {"logits": last["logits"], "loss": last["loss"]}
+        if not full_step:
+            outs["grad_h_s"] = last["h_s"].grad
+        for name, p in model.named_parameters():
+            outs[f"grad.{name}"] = p.grad
+            if full_step:
+                outs[f"param.{name}"] = p
+        dump_outputs(args.dump_outputs, {k: v.detach().cpu().numpy() for k, v in outs.items()})
     ms_kernel_pass = ms_stack
     if graphed:   # kernels inside a graph replay cannot be bracketed by events: per-kernel durations from an eager pass
         ms_kernel_pass, _, ksum = timed(eager_value_step, args.steps, args.warmup, timing_kernels=(rank == 0))
@@ -766,7 +813,15 @@ def main() -> None:
     ap.add_argument("--cpu-sample", type=int, default=None, help="windows per CPU-arm step (bounded sample)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--eager", action="store_true", help="time the call-by-call step where the workload defaults to graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step of `value` computed as DIR/<name>.npy (float32, "
+                         "at most 64 MB: larger outputs as a fixed sample of their rows); the inputs depend on the "
+                         "arguments alone, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     wl = WORKLOADS[args.workload]
     args.batch = wl["batch"] if args.batch is None else args.batch
     args.l_det = wl["l_det"] if args.l_det is None else args.l_det

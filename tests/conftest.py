@@ -11,10 +11,6 @@ if str(REPO) not in sys.path:
     sys.path.insert(0, str(REPO))
 
 TOPO = {"LTA": GOLDEN / "L-TOWN-A.topo.inp", "LT": GOLDEN / "L-TOWN.topo.inp"}
-REFERENCE_INP = {
-    "LTA": Path("/root/reference/data/raw/L-TOWN-A/L-TOWN_AreaA.inp"),
-    "LT": Path("/root/reference/data/raw/L-TOWN/L-TOWN.inp"),
-}
 
 
 # fp32 parity: cuDNN's RNN may otherwise run TF32 tensor-core math (torch default allow_tf32=True for

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import REFERENCE_INP, TOPO
+from conftest import TOPO
 from leak_det_gnn_b200.graph import batchify_edge_index, build_gcn_csr, build_wdn_graph_from_inp, parse_epanet_inp
 from oracle import pyg_restatement as pyg
 
@@ -44,16 +44,6 @@ def test_survey_known_answers(graph_golden):
     deg = np.bincount(g.edge_index[1].numpy(), minlength=661)
     assert np.bincount(deg).tolist() == [0, 24, 427, 187, 22, 1]
     assert (g.edge_index[0] != g.edge_index[1]).all()
-
-
-@pytest.mark.parametrize("net", ["LTA", "LT"])
-def test_original_inp_when_reference_present(graph_golden, net):
-    if not REFERENCE_INP[net].exists():
-        pytest.skip("/root/reference not present on this machine")
-    g0 = graph_golden(net)
-    g = build_wdn_graph_from_inp(REFERENCE_INP[net], [str(s) for s in g0["sensor_node_ids"]],
-                                 [str(s) for s in g0["pipe_ids"]], add_self_loops=False, make_undirected=True)
-    assert np.array_equal(g.edge_index.numpy(), g0["edge_index"]) and np.array_equal(g.pipe_ends, g0["pipe_ends"])
 
 
 def test_builder_options_and_errors(tmp_path):

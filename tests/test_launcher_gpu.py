@@ -60,7 +60,7 @@ dist.destroy_process_group()
 """
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_two_rank_gradients_equal_single_gpu_on_concatenated_batch(tmp_path, graph_golden):
     from leak_det_gnn_b200.models import LeakDetector
 
