@@ -689,11 +689,13 @@ pipe_head_bwd_dx_kernel(const DpreLoader loader, float4* __restrict__ dx, const 
 }  // namespace hb
 
 // ------------------------------------------------------------------ mean pool and its adjoint
-// out[u, :] = scale * sum of rows [r_lo, r_hi) of window b, u = b * units_per_b + block (one unit per window and
-// scale = 1 / N for the L-TOWN sizes; large graphs are split into row blocks and a second call sums the partials)
+// out[u, :] = (sum of rows [r_lo, r_hi) of window b) / div, u = b * units_per_b + block (one unit per window and
+// div = N for the L-TOWN sizes; large graphs are split into row blocks and a second call sums the partials).  A divide,
+// not a multiply by 1 / N: the rounded reciprocal is off by up to 6e-8 in one direction for every output (-3.6e-8 at
+// N = 661), a bias that tests/test_bench_sizes_gpu.py::test_mean_pool_at_bench_rows sees on same-sign inputs
 __global__ void __launch_bounds__(256)
 mean_pool_kernel(const float4* __restrict__ x, float4* __restrict__ pooled, int64_t B, int N, int d4, int units_per_b,
-                 int rows_per_unit, float inv) {
+                 int rows_per_unit, float div) {
     __shared__ float4 red[256];
     const int tid = threadIdx.x;
     const int c = tid % d4, r0 = tid / d4, rstep = 256 / d4;
@@ -715,7 +717,7 @@ mean_pool_kernel(const float4* __restrict__ x, float4* __restrict__ pooled, int6
                 const float4 o = red[k];
                 t.x += o.x; t.y += o.y; t.z += o.z; t.w += o.w;
             }
-            pooled[u * d4 + tid] = make_float4(t.x * inv, t.y * inv, t.z * inv, t.w * inv);
+            pooled[u * d4 + tid] = make_float4(t.x / div, t.y / div, t.z / div, t.w / div);
         }
         __syncthreads();
     }
@@ -840,13 +842,13 @@ extern "C" int ltgnn_mean_pool_fwd(int device, int64_t B, int32_t N, int32_t D, 
     LTGNN_USE_DEVICE(device);
     const int64_t cap = static_cast<int64_t>(di->sm_count) * 8;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    const float inv = 1.f / static_cast<float>(N);
+    const float n_f = static_cast<float>(N);
     int units_per_b = static_cast<int>((cap + B - 1) / B);
     const int max_units = (N + 2047) / 2048;  // at least 2048 rows per unit
     if (units_per_b > max_units) units_per_b = max_units;
     if (units_per_b <= 1) {
         mean_pool_kernel<<<static_cast<int>(B < cap ? B : cap), 256, 0, stream>>>(
-            reinterpret_cast<const float4*>(X), reinterpret_cast<float4*>(pooled), B, N, D / 4, 1, N, inv);
+            reinterpret_cast<const float4*>(X), reinterpret_cast<float4*>(pooled), B, N, D / 4, 1, N, n_f);
         LTGNN_CUDA_TRY(cudaGetLastError());
         return LTGNN_OK;
     }
@@ -859,7 +861,7 @@ extern "C" int ltgnn_mean_pool_fwd(int device, int64_t B, int32_t N, int32_t D, 
     mean_pool_kernel<<<static_cast<int>(n_units < cap ? n_units : cap), 256, 0, stream>>>(
         reinterpret_cast<const float4*>(X), part, B, N, D / 4, units_per_b, rows_per_unit, 1.f);
     mean_pool_kernel<<<static_cast<int>(B < cap ? B : cap), 256, 0, stream>>>(part, reinterpret_cast<float4*>(pooled), B,
-                                                                              units_per_b, D / 4, 1, units_per_b, inv);
+                                                                              units_per_b, D / 4, 1, units_per_b, n_f);
     cudaError_t e = cudaGetLastError();
     cudaFreeAsync(part, stream);
     LTGNN_CUDA_TRY(e);

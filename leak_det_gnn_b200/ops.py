@@ -747,6 +747,7 @@ class _GnnBody(torch.autograd.Function):
         ctx.lives = lives
         if DEBUG_CAPTURE is not None:
             DEBUG_CAPTURE["lives"] = lives
+            DEBUG_CAPTURE["xs"] = xs   # the gates of the layers without a live mask (None in `lives`)
         ctx.save_for_backward(h_s, slot, w0, *conv_params[0::2], *xs)
         # the kernels draw 16 random bits per element: keep probability 1 - round(p * 2^16) / 2^16
         ctx.graph, ctx.n_layers, ctx.scale = graph, n_layers, 1.0 / (1.0 - int(p * 65536.0 + 0.5) / 65536.0)

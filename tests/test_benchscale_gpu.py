@@ -35,10 +35,11 @@ def _head_ref(x, ends, w1, b1, w2, b2, live):
     return torch.nn.functional.linear(hid, w2, b2).squeeze(-1), x.mean(dim=1)
 
 
-@pytest.mark.parametrize("bsz,n,p", [(64, 661, 764), (256, 661, 764), (130, 785, 905)])
+@pytest.mark.parametrize("bsz,n,p", [(64, 661, 764), (256, 661, 764), (130, 785, 905), (4096, 661, 764)])
 def test_heads_many_tiles_per_cta(bsz, n, p):
-    """382 / 1528 / 920 row tiles of 128 pipe rows: 3 / 11 / 7 tiles per CTA through pipe_head_fwd, pipe_head_bwd_dx
-    and the tgrad<HeadDpre> weight gradient (reference detector.py:76-88,204-211)."""
+    """382 / 1528 / 920 / 24 448 row tiles of 128 pipe rows: 3 / 11 / 7 / 166 tiles per CTA through pipe_head_fwd,
+    pipe_head_bwd_dx and the tgrad<HeadDpre> weight gradient (reference detector.py:76-88,204-211); the last is the
+    lta4096 benchmark size, 3.1 M rows in dW1 / db1 / dw2.  The fp64 truth runs on the GPU."""
     assert (bsz * p + 127) // 128 > 2 * SM
     gen = torch.Generator().manual_seed(bsz + p)
     x = torch.randn(bsz, n, 64, generator=gen).relu()
@@ -66,9 +67,9 @@ def test_heads_many_tiles_per_cta(bsz, n, p):
     bits = (words.unsqueeze(-1) >> (31 - torch.arange(32, device=words.device))) & 1
     assert torch.equal(bits.reshape(bsz * p, 128).bool(), cap["head_live"])
 
-    t = [v.double().requires_grad_(True) for v in (x, w1, b1, w2, b2)]
-    lr, pr = _head_ref(t[0], ends, *t[1:], cap["head_live"].cpu().double().view(bsz, p, 128))
-    ((lr * dlog.double()).sum() + (pr * dpool.double()).sum()).backward()
+    t = [v.double().cuda().requires_grad_(True) for v in (x, w1, b1, w2, b2)]
+    lr, pr = _head_ref(t[0], ends.cuda(), *t[1:], cap["head_live"].double().view(bsz, p, 128))
+    ((lr * dlog.double().cuda()).sum() + (pr * dpool.double().cuda()).sum()).backward()
     rep = {"logits": rel_err(logits, lr), "pooled": rel_err(pooled, pr), "dx": rel_err(o[0].grad, t[0].grad),
            "dw1": rel_err(o[1].grad, t[1].grad), "db1": rel_err(o[2].grad, t[2].grad),
            "dw2": rel_err(o[3].grad, t[3].grad), "db2": rel_err(b2c.grad, t[4].grad)}
@@ -186,17 +187,17 @@ def _replay(orc, h_s, masks, head_live, noleak_keep, scale, n_nodes):
     kernels (eval mode: scale = 1 and live is the plain ReLU mask).  Replaying the mask removes the one effect that is
     not an arithmetic error: a pre-activation within fp32 rounding of zero lands on the other side in fp64, and with
     1e7-1e8 units per step a handful do, each moving a gradient row by O(1e-3) relative."""
-    dt = h_s.dtype
+    dt, dev = h_s.dtype, h_s.device
     b = h_s.shape[0]
     n = n_nodes
-    h0 = torch.zeros(b, n, h_s.shape[-1], dtype=dt)
+    h0 = torch.zeros(b, n, h_s.shape[-1], dtype=dt, device=dev)
     h0 = h0.index_copy(1, orc.sensor_node_idx, h_s)
-    mask = torch.zeros(n, 1, dtype=dt)
+    mask = torch.zeros(n, 1, dtype=dt, device=dev)
     mask[orc.sensor_node_idx, 0] = 1.0
     x = orc.sensor_to_node(torch.cat([h0, mask.unsqueeze(0).expand(b, -1, -1)], dim=-1)) * masks[0].to(dt) * scale
     x = x.reshape(b * n, -1)
     e = orc.edge_index_single.size(1)
-    edge_index = orc.edge_index_single.repeat(1, b) + (torch.arange(b).repeat_interleave(e) * n).unsqueeze(0)
+    edge_index = orc.edge_index_single.repeat(1, b) + (torch.arange(b, device=dev).repeat_interleave(e) * n).unsqueeze(0)
     for li, conv in enumerate(orc.convs):
         x = conv(x, edge_index) * masks[li + 1].to(dt).reshape(b * n, -1) * scale
     hn = x.view(b, n, -1)
@@ -204,7 +205,7 @@ def _replay(orc, h_s, masks, head_live, noleak_keep, scale, n_nodes):
     feat = torch.cat([h_u, h_v, (h_u - h_v).abs()], dim=-1)
     mlp = orc.edge_head.mlp
     pipe_logits = mlp[3](mlp[0](feat) * head_live.to(dt).view(b, -1, head_live.shape[-1]) * scale).squeeze(-1)
-    pooled = pyg.global_mean_pool(x, torch.arange(b).repeat_interleave(n))
+    pooled = pyg.global_mean_pool(x, torch.arange(b, device=dev).repeat_interleave(n))
     mlp = orc.noleak_head.mlp
     noleak = mlp[3](torch.relu(mlp[0](pooled)) * noleak_keep.to(dt))  # (B, 1); noleak_keep already carries 1 / (1 - p)
     return torch.cat([pipe_logits, noleak], dim=-1)
