@@ -247,11 +247,41 @@ int64_t ltgnn_pipe_head_ws_floats(int device);
  * torch's conv weight permuted (2, 0, 1)), bias / gamma / beta [C] (gamma = beta = null: no LayerNorm), res [r_rows, C]
  * with res_row int32 [M] or both null, Y [M, C].  C = 128.  tcgen05, 3xTF32; the weight is split into TF32 hi / lo and laid
  * out as shared-memory operand stages once per call (into ws: ltgnn_tcn_ws_floats(taps) floats) and streamed by bulk copies.
+ * res_row[m] = -1 adds nothing to row m (the input gradient below uses it for block-input rows no output row keeps).
  */
 int64_t ltgnn_tcn_ws_floats(int32_t taps);
 int ltgnn_tcn_conv(int device, int64_t M, int32_t C, int32_t taps, const float* X, const int32_t* src, const float* W,
                    const float* bias, const float* gamma, const float* beta, float eps, int relu, const float* res,
                    const int32_t* res_row, float* Y, float* ws, void* stream);
+
+/* ---- training of the TCN predictor on the same cone (reference train_predictor.py; csrc/tcn_train.cu) ---------
+ * The loss reads only the last time step (predictor.py:80), so every parameter gradient depends only on the cone rows.
+ * tcn_conv_train: the forward of one training convolution of a TCN block,
+ *     Y[m, :] = [res[res_row[m], :] +] dropout(relu(LayerNorm(Z[m, :]))),  Z = bias + sum_tap X[src[tap * M + m], :] W[tap]^T
+ *   with everything as in ltgnn_tcn_conv (gamma, beta required).  Also writes Z [M, C] (pre-norm rows), stats [M, 2]
+ *   (mean, rstd per row) and live uint32 [M, 4]: bit b of word w = (output channel 32 w + b is > 0 after ReLU and
+ *   dropout).  Dropout is inverted dropout from Philox keyed by drop_seed (+ the ltgnn_seed_source word); drop_p = 0
+ *   gives Y bit-identical to ltgnn_tcn_conv with relu = 1.  ws: ltgnn_tcn_ws_floats(taps) floats.
+ * tcn_ln_bwd: dZ = the LayerNorm backward of g = dY * live * scale (scale = 1 / (1 - drop_p)) from Z, stats and gamma;
+ *   dprm [3, C] = column sums over the M rows of g * x_hat (d gamma), g (d beta) and dZ (d bias).  Fixed-order partials:
+ *   deterministic.  ws: ltgnn_tcn_ln_bwd_ws_floats(device) floats.
+ * Input gradient of a training convolution: ltgnn_tcn_conv with X = dZ, src = inv, W[tap] = W[tap]^T, a zero bias, no
+ *   LayerNorm, relu = 0, where inv int32 [taps, x_rows] is the inverse index: inv[tap * x_rows + r] = the m with
+ *   src[tap * M + m] = r, or -1 if there is none (it must be unique: a tap's row map is injective).  A block input also
+ *   receives the block output's gradient on the rows it keeps: res = dY of the block, res_row = the kept-row inverse.
+ * tcn_wgrad: dW [taps, C, C], dW[tap] = dZ^T X[src[tap]] (row -1 of X = zeros), summed over the M rows on the tensor cores
+ *   (3xTF32, fp32 per-chunk flush; X rows gathered while loaded).  ws: ltgnn_tgrad_ws_floats(device, C) floats.
+ *   Deterministic.  C = 128 for all three.
+ */
+int ltgnn_tcn_conv_train(int device, int64_t M, int32_t C, int32_t taps, const float* X, const int32_t* src, const float* W,
+                         const float* bias, const float* gamma, const float* beta, float eps, const float* res,
+                         const int32_t* res_row, float drop_p, uint64_t drop_seed, float* Y, float* Z, float* stats,
+                         uint32_t* live, float* ws, void* stream);
+int64_t ltgnn_tcn_ln_bwd_ws_floats(int device);
+int ltgnn_tcn_ln_bwd(int device, int64_t M, int32_t C, const float* dY, const uint32_t* live, const float* Z,
+                     const float* stats, const float* gamma, float scale, float* dZ, float* dprm, float* ws, void* stream);
+int ltgnn_tcn_wgrad(int device, int64_t M, int32_t C, int32_t taps, const float* dZ, const float* X, const int32_t* src,
+                    float* dW, float* ws, void* stream);
 
 /* ---- shared per-sensor GRU encoder (detector.py:28-73; SURVEY 8f rank 2) -----------------------
  * Sequence q = b*S + s has input [r[b,t,s], tf[b,t,0..F)] at step t (the reference's cat([rr, tf]) order);

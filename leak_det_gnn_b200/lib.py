@@ -61,6 +61,14 @@ SIGNATURES = {
     "ltgnn_tcn_ws_floats": (c_int64, [c_int32]),
     "ltgnn_tcn_conv": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                c_float, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_tcn_conv_train": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_float, c_void_p, c_void_p, c_float, c_uint64, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p]),
+    "ltgnn_tcn_ln_bwd_ws_floats": (c_int64, [c_int]),
+    "ltgnn_tcn_ln_bwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
+                                 c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_tcn_wgrad": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                c_void_p]),
     "ltgnn_pipe_feat_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_head_out_fwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_float, c_uint64, c_void_p, c_void_p]),
     "ltgnn_head_out_ws_floats": (c_int64, [c_int, c_int32]),

@@ -8,7 +8,8 @@ rank 1).  It contains no graph layers (SURVEY F1).  ``state_dict`` keys equal th
 
 ``forward`` is the reference's dense evaluation (every time step of every layer); ``forward_last`` evaluates only the
 dependency cone of the last time step -- the only one the model reads (predictor.py:80): 99 instead of 288
-convolution evaluations per window -- and is what the residual builder (models/utils.py) calls.
+convolution evaluations per window -- and is what the residual builder (models/utils.py) calls.  ``forward_cone`` is
+the same cone, differentiable: what ``train_predictor_dp`` trains with.
 """
 from __future__ import annotations
 
@@ -84,6 +85,33 @@ class NormalPredictorTCN(nn.Module):
             raise RuntimeError("forward_last is the inference path of the frozen predictor (call .eval() first)")
         if self._native_ok(x):
             return self._forward_last_native(x, x_time)
+        return self._cone_torch(x, x_time)
+
+    def forward_cone(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
+        """``forward``'s result, differentiable in train and eval mode, from the dependency cone of the last time step.
+        The loss reads only that step, so the parameter gradients are the dense model's (positions outside the cone get
+        zero gradient there too), with 34 % of the convolution work at L = 36.  Dropout is the module's (train mode).
+        On CUDA at the shapes ``_native_ok`` accepts this is ONE autograd node on the sm_100a kernels
+        (``ops.tcn_cone``); otherwise the same cone through torch ops."""
+        if not self._native_ok(x):
+            return self._cone_torch(x, x_time)
+        from .. import ops
+
+        b, length, _ = x.shape
+        rows = self._native_rows(length, b, x.device)
+        inv = self._native_inverse(length, b, x.device)
+        eps = {blk.norm1.eps for blk in self.tcn} | {blk.norm2.eps for blk in self.tcn}
+        if len(eps) != 1:
+            raise ValueError("forward_cone: the native path takes one LayerNorm eps for all blocks")
+        p = self.tcn[0].dropout.p if self.training else 0.0
+        params = [self.input_proj.weight, self.input_proj.bias]
+        for blk in self.tcn:
+            params += [blk.conv1.conv.weight, blk.conv1.conv.bias, blk.norm1.weight, blk.norm1.bias,
+                       blk.conv2.conv.weight, blk.conv2.conv.bias, blk.norm2.weight, blk.norm2.bias]
+        return ops.tcn_cone(x, x_time, rows, inv, p, eps.pop(), params + [self.head.weight, self.head.bias])
+
+    def _cone_torch(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
+        """The cone through torch ops: the cross-check of the native kernels and the path of other shapes / devices."""
         b, length, _ = x.shape
         gather = self._cone_plan(length, x.device)
         h = F.linear(torch.cat([x, x_time], dim=-1), self.input_proj.weight[:, :, 0], self.input_proj.bias)  # (B, L, C)
@@ -94,7 +122,7 @@ class NormalPredictorTCN(nn.Module):
                 w = conv.conv.weight.permute(0, 2, 1).reshape(conv.conv.weight.shape[0], -1)   # (C, ks * C), tap-major
                 padded = torch.cat([y, zero], dim=1)            # last index = the zero row (left padding)
                 rows = padded.index_select(1, taps).view(b, -1, w.shape[1])    # (B, n_out, ks * C)
-                y = F.relu(norm(F.linear(rows, w, conv.conv.bias)))
+                y = blk.dropout(F.relu(norm(F.linear(rows, w, conv.conv.bias))))
             h = h.index_select(1, keep) + y
         return self.head(h[:, 0, :])
 
@@ -161,6 +189,39 @@ class NormalPredictorTCN(nn.Module):
                 n_src = n_out
             keep_rows = (win * n_in + keep.unsqueeze(0)).reshape(-1).to(torch.int32).contiguous()
             out.append((rows[0], rows[1], keep_rows))
+            n_in = keep.numel()
+        if len(cache) > 8:
+            cache.clear()
+        cache[key] = out
+        return out
+
+    def _native_inverse(self, length: int, batch: int, device):
+        """Inverses of ``_native_rows`` for the input gradients: per block (inv1, inv2, keep_inv), inv int32 (taps, rows
+        of the convolution's input) = the output row that reads input row r through that tap, or -1; keep_inv int32
+        (rows of the block input,) = the block output row that keeps input row r as its residual, or -1.  Each map must
+        be injective (within a window a fixed tap shifts positions by a constant), which is asserted here."""
+        cache = self.__dict__.setdefault("_native_inv", {})
+        key = (length, batch, str(device))
+        if key in cache:
+            return cache[key]
+
+        def invert(idx: torch.Tensor, n_rows: int) -> torch.Tensor:
+            idx = idx.view(-1, idx.shape[-1]).long()
+            out = torch.full((idx.shape[0], n_rows), -1, device=device, dtype=torch.int64)
+            m = torch.arange(idx.shape[1], device=device, dtype=torch.int64)
+            for t in range(idx.shape[0]):
+                ok = idx[t] >= 0
+                hit = idx[t][ok]
+                assert hit.unique().numel() == hit.numel(), "gather index is not injective: no gather-form input gradient"
+                out[t, hit] = m[ok]
+            return out.to(torch.int32).contiguous()
+
+        out = []
+        n_in = length
+        for (src1, src2, keep_rows), (taps1, _, keep) in zip(self._native_rows(length, batch, device),
+                                                              self._cone_plan(length, device)):
+            n_mid = taps1.numel() // src1.shape[0]
+            out.append((invert(src1, batch * n_in), invert(src2, batch * n_mid), invert(keep_rows, batch * n_in)[0]))
             n_in = keep.numel()
         if len(cache) > 8:
             cache.clear()

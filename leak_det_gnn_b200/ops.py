@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -945,3 +945,168 @@ def unblock32(t: torch.Tensor, l: int, q: int) -> torch.Tensor:
     w = t.shape[1] * 4
     qp = t.shape[0] * 32 // l
     return t.permute(0, 2, 1, 3).reshape(l, qp, w)[:, :q, :]
+
+
+# ----------------------------------------------------------------------------------------------
+# training of the TCN normal-state predictor on the dependency cone of the last time step (csrc/tcn_train.cu)
+# ----------------------------------------------------------------------------------------------
+def tcn_conv_train(x: torch.Tensor, src: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, gamma: torch.Tensor,
+                   beta: torch.Tensor, eps: float, res: Optional[torch.Tensor] = None, res_row: Optional[torch.Tensor] = None,
+                   drop_p: float = 0.0, drop_seed: int = 0):
+    """Raw training forward of one gathered-row convolution (see ltgnn_tcn_conv_train):
+    ``y[m] = [res[res_row[m]] +] dropout(relu(LayerNorm(z[m])))``, ``z = bias + sum_tap x[src[tap, m]] @ weight[tap].T``.
+    Returns ``(y, z, stats, live)``: stats (M, 2) = (mean, rstd) per row, live int32 (M, 4) = the 1-bit record of
+    ``dropout(relu(.)) > 0`` (bit b of word w <-> channel 32 w + b)."""
+    _check_act(x, "x")
+    _check_act(weight, "weight")
+    taps, m = src.shape
+    c = x.shape[-1]
+    if src.dtype != torch.int32 or not src.is_cuda or not src.is_contiguous():
+        raise ValueError("src must be a contiguous int32 CUDA tensor (taps, M)")
+    if tuple(weight.shape) != (taps, c, c):
+        raise ValueError(f"weight must be {(taps, c, c)}, got {tuple(weight.shape)}")
+    if (res is None) != (res_row is None):
+        raise ValueError("res and res_row come together")
+    y = torch.empty(m, c, device=x.device, dtype=torch.float32)
+    z = torch.empty(m, c, device=x.device, dtype=torch.float32)
+    stats = torch.empty(m, 2, device=x.device, dtype=torch.float32)
+    live = torch.empty(m, c // 32, device=x.device, dtype=torch.int32)
+    L = _lib.load()
+    ws = torch.empty(int(L.ltgnn_tcn_ws_floats(taps)), device=x.device, dtype=torch.float32)
+    tok = _inst.begin("tcn_conv_train")
+    _lib.check(L.ltgnn_tcn_conv_train(_dev_index(x), m, c, taps, x.data_ptr(), src.data_ptr(), weight.data_ptr(),
+                                      bias.data_ptr(), gamma.data_ptr(), beta.data_ptr(), float(eps),
+                                      None if res is None else res.data_ptr(), None if res_row is None else res_row.data_ptr(),
+                                      float(drop_p), int(drop_seed) & (2**64 - 1), y.data_ptr(), z.data_ptr(),
+                                      stats.data_ptr(), live.data_ptr(), ws.data_ptr(), _stream(x)))
+    _inst.end(tok)
+    return y, z, stats, live
+
+
+def tcn_ln_bwd(dy: torch.Tensor, live: torch.Tensor, z: torch.Tensor, stats: torch.Tensor, gamma: torch.Tensor,
+               scale: float):
+    """Raw epilogue backward (see ltgnn_tcn_ln_bwd): ``dz = LayerNorm_bwd(dy * live * scale)`` and the column sums
+    ``(d gamma, d beta, d bias)``.  Returns ``(dz, dgamma, dbeta, dbias)``."""
+    _check_act(dy, "dy")
+    m, c = dy.shape
+    dz = torch.empty_like(dy)
+    dprm = torch.empty(3, c, device=dy.device, dtype=torch.float32)
+    L = _lib.load()
+    dev = _dev_index(dy)
+    ws = torch.empty(int(L.ltgnn_tcn_ln_bwd_ws_floats(dev)), device=dy.device, dtype=torch.float32)
+    tok = _inst.begin("tcn_ln_bwd")
+    _lib.check(L.ltgnn_tcn_ln_bwd(dev, m, c, dy.data_ptr(), live.data_ptr(), z.data_ptr(), stats.data_ptr(),
+                                  gamma.data_ptr(), float(scale), dz.data_ptr(), dprm.data_ptr(), ws.data_ptr(), _stream(dy)))
+    _inst.end(tok)
+    return dz, dprm[0], dprm[1], dprm[2]
+
+
+def tcn_wgrad(dz: torch.Tensor, x: torch.Tensor, src: torch.Tensor) -> torch.Tensor:
+    """Raw weight gradient over gathered rows (see ltgnn_tcn_wgrad): ``dW[tap] = dz.T @ x[src[tap]]`` (row -1 = zeros),
+    returned as (taps, C_out, C_in)."""
+    _check_act(dz, "dz")
+    _check_act(x, "x")
+    taps, m = src.shape
+    c = x.shape[-1]
+    if dz.shape[0] != m or src.dtype != torch.int32 or not src.is_contiguous():
+        raise ValueError("tcn_wgrad: dz (M, C) and a contiguous int32 src (taps, M)")
+    dw = torch.empty(taps, c, c, device=dz.device, dtype=torch.float32)
+    L = _lib.load()
+    dev = _dev_index(dz)
+    ws = torch.empty(int(L.ltgnn_tgrad_ws_floats(dev, c)), device=dz.device, dtype=torch.float32)
+    tok = _inst.begin("tcn_wgrad")
+    _lib.check(L.ltgnn_tcn_wgrad(dev, m, c, taps, dz.data_ptr(), x.data_ptr(), src.data_ptr(), dw.data_ptr(), ws.data_ptr(),
+                                 _stream(dz)))
+    _inst.end(tok)
+    return dw
+
+
+class _TcnCone(torch.autograd.Function):
+    """The TCN predictor's cone as ONE autograd node: input projection -> per block two training convolutions (the
+    second with the residual) -> head on the last position; gradients for all parameters (the inputs are data).
+
+    Backward per convolution: epilogue backward (dz and the LayerNorm / bias column sums), weight gradient over the
+    gathered rows, input gradient as the forward's gathered GEMM with the inverse index and the per-tap transposed
+    weight (the block input's also receives the block output's gradient on the rows it keeps)."""
+
+    @staticmethod
+    def forward(ctx, inp, rows, inv, n_sensors, drop_p, eps, w_in, b_in, *rest):
+        n_blk = (len(rest) - 2) // 8
+        blocks = [rest[8 * i:8 * i + 8] for i in range(n_blk)]     # conv1 w, b, norm1 w, b, conv2 w, b, norm2 w, b
+        w_head, b_head = rest[-2], rest[-1]
+        c_in, c = w_in.shape[1], w_in.shape[0]
+        kp = inp.shape[1]
+        p = float(drop_p)
+        w_in_p = torch.zeros(c, kp, device=inp.device, dtype=torch.float32)
+        w_in_p[:, :c_in] = w_in[:, :, 0]
+        h = linear_tc(inp, w_in_p, b_in.contiguous())
+        saved, lives = [], []
+        for (w1, b1, g1, e1, w2, b2, g2, e2), (src1, src2, keep) in zip(blocks, rows):
+            w1p, w2p = w1.permute(2, 0, 1).contiguous(), w2.permute(2, 0, 1).contiguous()   # (taps, C_out, C_in)
+            y1, z1, s1, l1 = tcn_conv_train(h, src1, w1p, b1, g1, e1, eps, drop_p=p,
+                                            drop_seed=new_dropout_seed() if p > 0 else 0)
+            h2, z2, s2, l2 = tcn_conv_train(y1, src2, w2p, b2, g2, e2, eps, res=h, res_row=keep, drop_p=p,
+                                            drop_seed=new_dropout_seed() if p > 0 else 0)
+            saved += [h, y1, z1, s1, l1, z2, s2, l2, w1p, w2p, g1, g2]
+            lives += [l1, l2]
+            h = h2
+        if DEBUG_CAPTURE is not None:
+            DEBUG_CAPTURE["tcn_lives"] = lives
+        n_pad = (n_sensors + 31) // 32 * 32
+        w_out = torch.zeros(n_pad, c, device=inp.device, dtype=torch.float32)
+        w_out[:n_sensors] = w_head
+        b_out = torch.zeros(n_pad, device=inp.device, dtype=torch.float32)
+        b_out[:n_sensors] = b_head
+        pred = linear_tc(h, w_out, b_out)[:, :n_sensors]
+        ctx.save_for_backward(inp, h, w_out, *saved)
+        ctx.rows, ctx.inv, ctx.n_blk, ctx.c_in, ctx.n_sensors = rows, inv, n_blk, c_in, n_sensors
+        ctx.scale = 1.0 / (1.0 - p)
+        return pred
+
+    @staticmethod
+    def backward(ctx, dpred):
+        inp, h_last, w_out, *saved = ctx.saved_tensors
+        s, c = ctx.n_sensors, h_last.shape[1]
+        bsz = h_last.shape[0]
+        dp = torch.zeros(bsz, 64, device=dpred.device, dtype=torch.float32)   # wgrad_tc takes 64 or 128 output rows
+        dp[:, :s] = dpred
+        h_aug = torch.zeros(bsz, c + 32, device=dpred.device, dtype=torch.float32)
+        h_aug[:, :c] = h_last
+        h_aug[:, c] = 1.0                                           # the ones column: its product column is d bias
+        t_head = wgrad(dp, h_aug)
+        dh = linear_tc(dp[:, :w_out.shape[0]].contiguous(), w_out, transposed=True)
+        zero_bias = torch.zeros(c, device=dpred.device, dtype=torch.float32)
+        grads = [None] * (8 * ctx.n_blk)
+        for i in range(ctx.n_blk - 1, -1, -1):
+            h_in, y1, z1, s1, l1, z2, s2, l2, w1p, w2p, g1, g2 = saved[12 * i:12 * i + 12]
+            src1, src2, _ = ctx.rows[i]
+            inv1, inv2, keep_inv = ctx.inv[i]
+            dz2, dg2, de2, db2 = tcn_ln_bwd(dh.contiguous(), l2, z2, s2, g2, ctx.scale)
+            dw2 = tcn_wgrad(dz2, y1, src2)
+            dy1 = tcn_conv(dz2, inv2, w2p.transpose(1, 2).contiguous(), zero_bias, relu=False)
+            dz1, dg1, de1, db1 = tcn_ln_bwd(dy1, l1, z1, s1, g1, ctx.scale)
+            dw1 = tcn_wgrad(dz1, h_in, src1)
+            dh = tcn_conv(dz1, inv1, w1p.transpose(1, 2).contiguous(), zero_bias, relu=False, res=dh.contiguous(),
+                          res_row=keep_inv)
+            grads[8 * i:8 * i + 8] = [dw1.permute(1, 2, 0), db1, dg1, de1, dw2.permute(1, 2, 0), db2, dg2, de2]
+        t_in = wgrad(dh, inp)
+        d_w_in = t_in[:, :ctx.c_in].unsqueeze(-1)
+        d_b_in = t_in[:, ctx.c_in].contiguous()
+        return (None, None, None, None, None, None, d_w_in, d_b_in, *grads, t_head[:s, :c].contiguous(),
+                t_head[:s, c].contiguous())
+
+
+def tcn_cone(x: torch.Tensor, x_time: torch.Tensor, rows, inv, drop_p: float, eps: float, params) -> torch.Tensor:
+    """Differentiable prediction (B, S) of the TCN predictor from its dependency cone on the sm_100a kernels.
+    ``rows`` / ``inv``: per block the gather indices and their inverses (NormalPredictorTCN._native_rows /
+    _native_inverse); ``params``: the 36 tensors in the order input_proj.{weight, bias}, per block conv1.{weight, bias},
+    norm1.{weight, bias}, conv2.{weight, bias}, norm2.{weight, bias}, head.{weight, bias}."""
+    _check_act(x.contiguous(), "x")
+    b, length, s = x.shape
+    c_in = s + x_time.shape[-1]
+    kp = 64 if c_in < 64 else 96           # one zero-weight column for the ones that turn the weight gradient into d bias
+    inp = torch.zeros(b * length, kp, device=x.device, dtype=torch.float32)
+    inp.view(b, length, kp)[:, :, :s] = x
+    inp.view(b, length, kp)[:, :, s:c_in] = x_time
+    inp[:, c_in] = 1.0
+    return _TcnCone.apply(inp, rows, inv, s, float(drop_p), float(eps), *params)
