@@ -317,6 +317,19 @@ int64_t ltgnn_gru_ws_floats(int device);
 int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r, const float* tf,
                     const float* hseq, const float* dG, float* dBfused, float* ws, void* stream);
 
+/* ---- one layer of the GRU normal-state predictor (predictor.py:84-111), forward only (csrc/gru_pred.cu) -------------
+ * Q sequences of L steps, torch.nn.GRU equations and gate order (r, z, n), h_0 = 0.  The input projection is computed
+ * beforehand (ltgnn_linear, one launch per gate group):
+ *   gx [3][Q*L][H]: gx[g][q*L + t] = x_(q,t) W_ih[g]^T + b_ih[g], plus b_hh[g] for g = r, z (not for n)
+ * w_hh [3H, H] and b_hn = b_hh[2H:3H] in torch layout.  Writes h_last [Q, H] (the state after step L-1) and, if hseq is
+ * not NULL, every state: hseq [Q, L, H] (the next layer's input).  H = 128 only (else LTGNN_E_SHAPE); Q, L > 0 and
+ * gx, w_hh, b_hn, h_last non-NULL (else LTGNN_E_ARG); gx, w_hh, hseq, h_last 16-byte aligned (else LTGNN_E_ALIGN).
+ * Clusters of 4 CTAs per 128 sequences exchange the state through distributed shared memory; 3xTF32 tcgen05 products.
+ * Deterministic, no allocation or host synchronisation: capturable into a CUDA graph.
+ */
+int ltgnn_gru_layer_fwd(int device, int64_t Q, int32_t L, int32_t H, const float* gx, const float* w_hh, const float* b_hn,
+                        float* hseq, float* h_last, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

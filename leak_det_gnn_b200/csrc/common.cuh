@@ -7,6 +7,7 @@
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
+#include <utility>
 
 #include "ltgnn.h"
 
@@ -74,6 +75,26 @@ struct DeviceInfo {
 };
 // returns nullptr (and records the error) if the device cannot be queried
 const DeviceInfo* device_info(int device);
+
+// Launch `kernel` as clusters of `cluster_x` CTAs along x (grid.x must be a multiple of it).  A plain cudaLaunchKernelEx:
+// capturable into a CUDA graph like a <<<>>> launch.
+template <typename... Params, typename... Args>
+cudaError_t launch_cluster(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                           unsigned cluster_x, Args&&... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cluster_x;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
 
 // out[i] (+)= sum_{c < n_parts} parts[c * stride + i], i < n, added in index order: the deterministic
 // second stage of every cross-CTA reduction in this library (no float atomics anywhere)
@@ -281,6 +302,31 @@ __device__ __forceinline__ size_t b32(size_t row, int f4, int w4) { return ((row
 // exact floor(x / d) for any 32-bit x: magic = floor((2^64 - 1) / d) + 1 (host side, d >= 2)
 __device__ __forceinline__ uint32_t fastdiv(uint32_t x, uint64_t magic) {
     return static_cast<uint32_t>(__umul64hi(static_cast<uint64_t>(x), magic));
+}
+
+// ---- thread-block clusters: distributed shared memory and the cluster-wide barrier ----
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+// the shared::cluster address of the same shared::cta offset in CTA `rank` of this cluster
+__device__ __forceinline__ uint32_t mapa_shared(uint32_t saddr, uint32_t rank) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
+    return r;
+}
+__device__ __forceinline__ void st_cluster_v4(uint32_t addr, const float4& v) {
+    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+                 : "memory");
+}
+// Every thread of every CTA of the cluster arrives (release: its shared::cluster writes are published) and later waits
+// (acquire: the peers' writes before their arrive are visible).  Between the two a thread may do unrelated work.
+__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
+__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
+__device__ __forceinline__ void cluster_sync() {
+    cluster_arrive();
+    cluster_wait();
 }
 
 __device__ __forceinline__ bool elect_one() {

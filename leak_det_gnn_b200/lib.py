@@ -91,6 +91,8 @@ SIGNATURES = {
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_bwd_w": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gru_layer_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p]),
 }
 
 _lib = None

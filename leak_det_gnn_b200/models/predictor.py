@@ -259,7 +259,8 @@ class NormalPredictorTCN(nn.Module):
 
 
 class NormalPredictorGRU(nn.Module):
-    """Two-layer GRU baseline (predictor.py:84-111); cuDNN, not a kernel target."""
+    """Two-layer GRU baseline (predictor.py:84-111).  ``forward`` is the reference's (cuDNN); ``forward_last`` is the
+    frozen predictor's inference path, on the sm_100a kernels at hidden 128 (csrc/gru_pred.cu + csrc/linear.cu)."""
 
     def __init__(self, num_sensors: int, time_dim: int = 9, hidden_size: int = 128, num_layers: int = 2,
                  dropout: float = 0.1) -> None:
@@ -273,6 +274,50 @@ class NormalPredictorGRU(nn.Module):
     def forward(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
         out, _ = self.gru(torch.cat([x, x_time], dim=-1))
         return self.head(out[:, -1, :])
+
+    # use the hand-written sm_100a kernels for ``forward_last`` on CUDA where the shapes allow; False = the dense cuDNN
+    # ``forward``, kept as the cross-check
+    use_native = True
+
+    def _native_ok(self, x: torch.Tensor) -> bool:
+        g = self.gru
+        return (self.use_native and x.is_cuda and x.dtype == torch.float32 and g.hidden_size == 128 and g.bias
+                and g.num_layers >= 1 and self.num_sensors + self.time_dim <= 64)
+
+    @torch.no_grad()
+    def forward_last(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
+        """``forward``'s result in eval mode: every layer's recurrence on the tensor cores (``ops.gru_predictor_fwd``),
+        the head through ``ops.linear_tc``.  Other shapes and devices run the dense ``forward``."""
+        if self.training:
+            raise RuntimeError("forward_last is the inference path of the frozen predictor (call .eval() first)")
+        if not self._native_ok(x):
+            return self.forward(x, x_time)
+        from .. import ops
+
+        prep = self._native_weights(x.device)
+        h = ops.gru_predictor_fwd(x, x_time, prep["layers"])
+        return ops.linear_tc(h, prep["w_out"], prep["b_out"])[:, :self.num_sensors]
+
+    def _native_weights(self, device):
+        """Weights in the kernels' layouts, rebuilt when a parameter changes (the predictor is frozen in practice)."""
+        cache = self.__dict__.setdefault("_native_w", {})
+        ver = tuple(p._version for p in self.parameters()) + (str(device),)
+        if cache.get("ver") == ver:
+            return cache["prep"]
+        from .. import ops
+
+        g = self.gru
+        layers = ops.gru_predictor_weights([(getattr(g, f"weight_ih_l{i}"), getattr(g, f"weight_hh_l{i}"),
+                                             getattr(g, f"bias_ih_l{i}"), getattr(g, f"bias_hh_l{i}"))
+                                            for i in range(g.num_layers)])
+        n_out = (self.num_sensors + 15) // 16 * 16               # the head's N, padded to the kernel's granularity
+        w_out = torch.zeros(n_out, g.hidden_size, device=device)
+        w_out[: self.num_sensors] = self.head.weight
+        b_out = torch.zeros(n_out, device=device)
+        b_out[: self.num_sensors] = self.head.bias
+        prep = {"layers": layers, "w_out": w_out, "b_out": b_out}
+        cache.update(ver=ver, prep=prep)
+        return prep
 
 
 def cone_positions(length: int, kernel_size: int, dilations: List[int]) -> List[Tuple[List[int], List[int]]]:

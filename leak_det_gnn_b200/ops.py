@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -910,6 +910,68 @@ def gru_encode(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_
         raise ValueError("gru_encode: gradients with respect to the inputs are not implemented by the native GRU "
                          "(the reference never asks for them); use the cuDNN route (use_native = False)")
     return _GruEncoder.apply(r, tf, w_ih, w_hh, b_ih, b_hh)
+
+
+# ----------------------------------------------------------------------------------------------
+# GRU normal-state predictor at hidden 128 (reference models/predictor.py:84-111), inference only (csrc/gru_pred.cu)
+# ----------------------------------------------------------------------------------------------
+def gru_predictor_weights(layers, k0: int = 64) -> list:
+    """torch.nn.GRU parameters [(w_ih, w_hh, b_ih, b_hh) per layer] -> per layer (w_x [3, H, K], b_x [3, H], w_hh [3H, H],
+    b_hn [H]): the input projection per gate group with layer 0's input columns zero-padded to K = k0 (the projection
+    kernel's K granularity), b_hh of the r and z gates folded into b_x; b_hn = b_hh of the n gate stays inside r * (.)."""
+    out = []
+    for i, (w_ih, w_hh, b_ih, b_hh) in enumerate(layers):
+        h = w_hh.shape[1]
+        k = k0 if i == 0 else h
+        if w_ih.shape[1] > k:
+            raise ValueError(f"gru_predictor_weights: layer {i} has {w_ih.shape[1]} inputs, the projection takes <= {k}")
+        w_x = w_ih.new_zeros(3, h, k)
+        w_x[:, :, : w_ih.shape[1]] = w_ih.detach().view(3, h, -1)
+        b_x = b_ih.detach().view(3, h).clone()
+        b_x[:2] += b_hh.detach().view(3, h)[:2]
+        out.append((w_x, b_x, w_hh.detach().contiguous(), b_hh.detach()[2 * h:].contiguous()))
+    return out
+
+
+def gru_layer_fwd(inp: torch.Tensor, q: int, l: int, layer, seq: bool = False):
+    """Raw (non-differentiable) forward of one GRU layer over q sequences of l steps.  inp (q * l, K) fp32 CUDA, row
+    q_i * l + t = the input of sequence q_i at step t; ``layer`` = one entry of ``gru_predictor_weights``.
+    Returns (h_last (q, H), hseq (q * l, H) or None): gx = inp W_x[g]^T + b_x[g] by ``linear_tc`` (one N = H launch per
+    gate group), then the recurrence ``ltgnn_gru_layer_fwd``."""
+    _check_act(inp, "inp")
+    w_x, b_x, w_hh, b_hn = layer
+    hdim = w_hh.shape[1]
+    if inp.shape != (q * l, w_x.shape[2]):
+        raise ValueError(f"inp must be ({q * l}, {w_x.shape[2]}), got {tuple(inp.shape)}")
+    gx = torch.empty(3, q * l, hdim, device=inp.device, dtype=torch.float32)
+    for g in range(3):
+        linear_tc(inp, w_x[g], b_x[g], out=gx[g])
+    h_last = torch.empty(q, hdim, device=inp.device, dtype=torch.float32)
+    hseq = torch.empty(q * l, hdim, device=inp.device, dtype=torch.float32) if seq else None
+    L = _lib.load()
+    tok = _inst.begin("gru_pred_layer")
+    _lib.check(L.ltgnn_gru_layer_fwd(_dev_index(inp), q, l, hdim, gx.data_ptr(), w_hh.data_ptr(), b_hn.data_ptr(),
+                                     None if hseq is None else hseq.data_ptr(), h_last.data_ptr(), _stream(inp)))
+    _inst.end(tok)
+    return h_last, hseq
+
+
+def gru_predictor_fwd(x: torch.Tensor, x_time: torch.Tensor, layers) -> torch.Tensor:
+    """Raw (non-differentiable) stacked GRU: x (Q, L, S), x_time (Q, L, F) -> the last layer's state after step L-1, (Q, H).
+    Layer i's input is cat([x, x_time]) (zero-padded to K) for i = 0 and layer i-1's state sequence otherwise (no
+    inter-layer dropout: inference).  ``layers``: ``gru_predictor_weights(...)``."""
+    q, l, s = x.shape
+    f = x_time.shape[-1]
+    k0 = layers[0][0].shape[2]
+    if s + f > k0:
+        raise ValueError(f"gru_predictor_fwd: {s} + {f} inputs exceed K = {k0}")
+    inp = torch.zeros(q, l, k0, device=x.device, dtype=torch.float32)
+    inp[:, :, :s] = x
+    inp[:, :, s:s + f] = x_time
+    inp = inp.view(q * l, k0)
+    for i, layer in enumerate(layers):
+        h_last, inp = gru_layer_fwd(inp, q, l, layer, seq=i + 1 < len(layers))
+    return h_last
 
 
 def tcn_conv(x: torch.Tensor, src: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor,
