@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LTGNN_VERSION 100 /* major*10000 + minor*100 + patch : 0.1.0 */
+#define LTGNN_VERSION 200 /* major*10000 + minor*100 + patch : 0.2.0 */
 
 typedef enum ltgnn_status {
     LTGNN_OK = 0,
@@ -286,33 +286,22 @@ int ltgnn_tcn_wgrad(int device, int64_t M, int32_t C, int32_t taps, const float*
 /* ---- shared per-sensor GRU encoder (detector.py:28-73; SURVEY 8f rank 2) -----------------------
  * Sequence q = b*S + s has input [r[b,t,s], tf[b,t,0..F)] at step t (the reference's cat([rr, tf]) order);
  * weights in torch.nn.GRU layout (gate order r, z, n): w_ih [3H, 1+F], w_hh [3H, H], b_ih, b_hh [3H].  H = 64.
- * gru_fwd:    h_last [B*S, H] = hidden state after step L-1 (h_0 = 0).  For training also pass
- *             hseq (every state, logical [L*Qp, H]) and gates (r, z, n, W_hn h + b_hn; logical [L*Qp, 4H]; with
- *             save_hn = 0 only r, z, n: [L*Qp, 3H], for gru_bwd_dg_hn),
- *             Qp = B*S rounded up to 128, both in the kernels' blocked-32 layout [rows/32][W/4][32][4]; NULL otherwise.
- *             State lives in tensor memory; recurrent + input GEMM fused on tcgen05 (3xTF32).
- * gru_bwd_dg: back-propagation through time given dh_last [B*S, H]: writes dG (blocked-32, [L*Qp, 4H]), the gradient wrt
- *             the four pre-activation groups (r, z, W_hn h + b_hn, W_in x + b_in).
- * gru_bwd_w:  dBfused [4H, 96] = sum_(t,q) dG^T [h_{t-1} | x | tf | 1 | 0]: columns 0..H-1 are d w_hh, H..H+F
- *             d w_ih, H+F+1 the bias gradients (rows: r, z, hn-part, in-part).  ws: ltgnn_gru_ws_floats() floats.
+ * gru_fwd:       h_last [B*S, H] = hidden state after step L-1 (h_0 = 0).  For training also pass hseq (every state,
+ *                logical [L*Qp, H]) and gates (r, z, n; logical [L*Qp, 3H]), Qp = B*S rounded up to 128, both in the
+ *                kernels' blocked-32 layout [rows/32][W/4][32][4]; NULL otherwise.
+ *                State lives in tensor memory; recurrent + input GEMM fused on tcgen05 (3xTF32).
+ * gru_bwd_dg_hn: back-propagation through time given dh_last [B*S, H] and the forward's hseq and gates3 (r, z, n):
+ *                writes dG (blocked-32, [L*Qp, 4H]), the gradient wrt the four pre-activation groups
+ *                (r, z, W_hn h + b_hn, W_in x + b_in).  W_hn h_{t-1} + b_hn is rebuilt per step by one 64-column
+ *                tensor-core GEMM instead of being saved: 8.75 GB less written and read at B*S = 118 784, L = 288.
+ * gru_bwd_w:     dBfused [4H, 96] = sum_(t,q) dG^T [h_{t-1} | x | tf | 1 | 0]: columns 0..H-1 are d w_hh, H..H+F
+ *                d w_ih, H+F+1 the bias gradients (rows: r, z, hn-part, in-part).  ws: ltgnn_gru_ws_floats() floats.
  */
 int ltgnn_gru_fwd(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r, const float* tf,
                   const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, float* h_last,
-                  float* hseq, float* gates, int32_t save_hn, void* stream);
-int ltgnn_gru_bwd_dg(int device, int64_t Q, int32_t L, int32_t H, const float* w_hh, const float* gates,
-                     const float* hseq, const float* dh_last, float* dG, void* stream);
-/* gru_bwd_dg_hn: the BPTT for gates saved without the fourth group (gru_fwd with save_hn = 0): W_hn h_{t-1} + b_hn is
- * rebuilt per step by one 64-column tensor-core GEMM; 8.75 GB less written and read at L = 288.  Same dG. */
+                  float* hseq, float* gates, void* stream);
 int ltgnn_gru_bwd_dg_hn(int device, int64_t Q, int32_t L, int32_t H, const float* w_hh, const float* b_hh,
                         const float* gates3, const float* hseq, const float* dh_last, float* dG, void* stream);
-/* Recompute form of the BPTT: the forward saves only hseq (pass gates = NULL to gru_fwd), the gates are rebuilt per step
- * from h_{t-1} on the tensor cores.  gru_inproj: P [B*L, 3H] = W_ih[:, 1:] tf + b_ih (+ b_hh for the r and z rows), the
- * part of the pre-activations the S sensors of a window share.  gru_bwd_dg_rc: same dG as gru_bwd_dg. */
-int ltgnn_gru_inproj(int device, int64_t B, int32_t L, int32_t F, int32_t H, const float* tf, const float* w_ih,
-                     const float* b_ih, const float* b_hh, float* P, void* stream);
-int ltgnn_gru_bwd_dg_rc(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r,
-                        const float* w_ih, const float* w_hh, const float* b_hh, const float* P, const float* hseq,
-                        const float* dh_last, float* dG, void* stream);
 int64_t ltgnn_gru_ws_floats(int device);
 int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r, const float* tf,
                     const float* hseq, const float* dG, float* dBfused, float* ws, void* stream);

@@ -36,6 +36,7 @@ constexpr int kAuxIn = 31;       // x + up to 30 time features, held in register
 constexpr int kMmaWarp = kGateWarps;
 constexpr int kThreads = (kGateWarps + 1) * 32;
 constexpr uint32_t kAccCol = 0, kAhiCol = NG, kAloCol = NG + KA;  // TMEM column map (448 of 512 used)
+constexpr int kDg3W4 = 3 * H / 4;  // float4 per row of the saved r | z | n
 
 struct GruParams {
     const float* r;      // [B, L, S]
@@ -46,8 +47,7 @@ struct GruParams {
     const float* b_hh;   // [3H]
     float* h_last;       // [Q, H]
     float* hseq;         // blocked-32 [L * Qp, H] or nullptr
-    float* gates;        // blocked-32 [L * Qp, 4H] (r | z | n | W_hn h + b_hn), or 3H without the last group, or nullptr
-    int gates_w4;        // float4 per saved gates row: 64 (four groups) or 48 (r | z | n: hn is rebuilt by the backward)
+    float* gates;        // blocked-32 [L * Qp, 3H] (r | z | n: the backward rebuilds W_hn h + b_hn) or nullptr
     uint32_t Q;          // B * S sequences
     uint32_t Qp;         // Q rounded up to a multiple of 128
     int L, S, F;
@@ -70,12 +70,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const float* v) {
         ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]),
           "f"(v[9]), "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15])
         : "memory");
-}
-
-__device__ __forceinline__ void tmem_st4(uint32_t taddr, const float* v) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]),
-                 "f"(v[3])
-                 : "memory");
 }
 
 // element (n, k) of the fused operand described in the file header.  Rows are ordered in 4 blocks of 64 so that
@@ -231,14 +225,11 @@ gru_fwd_kernel(const GruParams p) {
                     const int f0 = 4 * u;  // float4 index of unit 16 u within a 64-wide group
                     if (p.gates) {
                         float4* g4 = reinterpret_cast<float4*>(p.gates);
-                        const int w4 = p.gates_w4;
 #pragma unroll
                         for (int j = 0; j < 4; ++j) {
-                            stg_stream(g4 + b32(row, 0 * (H / 4) + f0 + j, w4), make_float4(rr[4 * j], rr[4 * j + 1], rr[4 * j + 2], rr[4 * j + 3]));
-                            stg_stream(g4 + b32(row, 1 * (H / 4) + f0 + j, w4), make_float4(zz[4 * j], zz[4 * j + 1], zz[4 * j + 2], zz[4 * j + 3]));
-                            stg_stream(g4 + b32(row, 2 * (H / 4) + f0 + j, w4), make_float4(in[4 * j], in[4 * j + 1], in[4 * j + 2], in[4 * j + 3]));
-                            if (w4 == H)
-                                stg_stream(g4 + b32(row, 3 * (H / 4) + f0 + j, w4), make_float4(hn[4 * j], hn[4 * j + 1], hn[4 * j + 2], hn[4 * j + 3]));
+                            stg_stream(g4 + b32(row, 0 * (H / 4) + f0 + j, kDg3W4), make_float4(rr[4 * j], rr[4 * j + 1], rr[4 * j + 2], rr[4 * j + 3]));
+                            stg_stream(g4 + b32(row, 1 * (H / 4) + f0 + j, kDg3W4), make_float4(zz[4 * j], zz[4 * j + 1], zz[4 * j + 2], zz[4 * j + 3]));
+                            stg_stream(g4 + b32(row, 2 * (H / 4) + f0 + j, kDg3W4), make_float4(in[4 * j], in[4 * j + 1], in[4 * j + 2], in[4 * j + 3]));
                         }
                     }
                     if (p.hseq) {
@@ -320,247 +311,29 @@ gru_fwd_kernel(const GruParams p) {
 
 
 // =====================================================================================================
-// backward through time.  Per step t = L-1 .. 0 and tile of 128 sequences, with dh = d loss / d h_t:
+// backward through time, from the gates r, z, n and the states the forward saved.  Per step t = L-1 .. 0 and tile of 128
+// sequences, with dh = d loss / d h_t:
+//   hn = W_hn h_{t-1} + b_hn                       rebuilt by one 64-column tcgen05 GEMM (A = h_{t-1} hi / lo in TMEM)
 //   dn = dh (1 - z);  dn_pre = dn (1 - n^2);  dz_pre = dh (h_{t-1} - n) z (1 - z);
 //   dr_pre = dn_pre * hn * r (1 - r);  dhn = dn_pre * r;  din = dn_pre
 //   dG(t) = [dr_pre | dz_pre | dhn | din]  -> written to HBM for the weight-gradient GEMM (tgrad.cuh)
-//   dh_{t-1} = dh z + [dr_pre | dz_pre | dhn] [W_hr; W_hz; W_hn]          (tcgen05, A = dG in TMEM)
-// Gates r, z, n and hn = W_hn h + b_hn were saved by the forward, so no transcendental is recomputed.
+//   dh_{t-1} = dh z + [dr_pre | dz_pre | dhn] [W_hr; W_hz; W_hn]      (second tcgen05 GEMM, A = dG hi / lo in TMEM)
+// No transcendental is recomputed.  Rebuilding hn instead of saving it spares the forward's writes and the BPTT's reads
+// of one gate group (8.75 GB at B*S = 118 784, L = 288); the second MMA round trip stays under the HBM time of the step.
+// Tensor memory (448 of 512 columns): dh accumulator 64 | 192 columns that hold the hn accumulator (the first 64), then
+// dG lo | 192 columns that hold h_{t-1} hi + lo (the first 128), then dG hi.  Every reuse is by the thread that owned the
+// columns, after the MMA that read them has committed.
 // =====================================================================================================
 constexpr int KB = 3 * H;  // 192: K of the dh_{t-1} GEMM
-constexpr uint32_t kB_acc = 0, kB_hi = H, kB_lo = H + KB;  // TMEM: acc 64 | dG hi 192 | dG lo 192 = 448 columns
-
-struct GruBwdParams {
-    const float* w_hh;   // [3H, H]
-    const float* gates;  // blocked-32 [L * Qp, 4H]
-    const float* hseq;   // blocked-32 [L * Qp, H]
-    const float* dh_last;  // [Q, H]
-    float* dG;           // blocked-32 [L * Qp, 4H]
-    uint32_t Q, Qp;
-    int L;
-};
-
-__global__ void __launch_bounds__(kThreads, 1)
-gru_bwd_kernel(const GruBwdParams p) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ uint64_t bar_a, bar_d;
-    __shared__ uint32_t tmem_base_s;
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint8_t* b_hi = smem;                 // B2[n = h column (64)][k = gate row (192)] = w_hh[k][n], K-major SW128
-    uint8_t* b_lo = b_hi + H * KB * 4;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (warp == kMmaWarp) tmem_alloc(&tmem_base_s, 512);
-    if (tid == 0) {
-        mbar_init(&bar_a, kGateWarps);
-        mbar_init(&bar_d, 1);
-        fence_mbar_init();
-    }
-    for (int i = tid; i < KB * H; i += kThreads) {
-        const int k = i / H, n = i - k * H;  // coalesced read of w_hh[k][n]
-        const float w = __ldg(p.w_hh + i);
-        const float hi = tf32_hi(w);
-        const uint32_t off = sw128_offset(n, k >> 2, H) + (k & 3) * 4;
-        *reinterpret_cast<float*>(b_hi + off) = hi;
-        *reinterpret_cast<float*>(b_lo + off) = w - hi;
-    }
-    fence_proxy_async_smem();
-    fence_before_sync();
-    __syncthreads();
-    fence_after_sync();
-    const uint32_t tmem = tmem_base_s;
-    const uint32_t n_tiles = (p.Q + 127) / 128;
-    uint32_t ph_a = 0, ph_d = 0;
-
-    if (warp < kGateWarps) {
-        const int quad = warp & 3, half = warp >> 2;
-        const uint32_t lane_off = static_cast<uint32_t>(quad * 32) << 16;
-        const int j0 = half * 32;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const uint32_t q = tile * 128 + quad * 32 + lane;
-            const bool valid = q < p.Q;
-            float dh[32];
-            {
-                const float4* src = reinterpret_cast<const float4*>(p.dh_last + static_cast<size_t>(valid ? q : 0) * H + j0);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 v = valid ? __ldg(src + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    dh[4 * j] = v.x; dh[4 * j + 1] = v.y; dh[4 * j + 2] = v.z; dh[4 * j + 3] = v.w;
-                }
-            }
-            for (int t = p.L - 1; t >= 0; --t) {
-                const size_t row = static_cast<size_t>(t) * p.Qp + q;  // pad rows (q >= Q) exist in the saved tensors
-                const float4* g4 = reinterpret_cast<const float4*>(p.gates);
-                const float4* h4 = reinterpret_cast<const float4*>(p.hseq);
-                float4* dg4 = reinterpret_cast<float4*>(p.dG);
-                float zkeep[32];
-#pragma unroll
-                for (int c = 0; c < 32; c += 16) {
-                    float r[16], z[16], n[16], hn[16], hm[16];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-                        const int f0 = ((j0 + c) >> 2) + j;
-                        const float4 a = valid ? ldg_stream(g4 + b32(row, 0 * (H / 4) + f0, H)) : zero;
-                        const float4 b = valid ? ldg_stream(g4 + b32(row, 1 * (H / 4) + f0, H)) : zero;
-                        const float4 d = valid ? ldg_stream(g4 + b32(row, 2 * (H / 4) + f0, H)) : zero;
-                        const float4 e = valid ? ldg_stream(g4 + b32(row, 3 * (H / 4) + f0, H)) : zero;
-                        const float4 f = (valid && t > 0) ? ldg_stream(h4 + b32(row - p.Qp, f0, H / 4)) : zero;
-                        r[4 * j] = a.x; r[4 * j + 1] = a.y; r[4 * j + 2] = a.z; r[4 * j + 3] = a.w;
-                        z[4 * j] = b.x; z[4 * j + 1] = b.y; z[4 * j + 2] = b.z; z[4 * j + 3] = b.w;
-                        n[4 * j] = d.x; n[4 * j + 1] = d.y; n[4 * j + 2] = d.z; n[4 * j + 3] = d.w;
-                        hn[4 * j] = e.x; hn[4 * j + 1] = e.y; hn[4 * j + 2] = e.z; hn[4 * j + 3] = e.w;
-                        hm[4 * j] = f.x; hm[4 * j + 1] = f.y; hm[4 * j + 2] = f.z; hm[4 * j + 3] = f.w;
-                    }
-                    float dr[16], dz[16], dhn[16], din[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        const float g = dh[c + j];
-                        const float dnp = g * (1.f - z[j]) * (1.f - n[j] * n[j]);
-                        dz[j] = g * (hm[j] - n[j]) * z[j] * (1.f - z[j]);
-                        dr[j] = dnp * hn[j] * r[j] * (1.f - r[j]);
-                        dhn[j] = dnp * r[j];
-                        din[j] = dnp;
-                        zkeep[c + j] = z[j];
-                    }
-                    {   // pad rows carry zeros (their dh and gates are zero), so the weight-gradient GEMM may read them
-                        const int f0 = (j0 + c) >> 2;
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            stg_stream(dg4 + b32(row, 0 * (H / 4) + f0 + j, H), make_float4(dr[4 * j], dr[4 * j + 1], dr[4 * j + 2], dr[4 * j + 3]));
-                            stg_stream(dg4 + b32(row, 1 * (H / 4) + f0 + j, H), make_float4(dz[4 * j], dz[4 * j + 1], dz[4 * j + 2], dz[4 * j + 3]));
-                            stg_stream(dg4 + b32(row, 2 * (H / 4) + f0 + j, H), make_float4(dhn[4 * j], dhn[4 * j + 1], dhn[4 * j + 2], dhn[4 * j + 3]));
-                            stg_stream(dg4 + b32(row, 3 * (H / 4) + f0 + j, H), make_float4(din[4 * j], din[4 * j + 1], din[4 * j + 2], din[4 * j + 3]));
-                        }
-                    }
-                    // A operand of the dh_{t-1} GEMM: columns [g * 64 + j0 + c, +16) for g = r, z, hn
-                    float lo[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { const float x = dr[j]; dr[j] = tf32_hi(x); lo[j] = x - dr[j]; }
-                    tmem_st16(tmem + lane_off + kB_hi + 0 * H + j0 + c, dr);
-                    tmem_st16(tmem + lane_off + kB_lo + 0 * H + j0 + c, lo);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { const float x = dz[j]; dz[j] = tf32_hi(x); lo[j] = x - dz[j]; }
-                    tmem_st16(tmem + lane_off + kB_hi + 1 * H + j0 + c, dz);
-                    tmem_st16(tmem + lane_off + kB_lo + 1 * H + j0 + c, lo);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { const float x = dhn[j]; dhn[j] = tf32_hi(x); lo[j] = x - dhn[j]; }
-                    tmem_st16(tmem + lane_off + kB_hi + 2 * H + j0 + c, dhn);
-                    tmem_st16(tmem + lane_off + kB_lo + 2 * H + j0 + c, lo);
-                }
-                tmem_wait_st();
-                fence_before_sync();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&bar_a);
-
-                mbar_wait(&bar_d, ph_d);
-                ph_d ^= 1;
-                fence_after_sync();
-#pragma unroll
-                for (int c = 0; c < 32; c += 16) {
-                    float acc[16];
-                    tmem_ld16(tmem + lane_off + kB_acc + j0 + c, acc);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) dh[c + j] = fmaf(dh[c + j], zkeep[c + j], acc[j]);
-                }
-                fence_before_sync();
-            }
-        }
-    } else {
-        const uint32_t idesc = idesc_tf32(128, H);
-        const uint32_t bh = desc_lo(smem_u32(b_hi)), bl = desc_lo(smem_u32(b_lo));
-        constexpr uint32_t kg_units = H * 128u >> 4;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            for (int t = 0; t < p.L; ++t) {
-                mbar_wait(&bar_a, ph_a);
-                ph_a ^= 1;
-                fence_after_sync();
-                if (elect_one()) {
-#pragma unroll
-                    for (uint32_t ks = 0; ks < KB / 8; ++ks) {
-                        const uint32_t boff = (ks >> 2) * kg_units + 2 * (ks & 3);
-                        mma_tf32_ts(tmem + kB_acc, tmem + kB_lo + 8 * ks, bh + boff, idesc, ks == 0 ? 0u : 1u);
-                        mma_tf32_ts(tmem + kB_acc, tmem + kB_hi + 8 * ks, bl + boff, idesc, 1u);
-                        mma_tf32_ts(tmem + kB_acc, tmem + kB_hi + 8 * ks, bh + boff, idesc, 1u);
-                    }
-                    commit(&bar_d);
-                }
-                __syncwarp();
-            }
-        }
-    }
-    fence_before_sync();
-    __syncthreads();
-    if (warp == kMmaWarp) {
-        fence_after_sync();
-        tmem_dealloc(tmem, 512);
-    }
-}
-
-
-// =====================================================================================================
-// backward through time WITHOUT saved gates ("recompute" form).  The forward then saves only the states
-// (8.75 GB at B*S = 118 784, L = 288 instead of 43.8 GB), and the BPTT kernel reads 8.75 GB instead of 43.8 GB.
-// Per step t and tile of 128 sequences:
-//   pre[r | z | hn] = h_{t-1} W_hh^T                       tcgen05, A = h_{t-1} (hi / lo) in TMEM, 192 columns
-//   r, z = sigma(pre + P + w_x x_t),  hn = pre + b_hn,  n = tanh(P_in + w_xn x_t + r hn)
-//       P[b, t, :] = W_ih[:, 1:] tf_t + b_ih (+ b_hh for r, z) is shared by the S sensors of a window and comes from a
-//       small pre-pass (gru_inproj_kernel, 0.9 GB); w_x = W_ih[:, 0] and b_hn live in shared memory
-//   dG(t) as in gru_bwd_kernel -> HBM;  dh_{t-1} = dh z + [dr | dz | dhn] W_hh      (second tcgen05 round trip)
-// Tensor memory (448 columns): dh accumulator 64 | pre-activations 192, reused for dG lo | h_{t-1} hi+lo 128, reused
-// (192) for dG hi.  Every reuse is by the thread that owned the columns, after the MMA that read them has committed.
-// =====================================================================================================
 constexpr uint32_t kR_accDh = 0, kR_accR = H, kR_a = H + KB;  // 64 | 192 | 192
+constexpr int kGateWarpsHn = 16, kThreadsHn = kGateWarpsHn * 32;  // 4 gate warps per scheduler hide the loads
 
-struct GruBwdRcParams {
-    const float* w_hh;     // [3H, H]
-    const float* w_ih;     // [3H, 1 + F]
-    const float* b_hh;     // [3H]
-    const float* P;        // [B * L, 3H] input projections (r | z | in)
-    const float* r;        // [B, L, S] inputs
-    const float* hseq;     // blocked-32 [L * Qp, H]
-    const float* dh_last;  // [Q, H]
-    float* dG;             // blocked-32 [L * Qp, 4H]
-    uint32_t Q, Qp;
-    int L, S, F;
-    uint64_t magic_s;
-};
-
-// P[(b L + t), n] = b_ih[n] (+ b_hh[n] for the r and z rows) + sum_f W_ih[n, 1 + f] tf[b, t, f]
-__global__ void __launch_bounds__(KB)
-gru_inproj_kernel(const float* __restrict__ tf, const float* __restrict__ w_ih, const float* __restrict__ b_ih,
-                  const float* __restrict__ b_hh, float* __restrict__ P, int64_t rows, int F) {
-    // thread n keeps its weight row and bias in registers and walks the (b, t) rows: coalesced 768-byte stores
-    const int n = threadIdx.x, fi = 1 + F;
-    float w[kAuxIn];
-#pragma unroll
-    for (int f = 0; f < kAuxIn - 1; ++f) w[f] = f < F ? __ldg(w_ih + n * fi + 1 + f) : 0.f;
-    const float bias = __ldg(b_ih + n) + (n < 2 * H ? __ldg(b_hh + n) : 0.f);
-    for (int64_t row0 = static_cast<int64_t>(blockIdx.x) * 4; row0 < rows; row0 += static_cast<int64_t>(gridDim.x) * 4) {
-        float acc[4];  // four rows in flight: the loop is a chain of dependent-latency loads otherwise
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            acc[u] = bias;
-            if (row0 + u < rows) {
-#pragma unroll
-                for (int f = 0; f < kAuxIn - 1; ++f)
-                    if (f < F) acc[u] = fmaf(w[f], __ldg(tf + (row0 + u) * F + f), acc[u]);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-            if (row0 + u < rows) P[(row0 + u) * KB + n] = acc[u];
-    }
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const float* v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]),
+                 "f"(v[3])
+                 : "memory");
 }
 
-// =====================================================================================================
-// backward through time with r | z | n saved and hn = W_hn h_{t-1} + b_hn rebuilt per step (one extra 64-column
-// tcgen05 GEMM, no transcendental): the forward writes and the BPTT reads 8.75 GB less than with four saved
-// groups, at the price of a second MMA round trip that stays under the HBM time of the step.
-// Tensor memory as in gru_bwd_rc_kernel (the 64 hn columns sit at the start of the dG-lo region).
-// =====================================================================================================
-constexpr int kDg3W4 = 3 * H / 4;  // float4 per row of the saved r | z | n
-constexpr int kGateWarpsHn = 16, kThreadsHn = kGateWarpsHn * 32;  // 4 gate warps per scheduler hide the loads
 struct GruBwdHnParams {
     const float* w_hh;     // [3H, H]
     const float* b_hh;     // [3H]
@@ -774,231 +547,11 @@ gru_bwd_hn_kernel(const GruBwdHnParams p) {
     }
 }
 
-
-__global__ void __launch_bounds__(kThreadsHn, 1)
-gru_bwd_rc_kernel(const GruBwdRcParams p) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ uint64_t bar_a1, bar_a2, bar_r, bar_d;
-    __shared__ uint32_t tmem_base_s;
-    __shared__ float4 wx_s[KB / 4], bhn_s[H / 4];  // W_ih[:, 0] (r | z | n rows), b_hh of the n rows
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint8_t* b1_hi = smem;                  // B1[n = gate row (192)][k = h column (64)] = w_hh[n][k], K-major SW128
-    uint8_t* b1_lo = b1_hi + KB * H * 4;
-    uint8_t* b2_hi = b1_lo + KB * H * 4;    // B2[n = h column (64)][k = gate row (192)] = w_hh[k][n], K-major SW128
-    uint8_t* b2_lo = b2_hi + H * KB * 4;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (warp == 0) tmem_alloc(&tmem_base_s, 512);
-    if (tid == 0) {
-        mbar_init(&bar_a1, kGateWarpsHn);
-        mbar_init(&bar_a2, kGateWarpsHn);
-        mbar_init(&bar_r, 1);
-        mbar_init(&bar_d, 1);
-        fence_mbar_init();
-    }
-    for (int i = tid; i < KB * H; i += kThreadsHn) {
-        const int k = i / H, n = i - k * H;  // w_hh[k][n]: k = gate row, n = h column
-        const float w = __ldg(p.w_hh + i);
-        const float hi = tf32_hi(w), lo = w - hi;
-        const uint32_t o2 = sw128_offset(n, k >> 2, H) + (k & 3) * 4;
-        *reinterpret_cast<float*>(b2_hi + o2) = hi;
-        *reinterpret_cast<float*>(b2_lo + o2) = lo;
-        const uint32_t o1 = sw128_offset(k, n >> 2, KB) + (n & 3) * 4;
-        *reinterpret_cast<float*>(b1_hi + o1) = hi;
-        *reinterpret_cast<float*>(b1_lo + o1) = lo;
-    }
-    if (tid < KB) reinterpret_cast<float*>(wx_s)[tid] = __ldg(p.w_ih + tid * (1 + p.F));
-    if (tid < H) reinterpret_cast<float*>(bhn_s)[tid] = __ldg(p.b_hh + 2 * H + tid);
-    fence_proxy_async_smem();
-    fence_before_sync();
-    __syncthreads();
-    fence_after_sync();
-    const uint32_t tmem = tmem_base_s;
-    const uint32_t n_tiles = (p.Q + 127) / 128;
-    uint32_t ph = 0;  // one phase bit serves all four barriers: each completes exactly once per step
-
-    {
-        // 16 gate warps: thread = one sequence (TMEM lane) x 16 hidden units [16 part, +16).  Warp 0 also issues the
-        // two GEMMs of a step (it would only wait for them otherwise): 16 warps = 4 per scheduler, 128 registers each.
-        const uint32_t idesc1 = idesc_tf32(128, KB), idesc2 = idesc_tf32(128, H);
-        const uint32_t b1h = desc_lo(smem_u32(b1_hi)), b1l = desc_lo(smem_u32(b1_lo));
-        const uint32_t b2h = desc_lo(smem_u32(b2_hi)), b2l = desc_lo(smem_u32(b2_lo));
-        constexpr uint32_t kg1 = KB * 128u >> 4, kg2 = H * 128u >> 4;  // one 32-column k-atom block of B1 / B2
-        const int quad = warp & 3, part = warp >> 2;
-        const uint32_t lane_off = static_cast<uint32_t>(quad * 32) << 16;
-        const int j0 = part * 16;
-        const float4* h4 = reinterpret_cast<const float4*>(p.hseq);
-        float4* dg4 = reinterpret_cast<float4*>(p.dG);
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            const uint32_t q = tile * 128 + quad * 32 + lane;
-            const bool valid = q < p.Q;
-            const uint32_t b = p.magic_s ? fastdiv(valid ? q : 0, p.magic_s) : (valid ? q : 0);
-            const uint32_t sidx = (valid ? q : 0) - b * p.S;
-            const float* xr = p.r + static_cast<size_t>(b) * p.L * p.S + sidx;          // + t * S
-            const float4* Pb = reinterpret_cast<const float4*>(p.P) + static_cast<size_t>(b) * p.L * (KB / 4);  // + t * 48
-            float dh[16], hm[16];
-            {
-                const float4* src = reinterpret_cast<const float4*>(p.dh_last + static_cast<size_t>(valid ? q : 0) * H + j0);
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const float4 v = valid ? __ldg(src + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    dh[4 * j] = v.x; dh[4 * j + 1] = v.y; dh[4 * j + 2] = v.z; dh[4 * j + 3] = v.w;
-                }
-            }
-            auto load_h = [&](int t) {  // h_{t-1}[j0 .. j0 + 16): zero for t = 0 and for pad rows
-                const size_t prow = static_cast<size_t>(t > 0 ? t - 1 : 0) * p.Qp + q;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const float4 v = (valid && t > 0) ? ldg_stream(h4 + b32(prow, (j0 >> 2) + j, H / 4)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    hm[4 * j] = v.x; hm[4 * j + 1] = v.y; hm[4 * j + 2] = v.z; hm[4 * j + 3] = v.w;
-                }
-            };
-            load_h(p.L - 1);
-            for (int t = p.L - 1; t >= 0; --t) {
-                const size_t row = static_cast<size_t>(t) * p.Qp + q;
-                const float x = valid ? __ldg(xr + static_cast<size_t>(t) * p.S) : 0.f;
-                // ---- A = h_{t-1} (hi | lo), this thread's 16 of the 64 columns
-#pragma unroll
-                for (int c = 0; c < 16; c += 16) {
-                    float hi[16], lo[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { hi[j] = tf32_hi(hm[c + j]); lo[j] = hm[c + j] - hi[j]; }
-                    tmem_st16(tmem + lane_off + kR_a + j0 + c, hi);
-                    tmem_st16(tmem + lane_off + kR_a + H + j0 + c, lo);
-                }
-                tmem_wait_st();
-                fence_before_sync();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&bar_a1);
-                {
-                    const int f0 = j0 >> 2;  // float4 index of this thread's units inside a 64-wide group
-                    // P + w_x x_t for the r | z | n pre-activations: requested before the first GEMM is waited for (the
-                    // S sensors of a window read the same P lines: L1 hits after the first toucher)
-                    float4 r4[4], z4[4], n4[4];
-                    {
-                        const float4* Pt = Pb + static_cast<size_t>(t) * (KB / 4) + f0;
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            const float4 pr = __ldg(Pt + j), pz = __ldg(Pt + H / 4 + j), pn = __ldg(Pt + 2 * (H / 4) + j);
-                            const float4 wr = wx_s[f0 + j], wz = wx_s[H / 4 + f0 + j], wn = wx_s[2 * (H / 4) + f0 + j];
-                            r4[j] = make_float4(fmaf(wr.x, x, pr.x), fmaf(wr.y, x, pr.y), fmaf(wr.z, x, pr.z), fmaf(wr.w, x, pr.w));
-                            z4[j] = make_float4(fmaf(wz.x, x, pz.x), fmaf(wz.y, x, pz.y), fmaf(wz.z, x, pz.z), fmaf(wz.w, x, pz.w));
-                            n4[j] = make_float4(fmaf(wn.x, x, pn.x), fmaf(wn.y, x, pn.y), fmaf(wn.z, x, pn.z), fmaf(wn.w, x, pn.w));
-                        }
-                    }
-                    if (warp == 0) {  // r | z | hn pre-activations = h_{t-1} W_hh^T
-                        mbar_wait(&bar_a1, ph);
-                        fence_after_sync();
-                        if (elect_one()) {
-#pragma unroll
-                            for (uint32_t ks = 0; ks < H / 8; ++ks) {
-                                const uint32_t boff = (ks >> 2) * kg1 + 2 * (ks & 3);
-                                mma_tf32_ts(tmem + kR_accR, tmem + kR_a + H + 8 * ks, b1h + boff, idesc1, ks == 0 ? 0u : 1u);
-                                mma_tf32_ts(tmem + kR_accR, tmem + kR_a + 8 * ks, b1l + boff, idesc1, 1u);
-                                mma_tf32_ts(tmem + kR_accR, tmem + kR_a + 8 * ks, b1h + boff, idesc1, 1u);
-                            }
-                            commit(&bar_r);
-                        }
-                        __syncwarp();
-                    }
-                    mbar_wait(&bar_r, ph);
-                    fence_after_sync();
-                    float ar[16], az[16], hn[16];
-                    tmem_ld16(tmem + lane_off + kR_accR + 0 * H + j0, ar);
-                    tmem_ld16(tmem + lane_off + kR_accR + 1 * H + j0, az);
-                    tmem_ld16(tmem + lane_off + kR_accR + 2 * H + j0, hn);
-                    // four units at a time: gates, dG to HBM, its hi / lo to tensor memory (hi over the consumed
-                    // h_{t-1} columns, lo over the consumed pre-activation columns)
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const float4 bb = bhn_s[f0 + j];
-                        const float ir[4] = {r4[j].x, r4[j].y, r4[j].z, r4[j].w}, iz[4] = {z4[j].x, z4[j].y, z4[j].z, z4[j].w};
-                        const float in[4] = {n4[j].x, n4[j].y, n4[j].z, n4[j].w}, bh[4] = {bb.x, bb.y, bb.z, bb.w};
-                        float rr[4], zz[4], nn[4];
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            rr[e] = sigmoidf_fast(ar[4 * j + e] + ir[e]);
-                            zz[e] = sigmoidf_fast(az[4 * j + e] + iz[e]);
-                            nn[e] = tanhf_fast(fmaf(rr[e], hn[4 * j + e] + bh[e], in[e]));
-                        }
-                        float dr[4], dz[4], dhn[4], din[4];
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const float g = dh[4 * j + e], hv = hn[4 * j + e] + bh[e];
-                            const float dnp = g * (1.f - zz[e]) * (1.f - nn[e] * nn[e]);
-                            dz[e] = g * (hm[4 * j + e] - nn[e]) * zz[e] * (1.f - zz[e]);
-                            dr[e] = dnp * hv * rr[e] * (1.f - rr[e]);
-                            dhn[e] = dnp * rr[e];
-                            din[e] = dnp;
-                            dh[4 * j + e] = g * zz[e];  // the accumulator of the second GEMM is added after the wait below
-                        }
-                        // pad rows carry zeros (their dh is zero)
-                        stg_stream(dg4 + b32(row, 0 * (H / 4) + f0 + j, H), make_float4(dr[0], dr[1], dr[2], dr[3]));
-                        stg_stream(dg4 + b32(row, 1 * (H / 4) + f0 + j, H), make_float4(dz[0], dz[1], dz[2], dz[3]));
-                        stg_stream(dg4 + b32(row, 2 * (H / 4) + f0 + j, H), make_float4(dhn[0], dhn[1], dhn[2], dhn[3]));
-                        stg_stream(dg4 + b32(row, 3 * (H / 4) + f0 + j, H), make_float4(din[0], din[1], din[2], din[3]));
-                        float hi[4], lo[4];
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) { hi[e] = tf32_hi(dr[e]); lo[e] = dr[e] - hi[e]; }
-                        tmem_st4(tmem + lane_off + kR_a + 0 * H + j0 + 4 * j, hi);
-                        tmem_st4(tmem + lane_off + kR_accR + 0 * H + j0 + 4 * j, lo);
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) { hi[e] = tf32_hi(dz[e]); lo[e] = dz[e] - hi[e]; }
-                        tmem_st4(tmem + lane_off + kR_a + 1 * H + j0 + 4 * j, hi);
-                        tmem_st4(tmem + lane_off + kR_accR + 1 * H + j0 + 4 * j, lo);
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) { hi[e] = tf32_hi(dhn[e]); lo[e] = dhn[e] - hi[e]; }
-                        tmem_st4(tmem + lane_off + kR_a + 2 * H + j0 + 4 * j, hi);
-                        tmem_st4(tmem + lane_off + kR_accR + 2 * H + j0 + 4 * j, lo);
-                    }
-                }
-                tmem_wait_st();
-                fence_before_sync();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&bar_a2);
-                if (t > 0) load_h(t - 1);  // h_{t-2}: in flight while the second GEMM runs
-                if (warp == 0) {  // dh_{t-1} += [dr | dz | dhn] W_hh
-                    mbar_wait(&bar_a2, ph);
-                    fence_after_sync();
-                    if (elect_one()) {
-#pragma unroll
-                        for (uint32_t ks = 0; ks < KB / 8; ++ks) {
-                            const uint32_t boff = (ks >> 2) * kg2 + 2 * (ks & 3);
-                            mma_tf32_ts(tmem + kR_accDh, tmem + kR_accR + 8 * ks, b2h + boff, idesc2, ks == 0 ? 0u : 1u);
-                            mma_tf32_ts(tmem + kR_accDh, tmem + kR_a + 8 * ks, b2l + boff, idesc2, 1u);
-                            mma_tf32_ts(tmem + kR_accDh, tmem + kR_a + 8 * ks, b2h + boff, idesc2, 1u);
-                        }
-                        commit(&bar_d);
-                    }
-                    __syncwarp();
-                }
-                mbar_wait(&bar_d, ph);
-                fence_after_sync();
-#pragma unroll
-                for (int c = 0; c < 16; c += 16) {
-                    float acc[16];
-                    tmem_ld16(tmem + lane_off + kR_accDh + j0 + c, acc);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) dh[c + j] += acc[j];
-                }
-                fence_before_sync();
-                ph ^= 1;
-            }
-        }
-    }
-    fence_before_sync();
-    __syncthreads();
-    if (warp == 0) {
-        fence_after_sync();
-        tmem_dealloc(tmem, 512);
-    }
-}
-
 }  // namespace
 
 extern "C" int ltgnn_gru_fwd(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t Hdim, const float* r,
                              const float* tf, const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh,
-                             float* h_last, float* hseq, float* gates, int32_t save_hn, void* stream_) {
+                             float* h_last, float* hseq, float* gates, void* stream_) {
     LTGNN_REQUIRE(B >= 0 && L > 0 && S > 0 && F >= 0, LTGNN_E_ARG, "gru_fwd: B=%lld L=%d S=%d F=%d",
                   static_cast<long long>(B), L, S, F);
     LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_fwd: hidden size %d not supported (64 only)", Hdim);
@@ -1012,8 +565,7 @@ extern "C" int ltgnn_gru_fwd(int device, int64_t B, int32_t L, int32_t S, int32_
     LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "gru_fwd: device is sm_%d%d, need sm_100", di->cc_major,
                   di->cc_minor);
     LTGNN_USE_DEVICE(device);
-    GruParams p{r, F ? tf : nullptr, w_ih, w_hh, b_ih, b_hh, h_last, hseq, gates, save_hn ? H : 3 * H / 4,
-                static_cast<uint32_t>(B * S),
+    GruParams p{r, F ? tf : nullptr, w_ih, w_hh, b_ih, b_hh, h_last, hseq, gates, static_cast<uint32_t>(B * S),
                 static_cast<uint32_t>((B * S + 127) / 128 * 128), L, S, F,
                 S >= 2 ? (~0ull / static_cast<uint64_t>(S)) + 1 : 0ull};
     const size_t smem = 1024 + 2ull * NG * KA * 4;
@@ -1022,80 +574,6 @@ extern "C" int ltgnn_gru_fwd(int device, int64_t B, int32_t L, int32_t S, int32_
     const int64_t tiles = (B * S + 127) / 128;
     const int grid = static_cast<int>(tiles < di->sm_count ? tiles : di->sm_count);
     gru_fwd_kernel<<<grid, kThreads, smem, static_cast<cudaStream_t>(stream_)>>>(p);
-    LTGNN_CUDA_TRY(cudaGetLastError());
-    return LTGNN_OK;
-}
-
-extern "C" int ltgnn_gru_bwd_dg(int device, int64_t Q, int32_t L, int32_t Hdim, const float* w_hh, const float* gates,
-                                const float* hseq, const float* dh_last, float* dG, void* stream_) {
-    LTGNN_REQUIRE(Q >= 0 && L > 0, LTGNN_E_ARG, "gru_bwd_dg: Q=%lld L=%d", static_cast<long long>(Q), L);
-    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_bwd_dg: hidden size %d not supported (64 only)", Hdim);
-    LTGNN_REQUIRE(Q < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_bwd_dg: too many sequences");
-    if (Q == 0) return LTGNN_OK;
-    LTGNN_REQUIRE(w_hh && gates && hseq && dh_last && dG, LTGNN_E_ARG, "gru_bwd_dg: null tensor");
-    LTGNN_REQUIRE(aligned16(gates) && aligned16(hseq) && aligned16(dh_last) && aligned16(dG), LTGNN_E_ALIGN,
-                  "gru_bwd_dg: 16-byte alignment required");
-    const DeviceInfo* di = device_info(device);
-    if (!di) return LTGNN_E_CUDA;
-    LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "gru_bwd_dg: device is sm_%d%d, need sm_100", di->cc_major,
-                  di->cc_minor);
-    LTGNN_USE_DEVICE(device);
-    GruBwdParams p{w_hh, gates, hseq, dh_last, dG, static_cast<uint32_t>(Q), static_cast<uint32_t>((Q + 127) / 128 * 128), L};
-    const size_t smem = 1024 + 2ull * H * KB * 4;
-    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    const int64_t tiles = (Q + 127) / 128;
-    const int grid = static_cast<int>(tiles < di->sm_count ? tiles : di->sm_count);
-    gru_bwd_kernel<<<grid, kThreads, smem, static_cast<cudaStream_t>(stream_)>>>(p);
-    LTGNN_CUDA_TRY(cudaGetLastError());
-    return LTGNN_OK;
-}
-
-extern "C" int ltgnn_gru_inproj(int device, int64_t B, int32_t L, int32_t F, int32_t Hdim, const float* tf,
-                                const float* w_ih, const float* b_ih, const float* b_hh, float* P, void* stream_) {
-    LTGNN_REQUIRE(B >= 0 && L > 0 && F >= 0, LTGNN_E_ARG, "gru_inproj: B=%lld L=%d F=%d", static_cast<long long>(B), L, F);
-    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_inproj: hidden size %d not supported (64 only)", Hdim);
-    if (B == 0) return LTGNN_OK;
-    LTGNN_REQUIRE(w_ih && b_ih && b_hh && P && (tf || F == 0), LTGNN_E_ARG, "gru_inproj: null tensor");
-    const DeviceInfo* di = device_info(device);
-    if (!di) return LTGNN_E_CUDA;
-    LTGNN_USE_DEVICE(device);
-    const int64_t rows = B * L;
-    LTGNN_REQUIRE(F < kAuxIn, LTGNN_E_SHAPE, "gru_inproj: %d time features not supported", F);
-    int64_t blocks = (rows + 3) / 4;
-    const int64_t cap = static_cast<int64_t>(di->sm_count) * 10;
-    if (blocks > cap) blocks = cap;
-    gru_inproj_kernel<<<static_cast<int>(blocks), KB, 0, static_cast<cudaStream_t>(stream_)>>>(tf, w_ih, b_ih, b_hh, P,
-                                                                                                rows, F);
-    LTGNN_CUDA_TRY(cudaGetLastError());
-    return LTGNN_OK;
-}
-
-extern "C" int ltgnn_gru_bwd_dg_rc(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t Hdim, const float* r,
-                                   const float* w_ih, const float* w_hh, const float* b_hh, const float* P,
-                                   const float* hseq, const float* dh_last, float* dG, void* stream_) {
-    LTGNN_REQUIRE(B >= 0 && L > 0 && S > 0 && F >= 0, LTGNN_E_ARG, "gru_bwd_dg_rc: B=%lld L=%d S=%d F=%d",
-                  static_cast<long long>(B), L, S, F);
-    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_bwd_dg_rc: hidden size %d not supported (64 only)", Hdim);
-    LTGNN_REQUIRE(B * S < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_bwd_dg_rc: too many sequences");
-    if (B == 0) return LTGNN_OK;
-    LTGNN_REQUIRE(r && w_ih && w_hh && b_hh && P && hseq && dh_last && dG, LTGNN_E_ARG, "gru_bwd_dg_rc: null tensor");
-    LTGNN_REQUIRE(aligned16(P) && aligned16(hseq) && aligned16(dh_last) && aligned16(dG), LTGNN_E_ALIGN,
-                  "gru_bwd_dg_rc: 16-byte alignment required");
-    const DeviceInfo* di = device_info(device);
-    if (!di) return LTGNN_E_CUDA;
-    LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "gru_bwd_dg_rc: device is sm_%d%d, need sm_100", di->cc_major,
-                  di->cc_minor);
-    LTGNN_USE_DEVICE(device);
-    const int64_t Q = B * S;
-    GruBwdRcParams p{w_hh, w_ih, b_hh, P, r, hseq, dh_last, dG, static_cast<uint32_t>(Q),
-                     static_cast<uint32_t>((Q + 127) / 128 * 128), L, S, F,
-                     S >= 2 ? (~0ull / static_cast<uint64_t>(S)) + 1 : 0ull};
-    const size_t smem = 1024 + 4ull * H * KB * 4;
-    LTGNN_REQUIRE(smem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "gru_bwd_dg_rc: %zu B of shared memory", smem);
-    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_bwd_rc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    const int64_t tiles = (Q + 127) / 128;
-    const int grid = static_cast<int>(tiles < di->sm_count ? tiles : di->sm_count);
-    gru_bwd_rc_kernel<<<grid, kThreadsHn, smem, static_cast<cudaStream_t>(stream_)>>>(p);
     LTGNN_CUDA_TRY(cudaGetLastError());
     return LTGNN_OK;
 }

@@ -79,16 +79,10 @@ SIGNATURES = {
     "ltgnn_pipe_feat_bwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
-                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_bwd_dg_hn": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_void_p, c_void_p]),
-    "ltgnn_gru_bwd_dg": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                 c_void_p]),
     "ltgnn_gru_ws_floats": (c_int64, [c_int]),
-    "ltgnn_gru_inproj": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
-                                 c_void_p, c_void_p]),
-    "ltgnn_gru_bwd_dg_rc": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
-                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_bwd_w": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_layer_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -790,18 +790,9 @@ def gru_supported(hidden: int, n_time: int) -> bool:
     return hidden == 64 and 0 <= n_time <= 30
 
 
-# How the BPTT gets the gates of every step:
-#   "hn"    (default) the forward saves r | z | n next to the states, the BPTT rebuilds W_hn h + b_hn with one small GEMM
-#   "saved" the forward saves all four groups (r | z | n | hn), the BPTT only reads them
-#   "all"   memory-saving: the forward saves only the states (8.75 instead of 43.8 GB at B=4096, L=288) and the BPTT
-#           rebuilds every gate per step on the tensor cores (sigma / tanh inside the serial chain: slower)
-GRU_BPTT = "hn"
-
-
-def gru_fwd(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh, save: bool = False,
-            gate_groups: int = 4):
-    """Raw forward: r (B,L,S), tf (B,L,F) or None -> h_last (B,S,H) [, hseq, gates in blocked-32 layout].
-    ``gate_groups``: 4 saves r | z | n | hn, 3 saves r | z | n, 0 saves no gates (states only)."""
+def gru_fwd(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh, save: bool = False):
+    """Raw forward: r (B,L,S), tf (B,L,F) or None -> h_last (B,S,H) [, hseq, gates r | z | n in blocked-32 layout].
+    The BPTT rebuilds the fourth pre-activation group W_hn h + b_hn instead of reading it."""
     _check_act(r, "r")
     b, l, s = r.shape
     f = 0 if tf is None else tf.shape[-1]
@@ -813,14 +804,13 @@ def gru_fwd(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh,
     # stored as [L * Qp / 32, W / 4, 32, 4] (see csrc/gru.cu)
     qp = (b * s + 127) // 128 * 128
     hseq = torch.empty(l * qp // 32, hdim // 4, 32, 4, device=r.device, dtype=torch.float32) if save else None
-    gates = (torch.empty(l * qp // 32, gate_groups * hdim // 4, 32, 4, device=r.device, dtype=torch.float32)
-             if save and gate_groups else None)
+    gates = torch.empty(l * qp // 32, 3 * hdim // 4, 32, 4, device=r.device, dtype=torch.float32) if save else None
     L = _lib.load()
     tok = _inst.begin("gru_fwd")
     _lib.check(L.ltgnn_gru_fwd(_dev_index(r), b, l, s, f, hdim, r.data_ptr(), None if tf is None else tf.data_ptr(),
                                w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), h_last.data_ptr(),
                                None if hseq is None else hseq.data_ptr(), None if gates is None else gates.data_ptr(),
-                               int(gate_groups == 4), _stream(r)))
+                               _stream(r)))
     _inst.end(tok)
     return (h_last, hseq, gates) if save else h_last
 
@@ -835,25 +825,15 @@ class _GruEncoder(torch.autograd.Function):
         tf = None if tf is None else tf.contiguous()
         params = [t.contiguous() for t in (w_ih, w_hh, b_ih, b_hh)]
         if any(ctx.needs_input_grad[2:]):
-            if GRU_BPTT not in ("hn", "saved", "all"):
-                raise ValueError(f"ops.GRU_BPTT = {GRU_BPTT!r}")
-            ctx.mode = GRU_BPTT
-            h_last, hseq, gates = gru_fwd(r, tf, *params, save=True, gate_groups={"hn": 3, "saved": 4, "all": 0}[ctx.mode])
-            if ctx.mode == "all":
-                ctx.save_for_backward(r, tf, *params, hseq)
-            else:
-                ctx.save_for_backward(r, tf, params[1], params[3], hseq, gates)
-        else:
-            ctx.mode = None  # nothing requires a gradient: backward is never reached
+            h_last, hseq, gates = gru_fwd(r, tf, *params, save=True)
+            ctx.save_for_backward(r, tf, params[1], params[3], hseq, gates)
+        else:  # nothing requires a gradient: backward is never reached
             h_last = gru_fwd(r, tf, *params)
         return h_last
 
     @staticmethod
     def backward(ctx, dh):
-        if ctx.mode == "all":
-            r, tf, w_ih, w_hh, b_ih, b_hh, hseq = ctx.saved_tensors
-        else:
-            r, tf, w_hh, b_hh, hseq, gates = ctx.saved_tensors
+        r, tf, w_hh, b_hh, hseq, gates = ctx.saved_tensors
         b, l, s = r.shape
         f = 0 if tf is None else tf.shape[-1]
         hd = w_hh.shape[1]
@@ -862,31 +842,11 @@ class _GruEncoder(torch.autograd.Function):
         L = _lib.load()
         dh = dh.contiguous()
         dg = torch.empty(hseq.shape[0], hd, 32, 4, device=r.device, dtype=torch.float32)  # blocked-32 [L*Qp, 4H]
-        if ctx.mode == "all":
-            # input projections shared by the S sensors of a window: P [B*L, 3H]
-            proj = torch.empty(b * l, 3 * hd, device=r.device, dtype=torch.float32)
-            tok = _inst.begin("gru_inproj")
-            _lib.check(L.ltgnn_gru_inproj(dev, b, l, f, hd, None if tf is None else tf.data_ptr(), w_ih.data_ptr(),
-                                          b_ih.data_ptr(), b_hh.data_ptr(), proj.data_ptr(), _stream(r)))
-            _inst.end(tok)
-            tok = _inst.begin("gru_bwd_dg")
-            _lib.check(L.ltgnn_gru_bwd_dg_rc(dev, b, l, s, f, hd, r.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(),
-                                             b_hh.data_ptr(), proj.data_ptr(), hseq.data_ptr(), dh.data_ptr(),
-                                             dg.data_ptr(), _stream(r)))
-            _inst.end(tok)
-            del proj
-        elif ctx.mode == "hn":
-            tok = _inst.begin("gru_bwd_dg")
-            _lib.check(L.ltgnn_gru_bwd_dg_hn(dev, q, l, hd, w_hh.data_ptr(), b_hh.data_ptr(), gates.data_ptr(),
-                                             hseq.data_ptr(), dh.data_ptr(), dg.data_ptr(), _stream(r)))
-            _inst.end(tok)
-            del gates
-        else:
-            tok = _inst.begin("gru_bwd_dg")
-            _lib.check(L.ltgnn_gru_bwd_dg(dev, q, l, hd, w_hh.data_ptr(), gates.data_ptr(), hseq.data_ptr(),
-                                          dh.data_ptr(), dg.data_ptr(), _stream(r)))
-            _inst.end(tok)
-            del gates
+        tok = _inst.begin("gru_bwd_dg")
+        _lib.check(L.ltgnn_gru_bwd_dg_hn(dev, q, l, hd, w_hh.data_ptr(), b_hh.data_ptr(), gates.data_ptr(),
+                                         hseq.data_ptr(), dh.data_ptr(), dg.data_ptr(), _stream(r)))
+        _inst.end(tok)
+        del gates
         fused = torch.empty(4 * hd, 96, device=r.device, dtype=torch.float32)
         ws = torch.empty(int(L.ltgnn_gru_ws_floats(dev)), device=r.device, dtype=torch.float32)
         tok = _inst.begin("gru_bwd_w")

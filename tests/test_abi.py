@@ -23,7 +23,7 @@ def test_library_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in ltgnn.h but not exported"
     assert sorted(L.SIGNATURES) == names, "lib.SIGNATURES must mirror ltgnn.h"
-    assert lib.ltgnn_version() == 100
+    assert lib.ltgnn_version() == 200
 
 
 def test_no_cpu_fallback_in_product():

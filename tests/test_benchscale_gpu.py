@@ -105,10 +105,8 @@ def test_gru_forward_many_tiles_per_cta():
     assert all(v <= 2e-5 for v in rep.values()), rep
 
 
-@pytest.mark.parametrize("mode", ["hn", "saved", "all"])
-def test_gru_backward_many_tiles_per_cta(mode, monkeypatch):
-    """The three BPTT forms + the weight-gradient pass at 318 sequence tiles (> 2 per CTA)."""
-    monkeypatch.setattr(ops, "GRU_BPTT", mode)
+def test_gru_backward_many_tiles_per_cta():
+    """The BPTT + the weight-gradient pass at 318 sequence tiles (> 2 per CTA)."""
     b, l, s, f = 1400, 8, 29, 9
     torch.manual_seed(12)
     gru = torch.nn.GRU(input_size=1 + f, hidden_size=64, num_layers=1, batch_first=True).double()
@@ -120,7 +118,7 @@ def test_gru_backward_many_tiles_per_cta(mode, monkeypatch):
     h = ops.gru_encode(r.cuda(), tf.cuda(), *w)
     (h.reshape(b * s, 64) * dh.cuda()).sum().backward()
     rep = {n: rel_err(p.grad, getattr(gru, n).grad) for n, p in zip(GRU_NAMES, w)}
-    parity_log(f"gru_bwd_many_tiles mode={mode} B={b} L={l}", rep)
+    parity_log(f"gru_bwd_many_tiles B={b} L={l}", rep)
     assert all(v <= 5e-5 for v in rep.values()), rep
 
 

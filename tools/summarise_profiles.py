@@ -29,7 +29,7 @@ def short(name):
         return f"spmm_staged_kernel<epi={m.group(1)},gate={m.group(2)}>"
     if "spmm_staged" in name:
         return "spmm_staged_kernel"
-    for k in ("gru_fwd_kernel", "gru_bwd_kernel", "node_init_fwd_kernel", "gate_extract_kernel", "mean_pool_kernel",
+    for k in ("gru_fwd_kernel", "gru_bwd_hn_kernel", "node_init_fwd_kernel", "gate_extract_kernel", "mean_pool_kernel",
               "pool_bwd_fill_kernel", "reduce_parts_kernel", "colsum_reduce_kernel", "gather_partials_kernel",
               "spmm_gather_kernel"):
         if k in name:
