@@ -50,7 +50,7 @@ size_t ltgnn_last_error(char* buf, size_t cap);
 /* Device-resident dropout seed, for CUDA-graph capture of a TRAINING step (the reference draws fresh dropout masks on
  * every call of train_detector.py:310; a captured launch would otherwise replay the drop_seed it was captured with).
  * After ltgnn_seed_source(w), every dropout-bearing launch made FROM THE CALLING THREAD (ltgnn_node_init_fwd,
- * ltgnn_gcn_layer_fwd, ltgnn_spmm_fused, ltgnn_pipe_head_fwd) keys its random stream with drop_seed + *w, where the
+ * ltgnn_gcn_layer_fwd, ltgnn_spmm_fused, ltgnn_pipe_head_fwd, ltgnn_tcn_conv_train, ltgnn_gru_dropout) keys its random stream with drop_seed + *w, where the
  * 64-bit device word *w is read when the kernel runs: bump it between replays (on the stream) and every replay draws
  * new masks.  ltgnn_seed_source(NULL) (the default) restores drop_seed alone.  The word must outlive the launches. */
 void ltgnn_seed_source(const uint64_t* dev_word);
@@ -318,6 +318,34 @@ int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int32_t F, int3
  */
 int ltgnn_gru_layer_fwd(int device, int64_t Q, int32_t L, int32_t H, const float* gx, const float* w_hh, const float* b_hn,
                         float* hseq, float* h_last, void* stream);
+
+/* ---- training of the GRU normal-state predictor (predictor.py:84-111, train_predictor.py), same file ----------------
+ * gru_layer_fwd_train: ltgnn_gru_layer_fwd (same kernel, same h_last and hseq bit for bit) that also stores every step's
+ *   gates [4][Q*L][H] = r | z | n | hn, hn = W_hn h_{t-1} + b_hn, in gx's planar layout.  hseq and gates are required.
+ * gru_layer_bwd: back-propagation through time of one layer from what gru_layer_fwd_train saved.  dh_last [Q, H] is the
+ *   gradient of h_last (the top layer's, from the head) and dh_seq [Q*L, H] the gradient of every state (a lower layer's,
+ *   from the layer above; its row L-1 covers h_last); either may be NULL, not both.  Writes
+ *   dG [4][Q*L][H] = dr_pre | dz_pre | dn_pre | dhn (gradients of the r, z pre-activations, of gx_n and of hn), from which
+ *   the weight gradients are ltgnn_wgrad_tc products: dW_hh rows r, z, n = planes 0, 1, 3 against h_{t-1}, dW_ih rows
+ *   r, z, n = planes 0, 1, 2 against the layer input.  Clusters of 4 CTAs: each multiplies its own 96 gate columns by its
+ *   96 x 128 slice of W_hh (3xTF32 tcgen05) and sends its peers their 32-column blocks of the partial through distributed
+ *   shared memory; the owner adds the four partials in rank order.  Deterministic, capturable into a CUDA graph.
+ * gru_dropout: the inter-layer dropout of nn.GRU in train mode, y [M, H] = x * keep / (1 - drop_p), keep from Philox keyed
+ *   by drop_seed (+ the ltgnn_seed_source word); live uint32 [M, H/32]: bit b of word w = unit 32 (w % (H/32)) + b kept.
+ *   drop_p = 0 copies x bit for bit (every bit set).
+ * gru_dropout_bwd: dx [M, H] = (dy[0] + ... + dy[n_parts - 1]) * keep / (1 - drop_p), dy [n_parts][M][H] added in index
+ *   order (the input gradient of the layer above, one part per gate group), keep read from live (NULL: no dropout).
+ * All four: H = 128 only (else LTGNN_E_SHAPE); Q, L, M > 0, drop_p in [0, 1), 1 <= n_parts <= 4 and the required tensors
+ * non-NULL (else LTGNN_E_ARG); tensors 16-byte aligned (else LTGNN_E_ALIGN); sm_100 (else LTGNN_E_UNSUPPORTED).
+ */
+int ltgnn_gru_layer_fwd_train(int device, int64_t Q, int32_t L, int32_t H, const float* gx, const float* w_hh,
+                              const float* b_hn, float* hseq, float* h_last, float* gates, void* stream);
+int ltgnn_gru_layer_bwd(int device, int64_t Q, int32_t L, int32_t H, const float* w_hh, const float* gates,
+                        const float* hseq, const float* dh_last, const float* dh_seq, float* dG, void* stream);
+int ltgnn_gru_dropout(int device, int64_t M, int32_t H, const float* x, float drop_p, uint64_t drop_seed, float* y,
+                      uint32_t* live, void* stream);
+int ltgnn_gru_dropout_bwd(int device, int64_t M, int32_t H, const float* dy, int32_t n_parts, const uint32_t* live,
+                          float drop_p, float* dx, void* stream);
 
 #ifdef __cplusplus
 }

@@ -1,5 +1,6 @@
-// gru_pred.cu -- one layer of the GRU normal-state predictor (reference models/predictor.py:84-111) at hidden 128,
-// forward only: the frozen predictor's recurrence on the residual builder's windows.
+// gru_pred.cu -- one layer of the GRU normal-state predictor (reference models/predictor.py:84-111) at hidden 128:
+// the frozen predictor's recurrence on the residual builder's windows, and its training (saved-gates forward, backward
+// through time, inter-layer dropout).
 //
 // torch.nn.GRU equations and gate order (r, z, n), h_0 = 0:
 //   r = sigma(gx_r + W_hr h),  z = sigma(gx_z + W_hz h),  n = tanh(gx_n + r * (W_hn h + b_hn)),  h' = (1 - z) n + z h
@@ -26,6 +27,8 @@ using namespace ltgnn::ptx;
 using namespace ltgnn::umma;
 using ltgnn::rowgemm_ts::mma_tf32_ts;
 using ltgnn::rowgemm_ts::tmem_wait_st;
+using ltgnn::ptx::launch_seed;
+using ltgnn::ptx::philox4x32_7;
 
 namespace {
 
@@ -52,6 +55,7 @@ struct GruLayerParams {
     uint32_t Q;
     int L;
     size_t plane;       // Q * L * H: floats per gate group of gx
+    float* gates;       // training forward: [4][Q * L][H] = r | z | n | hn (hn = W_hn h_{t-1} + b_hn)
 };
 
 // same fast forms as the sensor GRU (gru.cu)
@@ -84,6 +88,8 @@ __device__ __forceinline__ void split16_store(uint32_t t_hi, uint32_t t_lo, cons
     tmem_st16(t_lo, lo);
 }
 
+// kTrain: also store every step's r, z, n and hn for the backward (hseq is then required)
+template <bool kTrain>
 __global__ void __launch_bounds__(kThreads, 1)
 gru_layer_fwd_kernel(const GruLayerParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -183,6 +189,21 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
                 const float zg = sigmoidf_fast(gz[j] + zz[j]);
                 const float n = tanhf_fast(fmaf(rg, hn[j] + bhn[j], gn[j]));
                 h[j] = fmaf(zg, h[j] - n, n);  // (1 - z) n + z h
+                if constexpr (kTrain) {
+                    rr[j] = rg;
+                    zz[j] = zg;
+                    gn[j] = n;
+                    hn[j] += bhn[j];
+                }
+            }
+            if constexpr (kTrain) {
+                if (valid) {
+                    float* g = p.gates + (row0 + t) * H + u0;
+                    store16(g, rr);
+                    store16(g + p.plane, zz);
+                    store16(g + 2 * p.plane, gn);
+                    store16(g + 3 * p.plane, hn);
+                }
             }
             if (t + 1 < L) load_gx(t + 1);  // in flight through the exchange and the next step's MMAs
             if (valid && p.hseq) store16(p.hseq + (row0 + t) * H + u0, h);
@@ -267,6 +288,288 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
     }
 }
 
+
+// =====================================================================================================
+// backward through time of one layer, from the gates r | z | n | hn and the states the training forward saved.  Per step
+// t = L-1 .. 0, with dh = d loss / d h_t (the carried gradient plus dh_seq[t], the gradient from the layer above):
+//   dn_pre = dh (1 - z)(1 - n^2);  dz_pre = dh (h_{t-1} - n) z (1 - z);  dr_pre = dn_pre hn r (1 - r);  dhn = dn_pre r
+//   dG(t) = [dr_pre | dz_pre | dn_pre | dhn]  -> HBM, planar, for the weight gradients (ltgnn_wgrad_tc)
+//   dh_{t-1} = dh z + [dr_pre | dz_pre | dhn] [W_hr; W_hz; W_hn]
+// The cluster shape is the forward's: CTA `rank` owns hidden units [32 rank, +32) and holds the 96 x 128 slice of W_hh
+// of their r, z and hn rows, transposed to K-major (B[n = h column][k = 32 g + unit]), hi / lo in 96 KiB of shared memory.
+// Its 96 gate columns (hi | lo, 192 tensor-memory columns) times that slice give a 128 x 128 PARTIAL of the contraction
+// over the 3H gate rows (12 K-steps x 3 tcgen05.mma).  Each CTA sends the three 32-column blocks that belong to its peers
+// into their double-buffered receive space (3 x 16 KiB per step, the forward's scheme); after one cluster barrier the
+// owner adds the four partials in rank order.  Shared memory 192 KiB + alignment; tensor memory 320 of 512 columns.
+// No atomics, fixed order: bitwise deterministic.
+// =====================================================================================================
+constexpr uint32_t kBwAccCol = 0, kBwAhiCol = H, kBwAloCol = H + NB;  // 128 | 96 | 96
+
+struct GruLayerBwdParams {
+    const float* w_hh;     // [3H, H]
+    const float* gates;    // [4][Q * L][H]: r | z | n | hn
+    const float* hseq;     // [Q * L][H]
+    const float* dh_last;  // [Q, H] or nullptr
+    const float* dh_seq;   // [Q * L][H] or nullptr
+    float* dG;             // [4][Q * L][H]: dr_pre | dz_pre | dn_pre | dhn
+    uint32_t Q;
+    int L;
+    size_t plane;          // Q * L * H
+};
+
+__global__ void __launch_bounds__(kThreads, 1)
+gru_layer_bwd_kernel(const GruLayerBwdParams p) {
+    extern __shared__ uint8_t smem_raw[];
+    __shared__ uint64_t bar_a, bar_d;
+    __shared__ uint32_t tmem_base_s;
+    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* b_hi = smem;                 // B[n][k] = w_hh[g H + 32 rank + u][n], k = 32 g + u: three k-atoms, one per gate
+    uint8_t* b_lo = b_hi + kBBytes;
+    uint8_t* recv = b_lo + kBBytes;       // [2 parity][3 slots][8 float4 columns][128 rows] float4
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const uint32_t rank = cluster_ctarank();
+    const uint32_t tile = blockIdx.x / kCluster;
+    if (warp == kMmaWarp) tmem_alloc(&tmem_base_s, 512);
+    if (tid == 0) {
+        mbar_init(&bar_a, kGateWarps);
+        mbar_init(&bar_d, 1);
+        fence_mbar_init();
+    }
+    for (int i = tid; i < NB * H; i += kThreads) {
+        const int k = i / H, n = i - k * H;  // consecutive threads read consecutive columns of one W_hh row
+        const int row = (k / kUnits) * H + kUnits * static_cast<int>(rank) + (k % kUnits);
+        const float w = __ldg(p.w_hh + static_cast<size_t>(row) * H + n);
+        const float hi = tf32_hi(w), lo = w - hi;
+        const uint32_t off = sw128_offset(n, k >> 2, H) + (k & 3) * 4;
+        *reinterpret_cast<float*>(b_hi + off) = hi;
+        *reinterpret_cast<float*>(b_lo + off) = lo;
+    }
+    fence_proxy_async_smem();
+    fence_before_sync();
+    __syncthreads();
+    fence_after_sync();
+    cluster_sync();  // every peer is running (its receive buffer exists) before the first remote store
+    const uint32_t tmem = tmem_base_s;
+    const int L = p.L;
+
+    if (warp < kGateWarps) {
+        // warp (quad, half): TMEM lanes / sequences 32 quad .. +31, units u0 = 32 rank + 16 half .. +15
+        const int quad = warp & 3, half = warp >> 2;
+        const uint32_t lane_off = static_cast<uint32_t>(quad * 32) << 16;
+        const int r = quad * 32 + lane;
+        const uint32_t q = tile * 128 + r;
+        const bool valid = q < p.Q;
+        const int u0 = kUnits * static_cast<int>(rank) + 16 * half;
+        const size_t row0 = static_cast<size_t>(valid ? q : 0) * L;
+        float dh[16], gr[16], gz[16], gn[16], ghn[16], hm[16];
+        auto zero16 = [](float* v) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) v[j] = 0.f;
+        };
+        if (valid && p.dh_last) load16(p.dh_last + static_cast<size_t>(q) * H + u0, dh);
+        else zero16(dh);
+        auto load_step = [&](int t) {  // saved gates and h_{t-1} (zero at t = 0); zeros for pad rows
+            if (valid) {
+                const float* g = p.gates + (row0 + t) * H + u0;
+                load16(g, gr);
+                load16(g + p.plane, gz);
+                load16(g + 2 * p.plane, gn);
+                load16(g + 3 * p.plane, ghn);
+                if (t > 0) load16(p.hseq + (row0 + t - 1) * H + u0, hm);
+                else zero16(hm);
+            } else {
+                zero16(gr); zero16(gz); zero16(gn); zero16(ghn); zero16(hm);
+            }
+        };
+        // the gradient from the layer above, dh_seq[t], joins the carried gradient before step t (its load is issued
+        // while the previous step's MMAs run)
+        const bool seq = valid && p.dh_seq;
+        auto add_seq = [&](const float* ds) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) dh[j] += ds[j];
+        };
+        if (seq) {
+            float ds[16];
+            load16(p.dh_seq + (row0 + L - 1) * H + u0, ds);
+            add_seq(ds);
+        }
+        load_step(L - 1);
+        const uint32_t recv_s = smem_u32(recv);
+        uint32_t ph = 0;
+        for (int t = L - 1; t >= 0; --t) {
+            // in place: gr <- dr_pre, gz <- dz_pre, gn <- dn_pre, ghn <- dhn, dh <- dh z
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const float g = dh[j];
+                const float rg = gr[j], zg = gz[j], n = gn[j];
+                const float dnp = g * (1.f - zg) * (1.f - n * n);
+                gz[j] = g * (hm[j] - n) * zg * (1.f - zg);
+                gr[j] = dnp * ghn[j] * rg * (1.f - rg);
+                ghn[j] = dnp * rg;
+                gn[j] = dnp;
+                dh[j] = g * zg;
+            }
+            if (valid) {
+                float* d = p.dG + (row0 + t) * H + u0;
+                store16(d, gr);
+                store16(d + p.plane, gz);
+                store16(d + 2 * p.plane, gn);
+                store16(d + 3 * p.plane, ghn);
+            }
+            if (t == 0) break;  // dh_{-1} is not needed
+            // A = this CTA's 96 gate columns [dr | dz | dhn] of its 32 units; the previous step's MMAs have completed
+            // (their commit was waited for below), so the columns are free
+            split16_store(tmem + lane_off + kBwAhiCol + 16 * half, tmem + lane_off + kBwAloCol + 16 * half, gr);
+            split16_store(tmem + lane_off + kBwAhiCol + kUnits + 16 * half, tmem + lane_off + kBwAloCol + kUnits + 16 * half, gz);
+            split16_store(tmem + lane_off + kBwAhiCol + 2 * kUnits + 16 * half,
+                          tmem + lane_off + kBwAloCol + 2 * kUnits + 16 * half, ghn);
+            tmem_wait_st();
+            fence_before_sync();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&bar_a);
+            float ds[16];
+            if (seq) load16(p.dh_seq + (row0 + t - 1) * H + u0, ds);
+            mbar_wait(&bar_d, ph);
+            fence_after_sync();
+            // 1. the peers' 32-column blocks of the partial into their receive space (slot of "from rank", as the forward)
+            const uint32_t par_off = static_cast<uint32_t>(t & 1) * (kCluster - 1) * kSlotBytes;
+#pragma unroll
+            for (uint32_t k = 1; k < kCluster; ++k) {
+                const uint32_t dst = (rank + k) & (kCluster - 1);
+                float v[16];
+                tmem_ld16(tmem + lane_off + kBwAccCol + kUnits * dst + 16 * half, v);
+                const uint32_t base = mapa_shared(recv_s + par_off + (kCluster - 1 - k) * kSlotBytes, dst);
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    st_cluster_v4(base + ((4 * half + j) * 128 + r) * 16,
+                                  make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]));
+            }
+            if (seq) add_seq(ds);  // dh_{t-1} = (dh_t z + dh_seq[t-1]) + partial 0 + 1 + 2 + 3, in this order
+            load_step(t - 1);      // in flight through the cluster barrier
+            __syncwarp();      // the cluster barrier is warp-collective (.aligned)
+            cluster_arrive();
+            cluster_wait();
+            // 2. the four partials of this thread's units, added to dh in rank order; the own one is still in the accumulator
+            // (the next MMA waits for this step's bar_a arrival), so it is not held in registers across the barrier
+#pragma unroll
+            for (uint32_t c = 0; c < kCluster; ++c) {
+                float v[16];
+                if (c == rank) {
+                    tmem_ld16(tmem + lane_off + kBwAccCol + kUnits * rank + 16 * half, v);
+                } else {
+                    const uint32_t s = (c - rank - 1) & (kCluster - 1);  // slot s holds CTA (rank + s + 1)'s partial
+                    const float4* in = reinterpret_cast<const float4*>(recv + par_off + s * kSlotBytes);
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        const float4 a = in[(4 * half + j) * 128 + r];
+                        v[4 * j] = a.x; v[4 * j + 1] = a.y; v[4 * j + 2] = a.z; v[4 * j + 3] = a.w;
+                    }
+                }
+#pragma unroll
+                for (int j = 0; j < 16; ++j) dh[j] += v[j];
+            }
+            ph ^= 1;
+        }
+    } else {
+        // ------------------------------- MMA issuer -------------------------------
+        const uint32_t idesc = idesc_tf32(128, H);
+        const uint32_t bh = desc_lo(smem_u32(b_hi)), bl = desc_lo(smem_u32(b_lo));
+        constexpr uint32_t kg_units = H * 128u >> 4;  // one 32-column k-atom block of B (128 rows x 128 B)
+        uint32_t ph = 0;
+        for (int t = L - 1; t > 0; --t) {
+            mbar_wait(&bar_a, ph);
+            ph ^= 1;
+            fence_after_sync();
+            if (elect_one()) {
+#pragma unroll
+                for (uint32_t ks = 0; ks < NB / 8; ++ks) {
+                    const uint32_t boff = (ks >> 2) * kg_units + 2 * (ks & 3);
+                    mma_tf32_ts(tmem + kBwAccCol, tmem + kBwAloCol + 8 * ks, bh + boff, idesc, ks == 0 ? 0u : 1u);
+                    mma_tf32_ts(tmem + kBwAccCol, tmem + kBwAhiCol + 8 * ks, bl + boff, idesc, 1u);
+                    mma_tf32_ts(tmem + kBwAccCol, tmem + kBwAhiCol + 8 * ks, bh + boff, idesc, 1u);
+                }
+                commit(&bar_d);
+            }
+            __syncwarp();
+            cluster_sync();  // the gate warps' per-step barrier counts every thread of the cluster
+        }
+    }
+    fence_before_sync();
+    __syncthreads();
+    cluster_sync();  // no CTA leaves while a peer could still address its shared memory
+    if (warp == kMmaWarp) {
+        fence_after_sync();
+        tmem_dealloc(tmem, 512);
+    }
+}
+
+// ---- inter-layer dropout (nn.GRU applies it to every layer's output but the last, in train mode), off the recurrence.
+// Thread = one 32-unit word of a row: y = x * keep / (1 - p) with Philox (launch seed + ltgnn_seed_source word), bit b
+// of live[word] = unit 32 (word % 4) + b kept.  p = 0 copies x bit for bit.
+__global__ void __launch_bounds__(256)
+gru_dropout_kernel(const float4* __restrict__ x, uint32_t thresh, float keep_scale, uint64_t drop_seed,
+                   const uint64_t* seed_src, float4* __restrict__ y, uint32_t* __restrict__ live, uint32_t n_words) {
+    const uint32_t w = blockIdx.x * 256 + threadIdx.x;
+    if (w >= n_words) return;
+    const uint64_t seed = thresh ? launch_seed(drop_seed, seed_src) : 0;
+    uint32_t bits = thresh ? 0u : ~0u;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const uint64_t idx4 = static_cast<uint64_t>(w) * 8 + j;
+        float4 v = ldg_stream(x + idx4);
+        if (thresh) {
+            const uint4 rv = philox4x32_7(static_cast<uint32_t>(idx4), static_cast<uint32_t>(idx4 >> 32),
+                                          static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32));
+            const bool k0 = rv.x >= thresh, k1 = rv.y >= thresh, k2 = rv.z >= thresh, k3 = rv.w >= thresh;
+            v.x = k0 ? v.x * keep_scale : 0.f;
+            v.y = k1 ? v.y * keep_scale : 0.f;
+            v.z = k2 ? v.z * keep_scale : 0.f;
+            v.w = k3 ? v.w * keep_scale : 0.f;
+            bits |= (static_cast<uint32_t>(k0) | static_cast<uint32_t>(k1) << 1 | static_cast<uint32_t>(k2) << 2 |
+                     static_cast<uint32_t>(k3) << 3) << (4 * j);
+        }
+        stg_stream(y + idx4, v);
+    }
+    live[w] = bits;
+}
+
+// dx = (dy[0] + dy[1] + ...) * (live ? keep / (1 - p) : 1), the parts added in index order
+__global__ void __launch_bounds__(256)
+gru_dropout_bwd_kernel(const float4* __restrict__ dy, int n_parts, size_t plane4, const uint32_t* __restrict__ live,
+                       float keep_scale, float4* __restrict__ dx, uint32_t n_words) {
+    const uint32_t w = blockIdx.x * 256 + threadIdx.x;
+    if (w >= n_words) return;
+    const uint32_t bits = live ? __ldg(live + w) : ~0u;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const size_t idx4 = static_cast<size_t>(w) * 8 + j;
+        float4 s = ldg_stream(dy + idx4);
+        for (int k = 1; k < n_parts; ++k) {
+            const float4 a = ldg_stream(dy + k * plane4 + idx4);
+            s.x += a.x; s.y += a.y; s.z += a.z; s.w += a.w;
+        }
+        if (live) {
+            const uint32_t nib = bits >> (4 * j);
+            s.x = nib & 1u ? s.x * keep_scale : 0.f;
+            s.y = nib & 2u ? s.y * keep_scale : 0.f;
+            s.z = nib & 4u ? s.z * keep_scale : 0.f;
+            s.w = nib & 8u ? s.w * keep_scale : 0.f;
+        }
+        stg_stream(dx + idx4, s);
+    }
+}
+
+// the device and shape checks every entry point of this file makes
+int check_device(int device, const char* fn) {
+    const DeviceInfo* di = device_info(device);
+    if (!di) return LTGNN_E_CUDA;
+    LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "%s: device is sm_%d%d, need sm_100", fn, di->cc_major,
+                  di->cc_minor);
+    LTGNN_REQUIRE(kSmem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "%s: %zu B of shared memory", fn, kSmem);
+    return LTGNN_OK;
+}
+
 }  // namespace
 
 extern "C" int ltgnn_gru_layer_fwd(int device, int64_t Q, int32_t L, int32_t Hdim, const float* gx, const float* w_hh,
@@ -283,11 +586,89 @@ extern "C" int ltgnn_gru_layer_fwd(int device, int64_t Q, int32_t L, int32_t Hdi
                   di->cc_minor);
     LTGNN_REQUIRE(kSmem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "gru_layer_fwd: %zu B of shared memory", kSmem);
     LTGNN_USE_DEVICE(device);
-    GruLayerParams p{gx, w_hh, b_hn, hseq, h_last, static_cast<uint32_t>(Q), L, static_cast<size_t>(Q) * L * H};
-    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_layer_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmem)));
+    GruLayerParams p{gx, w_hh, b_hn, hseq, h_last, static_cast<uint32_t>(Q), L, static_cast<size_t>(Q) * L * H, nullptr};
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_layer_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmem)));
     const int64_t tiles = (Q + 127) / 128;
-    LTGNN_CUDA_TRY(launch_cluster(gru_layer_fwd_kernel, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
+    LTGNN_CUDA_TRY(launch_cluster(gru_layer_fwd_kernel<false>, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
                                   static_cast<cudaStream_t>(stream_), kCluster, p));
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_layer_fwd_train(int device, int64_t Q, int32_t L, int32_t Hdim, const float* gx, const float* w_hh,
+                                         const float* b_hn, float* hseq, float* h_last, float* gates, void* stream_) {
+    LTGNN_REQUIRE(Q > 0 && L > 0, LTGNN_E_ARG, "gru_layer_fwd_train: Q=%lld L=%d", static_cast<long long>(Q), L);
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_layer_fwd_train: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(Q < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_layer_fwd_train: too many sequences");
+    LTGNN_REQUIRE(gx && w_hh && b_hn && hseq && h_last && gates, LTGNN_E_ARG, "gru_layer_fwd_train: null tensor");
+    LTGNN_REQUIRE(aligned16(gx) && aligned16(w_hh) && aligned16(hseq) && aligned16(h_last) && aligned16(gates), LTGNN_E_ALIGN,
+                  "gru_layer_fwd_train: gx, w_hh, hseq, h_last and gates must be 16-byte aligned");
+    if (int rc = check_device(device, "gru_layer_fwd_train")) return rc;
+    LTGNN_USE_DEVICE(device);
+    GruLayerParams p{gx, w_hh, b_hn, hseq, h_last, static_cast<uint32_t>(Q), L, static_cast<size_t>(Q) * L * H, gates};
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_layer_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmem)));
+    const int64_t tiles = (Q + 127) / 128;
+    LTGNN_CUDA_TRY(launch_cluster(gru_layer_fwd_kernel<true>, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
+                                  static_cast<cudaStream_t>(stream_), kCluster, p));
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_layer_bwd(int device, int64_t Q, int32_t L, int32_t Hdim, const float* w_hh, const float* gates,
+                                   const float* hseq, const float* dh_last, const float* dh_seq, float* dG, void* stream_) {
+    LTGNN_REQUIRE(Q > 0 && L > 0, LTGNN_E_ARG, "gru_layer_bwd: Q=%lld L=%d", static_cast<long long>(Q), L);
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_layer_bwd: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(Q < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_layer_bwd: too many sequences");
+    LTGNN_REQUIRE(w_hh && gates && hseq && dG && (dh_last || dh_seq), LTGNN_E_ARG,
+                  "gru_layer_bwd: null tensor (dh_last and dh_seq may not both be NULL)");
+    LTGNN_REQUIRE(aligned16(w_hh) && aligned16(gates) && aligned16(hseq) && aligned16(dh_last) && aligned16(dh_seq) &&
+                  aligned16(dG), LTGNN_E_ALIGN, "gru_layer_bwd: every tensor must be 16-byte aligned");
+    if (int rc = check_device(device, "gru_layer_bwd")) return rc;
+    LTGNN_USE_DEVICE(device);
+    GruLayerBwdParams p{w_hh, gates, hseq, dh_last, dh_seq, dG, static_cast<uint32_t>(Q), L, static_cast<size_t>(Q) * L * H};
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_layer_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmem)));
+    const int64_t tiles = (Q + 127) / 128;
+    LTGNN_CUDA_TRY(launch_cluster(gru_layer_bwd_kernel, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
+                                  static_cast<cudaStream_t>(stream_), kCluster, p));
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_dropout(int device, int64_t M, int32_t Hdim, const float* x, float drop_p, uint64_t drop_seed,
+                                 float* y, uint32_t* live, void* stream_) {
+    LTGNN_REQUIRE(M > 0 && M < (1ll << 31), LTGNN_E_ARG, "gru_dropout: M=%lld", static_cast<long long>(M));
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_dropout: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(drop_p >= 0.f && drop_p < 1.f, LTGNN_E_ARG, "gru_dropout: drop_p=%g", static_cast<double>(drop_p));
+    LTGNN_REQUIRE(x && y && live, LTGNN_E_ARG, "gru_dropout: null tensor");
+    LTGNN_REQUIRE(aligned16(x) && aligned16(y) && aligned16(live), LTGNN_E_ALIGN, "gru_dropout: 16-byte alignment");
+    if (int rc = check_device(device, "gru_dropout")) return rc;
+    LTGNN_USE_DEVICE(device);
+    const double t = static_cast<double>(drop_p) * 4294967296.0;
+    const uint32_t thresh = drop_p > 0.f ? static_cast<uint32_t>(t < 4294967295.0 ? t : 4294967295.0) : 0u;
+    const float keep_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
+    const uint32_t n_words = static_cast<uint32_t>(M * (H / 32));
+    gru_dropout_kernel<<<(n_words + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream_)>>>(
+        reinterpret_cast<const float4*>(x), thresh, keep_scale, drop_seed, seed_source(), reinterpret_cast<float4*>(y), live,
+        n_words);
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_dropout_bwd(int device, int64_t M, int32_t Hdim, const float* dy, int32_t n_parts,
+                                     const uint32_t* live, float drop_p, float* dx, void* stream_) {
+    LTGNN_REQUIRE(M > 0 && M < (1ll << 31), LTGNN_E_ARG, "gru_dropout_bwd: M=%lld", static_cast<long long>(M));
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_dropout_bwd: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(n_parts >= 1 && n_parts <= 4, LTGNN_E_ARG, "gru_dropout_bwd: n_parts=%d", n_parts);
+    LTGNN_REQUIRE(drop_p >= 0.f && drop_p < 1.f, LTGNN_E_ARG, "gru_dropout_bwd: drop_p=%g", static_cast<double>(drop_p));
+    LTGNN_REQUIRE(dy && dx, LTGNN_E_ARG, "gru_dropout_bwd: null tensor");
+    LTGNN_REQUIRE(aligned16(dy) && aligned16(dx) && aligned16(live), LTGNN_E_ALIGN, "gru_dropout_bwd: 16-byte alignment");
+    if (int rc = check_device(device, "gru_dropout_bwd")) return rc;
+    LTGNN_USE_DEVICE(device);
+    const float keep_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
+    const uint32_t n_words = static_cast<uint32_t>(M * (H / 32));
+    gru_dropout_bwd_kernel<<<(n_words + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream_)>>>(
+        reinterpret_cast<const float4*>(dy), n_parts, static_cast<size_t>(M) * (H / 4), live, keep_scale,
+        reinterpret_cast<float4*>(dx), n_words);
     LTGNN_CUDA_TRY(cudaGetLastError());
     return LTGNN_OK;
 }

@@ -87,6 +87,12 @@ SIGNATURES = {
                                 c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_layer_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_void_p]),
+    "ltgnn_gru_layer_fwd_train": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
+                                          c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gru_layer_bwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p]),
+    "ltgnn_gru_dropout": (c_int, [c_int, c_int64, c_int32, c_void_p, c_float, c_uint64, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gru_dropout_bwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_int32, c_void_p, c_float, c_void_p, c_void_p]),
 }
 
 _lib = None

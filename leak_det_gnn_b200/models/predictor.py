@@ -260,7 +260,8 @@ class NormalPredictorTCN(nn.Module):
 
 class NormalPredictorGRU(nn.Module):
     """Two-layer GRU baseline (predictor.py:84-111).  ``forward`` is the reference's (cuDNN); ``forward_last`` is the
-    frozen predictor's inference path, on the sm_100a kernels at hidden 128 (csrc/gru_pred.cu + csrc/linear.cu)."""
+    frozen predictor's inference path and ``forward_cone`` its differentiable training path, both on the sm_100a kernels
+    at hidden 128 (csrc/gru_pred.cu + csrc/linear.cu + csrc/wgrad.cu)."""
 
     def __init__(self, num_sensors: int, time_dim: int = 9, hidden_size: int = 128, num_layers: int = 2,
                  dropout: float = 0.1) -> None:
@@ -275,8 +276,8 @@ class NormalPredictorGRU(nn.Module):
         out, _ = self.gru(torch.cat([x, x_time], dim=-1))
         return self.head(out[:, -1, :])
 
-    # use the hand-written sm_100a kernels for ``forward_last`` on CUDA where the shapes allow; False = the dense cuDNN
-    # ``forward``, kept as the cross-check
+    # use the hand-written sm_100a kernels for ``forward_last`` and ``forward_cone`` on CUDA where the shapes allow;
+    # False = the dense cuDNN ``forward``, kept as the cross-check
     use_native = True
 
     def _native_ok(self, x: torch.Tensor) -> bool:
@@ -297,6 +298,23 @@ class NormalPredictorGRU(nn.Module):
         prep = self._native_weights(x.device)
         h = ops.gru_predictor_fwd(x, x_time, prep["layers"])
         return ops.linear_tc(h, prep["w_out"], prep["b_out"])[:, :self.num_sensors]
+
+    def forward_cone(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
+        """``forward``'s result, differentiable in train and eval mode, with the module's inter-layer dropout in train mode.
+        The name is the TCN predictor's: for a GRU the last step's dependency cone is the whole sequence, and
+        ``train_predictor_dp`` trains either model through it.  On CUDA at the shapes ``_native_ok`` accepts this is ONE
+        autograd node on the sm_100a kernels (``ops.gru_predictor_cone``); otherwise the dense ``forward``."""
+        if not self._native_ok(x):
+            return self.forward(x, x_time)
+        from .. import ops
+
+        g = self.gru
+        params = []
+        for i in range(g.num_layers):
+            params += [getattr(g, f"weight_ih_l{i}"), getattr(g, f"weight_hh_l{i}"), getattr(g, f"bias_ih_l{i}"),
+                       getattr(g, f"bias_hh_l{i}")]
+        return ops.gru_predictor_cone(x, x_time, g.dropout if self.training else 0.0,
+                                      params + [self.head.weight, self.head.bias])
 
     def _native_weights(self, device):
         """Weights in the kernels' layouts, rebuilt when a parameter changes (the predictor is frozen in practice)."""

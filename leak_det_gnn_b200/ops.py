@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -933,6 +933,201 @@ def gru_predictor_fwd(x: torch.Tensor, x_time: torch.Tensor, layers) -> torch.Te
         h_last, inp = gru_layer_fwd(inp, q, l, layer, seq=i + 1 < len(layers))
     return h_last
 
+
+
+# ----------------------------------------------------------------------------------------------
+# training of the GRU normal-state predictor (csrc/gru_pred.cu): saved-gates forward, BPTT, inter-layer dropout
+# ----------------------------------------------------------------------------------------------
+def gru_layer_fwd_train(gx: torch.Tensor, q: int, l: int, w_hh: torch.Tensor, b_hn: torch.Tensor):
+    """Raw training forward of one layer's recurrence (see ltgnn_gru_layer_fwd_train) on a precomputed input projection
+    gx [3, q * l, H].  Returns (h_last (q, H), hseq (q * l, H), gates [4, q * l, H] = r | z | n | hn)."""
+    _check_act(gx, "gx")
+    hdim = w_hh.shape[1]
+    h_last = torch.empty(q, hdim, device=gx.device, dtype=torch.float32)
+    hseq = torch.empty(q * l, hdim, device=gx.device, dtype=torch.float32)
+    gates = torch.empty(4, q * l, hdim, device=gx.device, dtype=torch.float32)
+    L = _lib.load()
+    tok = _inst.begin("gru_pred_layer_train")
+    _lib.check(L.ltgnn_gru_layer_fwd_train(_dev_index(gx), q, l, hdim, gx.data_ptr(), w_hh.data_ptr(), b_hn.data_ptr(),
+                                           hseq.data_ptr(), h_last.data_ptr(), gates.data_ptr(), _stream(gx)))
+    _inst.end(tok)
+    return h_last, hseq, gates
+
+
+def gru_layer_bwd(q: int, l: int, w_hh: torch.Tensor, gates: torch.Tensor, hseq: torch.Tensor,
+                  dh_last: Optional[torch.Tensor] = None, dh_seq: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Raw backward through time of one layer (see ltgnn_gru_layer_bwd): dG [4, q * l, H] = dr_pre | dz_pre | dn_pre | dhn
+    from the gradient of h_last (q, H) and / or of every state (q * l, H)."""
+    for t, nm in ((w_hh, "w_hh"), (gates, "gates"), (hseq, "hseq")):
+        _check_act(t, nm)
+    for t, nm in ((dh_last, "dh_last"), (dh_seq, "dh_seq")):
+        if t is not None:
+            _check_act(t, nm)
+    hdim = w_hh.shape[1]
+    dg = torch.empty(4, q * l, hdim, device=gates.device, dtype=torch.float32)
+    L = _lib.load()
+    tok = _inst.begin("gru_pred_layer_bwd")
+    _lib.check(L.ltgnn_gru_layer_bwd(_dev_index(gates), q, l, hdim, w_hh.data_ptr(), gates.data_ptr(), hseq.data_ptr(),
+                                     None if dh_last is None else dh_last.data_ptr(),
+                                     None if dh_seq is None else dh_seq.data_ptr(), dg.data_ptr(), _stream(gates)))
+    _inst.end(tok)
+    return dg
+
+
+def gru_dropout(x: torch.Tensor, drop_p: float, drop_seed: int):
+    """Raw inter-layer dropout (see ltgnn_gru_dropout): (y, live) with live int32 (M, H / 32), bit b of word w = unit
+    32 w + b kept."""
+    _check_act(x, "x")
+    m, hdim = x.shape
+    y = torch.empty_like(x)
+    live = torch.empty(m, hdim // 32, device=x.device, dtype=torch.int32)
+    L = _lib.load()
+    tok = _inst.begin("gru_dropout")
+    _lib.check(L.ltgnn_gru_dropout(_dev_index(x), m, hdim, x.data_ptr(), float(drop_p), int(drop_seed) & (2**64 - 1),
+                                   y.data_ptr(), live.data_ptr(), _stream(x)))
+    _inst.end(tok)
+    return y, live
+
+
+def gru_dropout_bwd(parts: torch.Tensor, live: Optional[torch.Tensor], drop_p: float) -> torch.Tensor:
+    """Raw backward of the inter-layer dropout (see ltgnn_gru_dropout_bwd): parts [n, M, H] added in order, times the
+    kept mask / (1 - p) (``live = None``: no dropout)."""
+    _check_act(parts, "parts")
+    n, m, hdim = parts.shape
+    dx = torch.empty(m, hdim, device=parts.device, dtype=torch.float32)
+    L = _lib.load()
+    tok = _inst.begin("gru_dropout_bwd")
+    _lib.check(L.ltgnn_gru_dropout_bwd(_dev_index(parts), m, hdim, parts.data_ptr(), n,
+                                       None if live is None else live.data_ptr(), float(drop_p), dx.data_ptr(),
+                                       _stream(parts)))
+    _inst.end(tok)
+    return dx
+
+
+def unpack_gru_live(live: torch.Tensor) -> torch.Tensor:
+    """int32 (M, H / 32) -> bool (M, H): the units ``gru_dropout`` kept (tests and debugging)."""
+    bits = (live.unsqueeze(-1) >> torch.arange(32, device=live.device, dtype=torch.int32)) & 1
+    return bits.reshape(live.shape[0], -1).bool()
+
+
+def _ones_aug(x: torch.Tensor, width: int) -> torch.Tensor:
+    """[x | 1 | 0 ...] with ``width`` columns: the operand whose ones column turns a weight gradient into the bias's."""
+    out = torch.zeros(x.shape[0], width, device=x.device, dtype=torch.float32)
+    out[:, :x.shape[1]] = x
+    out[:, x.shape[1]] = 1.0
+    return out
+
+
+def gru_layer_param_grads(dg: torch.Tensor, hseq: torch.Tensor, x_aug: torch.Tensor, n_in: int, q: int, l: int):
+    """(d weight_ih, d weight_hh, d bias_ih, d bias_hh) of one torch.nn.GRU layer from its dG [4, q * l, H]
+    (``gru_layer_bwd``), its states hseq (q * l, H) and its input with a ones column at ``n_in``, x_aug (q * l, K), K a
+    multiple of 32: six ``wgrad`` products, dG planes r, z, hn against [h_{t-1} | 1 | 0] and r, z, n against x_aug."""
+    hdim = hseq.shape[1]
+    hprev = torch.zeros(q, l, hdim + 32, device=dg.device, dtype=torch.float32)
+    hprev[:, 1:, :hdim] = hseq.view(q, l, hdim)[:, :-1]
+    hprev[:, :, hdim] = 1.0
+    hprev = hprev.view(q * l, hdim + 32)
+    t_r, t_z, t_hn = (wgrad(dg[g], hprev) for g in (0, 1, 3))
+    del hprev
+    u_r, u_z, u_n = (wgrad(dg[g], x_aug) for g in (0, 1, 2))
+    d_w_ih = torch.cat([u_r[:, :n_in], u_z[:, :n_in], u_n[:, :n_in]], dim=0)
+    d_w_hh = torch.cat([t_r[:, :hdim], t_z[:, :hdim], t_hn[:, :hdim]], dim=0)
+    d_b_ih = torch.cat([t_r[:, hdim], t_z[:, hdim], u_n[:, n_in]], dim=0)   # b_hr, b_hz are folded into gx: same sums
+    d_b_hh = torch.cat([t_r[:, hdim], t_z[:, hdim], t_hn[:, hdim]], dim=0)
+    return [d_w_ih, d_w_hh, d_b_ih, d_b_hh]
+
+
+class _GruPredictor(torch.autograd.Function):
+    """The GRU predictor -- every layer and the head on the last step -- as ONE autograd node: gradients for all GRU and
+    head parameters (the inputs are data).
+
+    Forward per layer: input projection (``linear_tc``, b_hr and b_hz folded), the recurrence saving its gates, and for
+    every layer but the last the inter-layer dropout.  Backward per layer, top down: BPTT -> dG; dW_hh and d b_hh from
+    planes r, z, hn against [h_{t-1} | 1 | 0]; dW_ih and d b_ih (n) from planes r, z, n against [input | 1 | 0]; for a
+    lower layer, its state gradient sum_g dG[g] W_ih[g] through the dropout's mask."""
+
+    @staticmethod
+    def forward(ctx, inp, q, l, c_in, n_sensors, drop_p, *params):
+        n_layers = (len(params) - 2) // 4
+        raw = [params[4 * i:4 * i + 4] for i in range(n_layers)]
+        w_head, b_head = params[-2], params[-1]
+        hdim = raw[0][1].shape[1]
+        p = float(drop_p)
+        layers = gru_predictor_weights(raw, k0=inp.shape[1])
+        x, saved, lives = inp, [], []
+        for i, (w_x, b_x, w_hh, b_hn) in enumerate(layers):
+            gx = torch.empty(3, q * l, hdim, device=inp.device, dtype=torch.float32)
+            for g in range(3):
+                linear_tc(x, w_x[g], b_x[g], out=gx[g])
+            h_last, hseq, gates = gru_layer_fwd_train(gx, q, l, w_hh, b_hn)
+            del gx
+            saved.append((x, hseq, gates, w_hh, raw[i][0].detach().view(3, hdim, -1)))
+            if i + 1 < n_layers:
+                live = None
+                if p > 0:
+                    x, live = gru_dropout(hseq, p, new_dropout_seed())
+                else:
+                    x = hseq
+                lives.append(live)
+        if DEBUG_CAPTURE is not None:
+            DEBUG_CAPTURE["gru_lives"] = lives
+        n_pad = (n_sensors + 31) // 32 * 32
+        w_out = torch.zeros(n_pad, hdim, device=inp.device, dtype=torch.float32)
+        w_out[:n_sensors] = w_head
+        b_out = torch.zeros(n_pad, device=inp.device, dtype=torch.float32)
+        b_out[:n_sensors] = b_head
+        pred = linear_tc(h_last, w_out, b_out)[:, :n_sensors]
+        ctx.save_for_backward(h_last, w_out, *[t for layer in saved for t in layer],
+                              *[lv for lv in lives if lv is not None])
+        ctx.q, ctx.l, ctx.c_in, ctx.n_sensors, ctx.n_layers, ctx.p = q, l, c_in, n_sensors, n_layers, p
+        ctx.has_live = [lv is not None for lv in lives]
+        return pred
+
+    @staticmethod
+    def backward(ctx, dpred):
+        h_last, w_out, *rest = ctx.saved_tensors
+        n, q, l, s = ctx.n_layers, ctx.q, ctx.l, ctx.n_sensors
+        saved = [rest[5 * i:5 * i + 5] for i in range(n)]
+        it = iter(rest[5 * n:])
+        lives = [next(it) if has else None for has in ctx.has_live]
+        hdim = h_last.shape[1]
+        bsz = h_last.shape[0]
+        dp = torch.zeros(bsz, 64 if s <= 64 else 128, device=dpred.device, dtype=torch.float32)
+        dp[:, :s] = dpred
+        t_head = wgrad(dp, _ones_aug(h_last, hdim + 32))
+        dh_last = linear_tc(dp[:, :w_out.shape[0]].contiguous(), w_out, transposed=True)
+        dh_seq = None
+        grads = [None] * (4 * n)
+        for i in range(n - 1, -1, -1):
+            x, hseq, gates, w_hh, w_ih3 = saved[i]
+            dg = gru_layer_bwd(q, l, w_hh, gates, hseq, dh_last=dh_last, dh_seq=dh_seq)
+            if i == 0:
+                grads[0:4] = gru_layer_param_grads(dg, hseq, x, ctx.c_in, q, l)   # layer 0's input carries the ones
+            else:
+                grads[4 * i:4 * i + 4] = gru_layer_param_grads(dg, hseq, _ones_aug(x, hdim + 32), hdim, q, l)
+            if i > 0:
+                parts = torch.empty(3, q * l, hdim, device=dg.device, dtype=torch.float32)
+                for g in range(3):
+                    linear_tc(dg[g], w_ih3[g], transposed=True, out=parts[g])
+                dh_seq = gru_dropout_bwd(parts, lives[i - 1], ctx.p)
+                dh_last = None
+            del dg
+        return (None, None, None, None, None, None, *grads, t_head[:s, :hdim].contiguous(), t_head[:s, hdim].contiguous())
+
+
+def gru_predictor_cone(x: torch.Tensor, x_time: torch.Tensor, drop_p: float, params) -> torch.Tensor:
+    """Differentiable prediction (B, S) of the GRU predictor's last step on the sm_100a kernels.  ``params``: per layer
+    weight_ih, weight_hh, bias_ih, bias_hh (torch.nn.GRU), then head.{weight, bias}; ``drop_p``: the inter-layer dropout
+    (0 in eval mode)."""
+    _check_act(x.contiguous(), "x")
+    b, length, s = x.shape
+    c_in = s + x_time.shape[-1]
+    kp = 64 if c_in < 64 else 96           # one zero-weight column for the ones that turn the weight gradient into d bias
+    inp = torch.zeros(b * length, kp, device=x.device, dtype=torch.float32)
+    inp.view(b, length, kp)[:, :, :s] = x
+    inp.view(b, length, kp)[:, :, s:c_in] = x_time
+    inp[:, c_in] = 1.0
+    return _GruPredictor.apply(inp, b, length, c_in, s, float(drop_p), *params)
 
 def tcn_conv(x: torch.Tensor, src: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor,
              gamma: Optional[torch.Tensor] = None, beta: Optional[torch.Tensor] = None, eps: float = 1e-5, relu: bool = True,
