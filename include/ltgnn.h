@@ -285,7 +285,8 @@ int ltgnn_tcn_wgrad(int device, int64_t M, int32_t C, int32_t taps, const float*
 
 /* ---- shared per-sensor GRU encoder (detector.py:28-73; SURVEY 8f rank 2) -----------------------
  * Sequence q = b*S + s has input [r[b,t,s], tf[b,t,0..F)] at step t (the reference's cat([rr, tf]) order);
- * weights in torch.nn.GRU layout (gate order r, z, n): w_ih [3H, 1+F], w_hh [3H, H], b_ih, b_hh [3H].  H = 64.
+ * weights in torch.nn.GRU layout (gate order r, z, n): w_ih [3H, 1+F], w_hh [3H, H], b_ih, b_hh [3H].  H = 64
+ * (H = 128: ltgnn_gru_sensor_fwd below).
  * gru_fwd:       h_last [B*S, H] = hidden state after step L-1 (h_0 = 0).  For training also pass hseq (every state,
  *                logical [L*Qp, H]) and gates (r, z, n; logical [L*Qp, 3H]), Qp = B*S rounded up to 128, both in the
  *                kernels' blocked-32 layout [rows/32][W/4][32][4]; NULL otherwise.
@@ -346,6 +347,27 @@ int ltgnn_gru_dropout(int device, int64_t M, int32_t H, const float* x, float dr
                       uint32_t* live, void* stream);
 int ltgnn_gru_dropout_bwd(int device, int64_t M, int32_t H, const float* dy, int32_t n_parts, const uint32_t* live,
                           float drop_p, float* dx, void* stream);
+
+/* ---- the shared sensor GRU encoder at hidden 128 (detector.py:28-73 with sensor_hidden = 128), same file -------------
+ * gru_sensor_fwd: the cluster recurrence of ltgnn_gru_layer_fwd / _fwd_train with the encoder's input formed in the
+ *   kernel.  Sequence q = b*S + s has input [r[b,t,s], tf[b,t,:]] at step t; the time features are the same for the S
+ *   sensors of a window, so their projection is computed once per (window, step) beforehand (ltgnn_linear):
+ *     tproj [3][B*L][H]: tproj[g][b*L + t] = tf[b,t,:] W_ih[g][:, 1:]^T + b_ih[g], plus b_hh[g] for g = r, z (not n)
+ *   and the gate thread adds w_r[g] * r[b,t,s], w_r [3][H] = W_ih[:, 0] (the residual column).  One call runs the
+ *   sequences q0 .. q0+Q-1 of the B*S (so a caller can run them in slabs); its outputs are those of the planar form for
+ *   these Q sequences, local sequence i = sequence q0 + i: h_last [Q, H]; if hseq is not NULL, hseq [Q*L, H]; if gates is
+ *   not NULL (training: hseq required), gates [4][Q*L][H] = r | z | n | hn, which ltgnn_gru_layer_bwd reads unchanged.
+ *   The weight gradients are the ltgnn_wgrad_tc products of ltgnn_gru_layer_bwd's comment, the layer input being
+ *   [r | tf | 1] per row.  H = 128 only and B*S < 2^31 - 128 (else LTGNN_E_SHAPE); B, L, S, Q > 0, q0 >= 0,
+ *   q0 + Q <= B*S and r, tproj, w_r, w_hh, b_hn, h_last non-NULL (else LTGNN_E_ARG); tproj, w_r, w_hh, hseq, h_last,
+ *   gates 16-byte aligned (else LTGNN_E_ALIGN).  Deterministic, no allocation or host synchronisation: capturable.
+ * gru_resident_tiles: *tiles = how many 128-sequence tiles (4-CTA clusters) of these recurrences the device runs at
+ *   once (cudaOccupancyMaxActiveClusters): one wave.  Callers size their slabs in whole waves.
+ */
+int ltgnn_gru_sensor_fwd(int device, int64_t B, int32_t L, int32_t S, int64_t q0, int64_t Q, int32_t H, const float* r,
+                         const float* tproj, const float* w_r, const float* w_hh, const float* b_hn, float* hseq,
+                         float* h_last, float* gates, void* stream);
+int ltgnn_gru_resident_tiles(int device, int32_t* tiles);
 
 #ifdef __cplusplus
 }

@@ -19,6 +19,8 @@
 //     3 peers (16 KiB per peer per step, double-buffered: 96 KiB of receive space);
 //   * one cluster barrier per step publishes the slices; each CTA then moves what it received into its A columns.
 // Shared memory 192 KiB + alignment; tensor memory 352 of 512 columns.  No atomics, fixed order: bitwise deterministic.
+// The same kernel runs the shared sensor encoder at hidden 128 (kSensor): there the input term is formed in the gate
+// threads from one residual and a time-feature projection shared by the window's sensors (ltgnn_gru_sensor_fwd).
 #include "umma.cuh"
 #include "rowgemm_ts.cuh"
 
@@ -45,6 +47,7 @@ constexpr uint32_t kBBytes = NB * H * 4;                        // one of b_hi /
 constexpr uint32_t kSlotBytes = 128 * kUnits * 4;               // one peer's slice of h: 16 KiB
 constexpr uint32_t kRecvBytes = 2 * (kCluster - 1) * kSlotBytes;  // double-buffered, 3 peers: 96 KiB
 constexpr size_t kSmem = 1024 + 2ull * kBBytes + kRecvBytes;
+constexpr size_t kSensorSmem = kSmem + 3 * H * 4;                // + w_r for the sensor input form
 
 struct GruLayerParams {
     const float* gx;    // [3][Q * L][H]: gate group g of row q * L + t
@@ -56,6 +59,13 @@ struct GruLayerParams {
     int L;
     size_t plane;       // Q * L * H: floats per gate group of gx
     float* gates;       // training forward: [4][Q * L][H] = r | z | n | hn (hn = W_hn h_{t-1} + b_hn)
+    // sensor input form: gx is T [3][B * L][H] (plane tplane) and sequence q = b S + s of the caller's B S sequences reads
+    // gx_g = w_r[g] r[b, t, s] + T[g][b L + t]; local sequence q of this launch is sequence q0 + q of the B S
+    const float* r_in;  // [B, L, S]
+    const float* w_r;   // [3][H]: the residual column of W_ih
+    uint32_t S;
+    uint32_t q0;
+    size_t tplane;      // B * L * H
 };
 
 // same fast forms as the sensor GRU (gru.cu)
@@ -88,8 +98,10 @@ __device__ __forceinline__ void split16_store(uint32_t t_hi, uint32_t t_lo, cons
     tmem_st16(t_lo, lo);
 }
 
-// kTrain: also store every step's r, z, n and hn for the backward (hseq is then required)
-template <bool kTrain>
+// kTrain: also store every step's r, z, n and hn for the backward (hseq is then required).
+// kSensor: the sensor encoder's input form (see GruLayerParams): one residual value and one T row per step instead of a
+// gx row per sequence; every output is the planar form's, row (local q) L + t.
+template <bool kTrain, bool kSensor = false>
 __global__ void __launch_bounds__(kThreads, 1)
 gru_layer_fwd_kernel(const GruLayerParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -99,11 +111,16 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
     uint8_t* b_hi = smem;                 // B[n][k], n = 48 u + 16 g + jj <-> gate g of unit 32 rank + 16 u + jj
     uint8_t* b_lo = b_hi + kBBytes;
     uint8_t* recv = b_lo + kBBytes;       // [2 parity][3 slots][8 float4 columns][128 rows] float4
+                                          // kSensor: then w_r [3][H] (kSensorSmem)
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const uint32_t rank = cluster_ctarank();
     const uint32_t tile = blockIdx.x / kCluster;
     if (warp == kMmaWarp) tmem_alloc(&tmem_base_s, 512);
+    if constexpr (kSensor) {
+        for (int i = tid; i < 3 * H / 4; i += kThreads)
+            reinterpret_cast<float4*>(recv + kRecvBytes)[i] = __ldg(reinterpret_cast<const float4*>(p.w_r) + i);
+    }
     if (tid == 0) {
         mbar_init(&bar_a, kGateWarps);
         mbar_init(&bar_d[0], 1);
@@ -145,12 +162,29 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
         }
         const size_t row0 = static_cast<size_t>(valid ? q : 0) * L;  // gx / hseq row of step 0
         float gr[16], gz[16], gn[16];
+        // sensor form: the T row of step 0 (b L) and the residual of step 0 (b L S + s)
+        float xr = 0.f;
+        size_t trow0 = 0;
+        const float* rsrc = nullptr;
+        if constexpr (kSensor) {
+            const uint32_t qg = p.q0 + (valid ? q : 0), b = qg / p.S;
+            trow0 = static_cast<size_t>(b) * L;
+            rsrc = p.r_in + trow0 * p.S + (qg - b * p.S);
+        }
         auto load_gx = [&](int t) {
             if (valid) {
-                const float* src = p.gx + (row0 + t) * H + u0;
-                load16(src, gr);
-                load16(src + p.plane, gz);
-                load16(src + 2 * p.plane, gn);
+                if constexpr (kSensor) {
+                    const float* src = p.gx + (trow0 + t) * H + u0;
+                    load16(src, gr);
+                    load16(src + p.tplane, gz);
+                    load16(src + 2 * p.tplane, gn);
+                    xr = __ldg(rsrc + static_cast<size_t>(t) * p.S);
+                } else {
+                    const float* src = p.gx + (row0 + t) * H + u0;
+                    load16(src, gr);
+                    load16(src + p.plane, gz);
+                    load16(src + 2 * p.plane, gn);
+                }
             } else {
 #pragma unroll
                 for (int j = 0; j < 16; ++j) gr[j] = gz[j] = gn[j] = 0.f;
@@ -185,6 +219,12 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
             tmem_ld16(tmem + lane_off + kAccCol + kBlk * half + 32, hn);
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
+                if constexpr (kSensor) {  // the input term, formed here so that its loads stay off the critical path
+                    const float* wr = reinterpret_cast<const float*>(recv + kRecvBytes) + u0 + j;  // warp-uniform
+                    gr[j] = fmaf(wr[0], xr, gr[j]);
+                    gz[j] = fmaf(wr[H], xr, gz[j]);
+                    gn[j] = fmaf(wr[2 * H], xr, gn[j]);
+                }
                 const float rg = sigmoidf_fast(gr[j] + rr[j]);
                 const float zg = sigmoidf_fast(gz[j] + zz[j]);
                 const float n = tanhf_fast(fmaf(rg, hn[j] + bhn[j], gn[j]));
@@ -561,12 +601,12 @@ gru_dropout_bwd_kernel(const float4* __restrict__ dy, int n_parts, size_t plane4
 }
 
 // the device and shape checks every entry point of this file makes
-int check_device(int device, const char* fn) {
+int check_device(int device, const char* fn, size_t smem = kSmem) {
     const DeviceInfo* di = device_info(device);
     if (!di) return LTGNN_E_CUDA;
     LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "%s: device is sm_%d%d, need sm_100", fn, di->cc_major,
                   di->cc_minor);
-    LTGNN_REQUIRE(kSmem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "%s: %zu B of shared memory", fn, kSmem);
+    LTGNN_REQUIRE(smem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "%s: %zu B of shared memory", fn, smem);
     return LTGNN_OK;
 }
 
@@ -611,6 +651,54 @@ extern "C" int ltgnn_gru_layer_fwd_train(int device, int64_t Q, int32_t L, int32
     LTGNN_CUDA_TRY(launch_cluster(gru_layer_fwd_kernel<true>, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
                                   static_cast<cudaStream_t>(stream_), kCluster, p));
     LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_sensor_fwd(int device, int64_t B, int32_t L, int32_t S, int64_t q0, int64_t Q, int32_t Hdim,
+                                    const float* r, const float* tproj, const float* w_r, const float* w_hh,
+                                    const float* b_hn, float* hseq, float* h_last, float* gates, void* stream_) {
+    LTGNN_REQUIRE(B > 0 && L > 0 && S > 0 && q0 >= 0 && Q > 0 && q0 + Q <= B * S, LTGNN_E_ARG,
+                  "gru_sensor_fwd: B=%lld L=%d S=%d q0=%lld Q=%lld", static_cast<long long>(B), L, S,
+                  static_cast<long long>(q0), static_cast<long long>(Q));
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_sensor_fwd: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(B * S < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_sensor_fwd: too many sequences");
+    LTGNN_REQUIRE(r && tproj && w_r && w_hh && b_hn && h_last && (hseq || !gates), LTGNN_E_ARG,
+                  "gru_sensor_fwd: null tensor (gates needs hseq)");
+    LTGNN_REQUIRE(aligned16(tproj) && aligned16(w_r) && aligned16(w_hh) && aligned16(hseq) && aligned16(h_last) &&
+                  aligned16(gates), LTGNN_E_ALIGN, "gru_sensor_fwd: tproj, w_r, w_hh, hseq, h_last and gates must be 16-byte aligned");
+    if (int rc = check_device(device, "gru_sensor_fwd", kSensorSmem)) return rc;
+    LTGNN_USE_DEVICE(device);
+    GruLayerParams p{tproj, w_hh, b_hn, hseq, h_last, static_cast<uint32_t>(Q), L, static_cast<size_t>(Q) * L * H, gates,
+                     r, w_r, static_cast<uint32_t>(S), static_cast<uint32_t>(q0), static_cast<size_t>(B) * L * H};
+    auto kernel = gates ? gru_layer_fwd_kernel<true, true> : gru_layer_fwd_kernel<false, true>;
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSensorSmem)));
+    const int64_t tiles = (Q + 127) / 128;
+    LTGNN_CUDA_TRY(launch_cluster(kernel, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSensorSmem,
+                                  static_cast<cudaStream_t>(stream_), kCluster, p));
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_resident_tiles(int device, int32_t* tiles) {
+    LTGNN_REQUIRE(tiles, LTGNN_E_ARG, "gru_resident_tiles: null output");
+    if (int rc = check_device(device, "gru_resident_tiles", kSensorSmem)) return rc;
+    LTGNN_USE_DEVICE(device);
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(gru_layer_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(kSensorSmem)));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(kCluster);
+    cfg.blockDim = dim3(kThreads);
+    cfg.dynamicSmemBytes = kSensorSmem;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = kCluster;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int n = 0;
+    LTGNN_CUDA_TRY(cudaOccupancyMaxActiveClusters(&n, gru_layer_fwd_kernel<true, true>, &cfg));
+    *tiles = n;
     return LTGNN_OK;
 }
 

@@ -259,7 +259,6 @@ int check_common(int device, int64_t B, int32_t N, int32_t S, int32_t ds, int32_
                   static_cast<long long>(B), N, S, ds, D);
     LTGNN_REQUIRE(D % 4 == 0 && kThreads % (D / 4) == 0, LTGNN_E_SHAPE, "%s: D=%d must be 4 * a divisor of %d", who, D,
                   kThreads);
-    LTGNN_REQUIRE(D * (ds + 1) <= 40 * kThreads, LTGNN_E_SHAPE, "%s: D*(ds+1)=%d too large", who, D * (ds + 1));
     *di = device_info(device);
     if (!*di) return LTGNN_E_CUDA;
     LTGNN_REQUIRE((*di)->cc_major == 10, LTGNN_E_UNSUPPORTED, "%s: device is sm_%d%d, need sm_100", who,

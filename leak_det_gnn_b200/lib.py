@@ -93,6 +93,9 @@ SIGNATURES = {
                                     c_void_p, c_void_p]),
     "ltgnn_gru_dropout": (c_int, [c_int, c_int64, c_int32, c_void_p, c_float, c_uint64, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_dropout_bwd": (c_int, [c_int, c_int64, c_int32, c_void_p, c_int32, c_void_p, c_float, c_void_p, c_void_p]),
+    "ltgnn_gru_sensor_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int64, c_int64, c_int32, c_void_p, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gru_resident_tiles": (c_int, [c_int, c_void_p]),
 }
 
 _lib = None

@@ -787,7 +787,8 @@ def gnn_body(h_s: torch.Tensor, slot: torch.Tensor, graph: PipeGraph, drop_p: fl
 # shared per-sensor GRU encoder (reference models/detector.py:28-73)
 # ----------------------------------------------------------------------------------------------
 def gru_supported(hidden: int, n_time: int) -> bool:
-    return hidden == 64 and 0 <= n_time <= 30
+    """Hidden 64: csrc/gru.cu; hidden 128: the cluster recurrence of csrc/gru_pred.cu (``_SensorGru128``)."""
+    return hidden in (64, 128) and 0 <= n_time <= 30
 
 
 def gru_fwd(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh, save: bool = False):
@@ -864,11 +865,15 @@ class _GruEncoder(torch.autograd.Function):
 
 
 def gru_encode(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh) -> torch.Tensor:
-    """Differentiable (wrt the parameters) shared sensor GRU: (B,L,S) [+ (B,L,F)] -> (B,S,64)."""
+    """Differentiable (wrt the parameters) shared sensor GRU: (B,L,S) [+ (B,L,F)] -> (B,S,H), H = 64 or 128."""
     _check_act(r.contiguous(), "r")
     if r.requires_grad or (tf is not None and tf.requires_grad):
         raise ValueError("gru_encode: gradients with respect to the inputs are not implemented by the native GRU "
                          "(the reference never asks for them); use the cuDNN route (use_native = False)")
+    if w_hh.shape[1] == 128:
+        if not torch.is_grad_enabled():   # eval, event evaluation: one launch, nothing saved
+            return _SensorGru128.infer(r.contiguous(), None if tf is None else tf.contiguous(), w_ih, w_hh, b_ih, b_hh)
+        return _SensorGru128.apply(r, tf, w_ih, w_hh, b_ih, b_hh)
     return _GruEncoder.apply(r, tf, w_ih, w_hh, b_ih, b_hh)
 
 
@@ -1128,6 +1133,148 @@ def gru_predictor_cone(x: torch.Tensor, x_time: torch.Tensor, drop_p: float, par
     inp.view(b, length, kp)[:, :, s:c_in] = x_time
     inp[:, c_in] = 1.0
     return _GruPredictor.apply(inp, b, length, c_in, s, float(drop_p), *params)
+
+
+# ----------------------------------------------------------------------------------------------
+# shared sensor GRU encoder at hidden 128 (reference models/detector.py:28-73, sensor_hidden = 128): the predictor's
+# cluster recurrence and BPTT (csrc/gru_pred.cu) with the encoder's input formed in the kernel
+# ----------------------------------------------------------------------------------------------
+_SLAB_BYTES = 8 << 30     # backward temporaries of one slab: dG, [h_{t-1} | 1 | 0], [r | tf | 1 | 0] = 2 816 B per row
+_RESIDENT_TILES: Dict[int, int] = {}
+
+
+def gru_resident_tiles(dev: int) -> int:
+    """128-sequence tiles the cluster recurrence runs at once on device ``dev`` (one wave); cached per device."""
+    if dev not in _RESIDENT_TILES:
+        n = ctypes.c_int32(0)
+        _lib.check(_lib.load().ltgnn_gru_resident_tiles(dev, ctypes.byref(n)))
+        if n.value <= 0:
+            raise RuntimeError(f"gru_resident_tiles: the device runs no 4-CTA cluster of the GRU recurrence ({n.value})")
+        _RESIDENT_TILES[dev] = n.value
+    return _RESIDENT_TILES[dev]
+
+
+def gru_sensor_slabs(q: int, l: int, dev: int) -> list:
+    """[(q0, n)]: the training slabs of q sequences of l steps, each a whole number of waves of resident tiles (the last
+    one what is left), as many waves per slab as keep its backward temporaries within _SLAB_BYTES (at least one)."""
+    wave = 128 * gru_resident_tiles(dev)
+    n = max(1, _SLAB_BYTES // (wave * l * 2816)) * wave
+    return [(q0, min(n, q - q0)) for q0 in range(0, q, n)]
+
+
+def gru_sensor_tproj(tf: Optional[torch.Tensor], w_ih: torch.Tensor, b_ih: torch.Tensor, b_hh: torch.Tensor,
+                     b: int, l: int) -> torch.Tensor:
+    """T [3, b * l, H] = tf W_ih[:, 1:]^T + b_ih, plus b_hh for r and z (folded as ``gru_predictor_weights`` folds them):
+    ``linear_tc`` at K = 32 on the zero-padded time features, one launch per gate group; without time features every
+    row is the folded bias."""
+    h = w_ih.shape[0] // 3
+    f = w_ih.shape[1] - 1
+    b_x = b_ih.detach().view(3, h).clone()
+    b_x[:2] += b_hh.detach().view(3, h)[:2]
+    if f == 0:
+        return b_x.unsqueeze(1).expand(3, b * l, h).contiguous()
+    x = torch.zeros(b * l, 32, device=w_ih.device, dtype=torch.float32)
+    x[:, :f] = tf.reshape(b * l, f)
+    w_t = torch.zeros(3, h, 32, device=w_ih.device, dtype=torch.float32)
+    w_t[:, :, :f] = w_ih.detach()[:, 1:].reshape(3, h, f)
+    t = torch.empty(3, b * l, h, device=w_ih.device, dtype=torch.float32)
+    for g in range(3):
+        linear_tc(x, w_t[g], b_x[g], out=t[g])
+    return t
+
+
+def gru_sensor_fwd(r: torch.Tensor, tproj: torch.Tensor, w_r: torch.Tensor, w_hh: torch.Tensor, b_hn: torch.Tensor,
+                   q0: int, n: int, h_last: torch.Tensor, hseq: Optional[torch.Tensor] = None,
+                   gates: Optional[torch.Tensor] = None) -> None:
+    """Raw forward of sequences q0 .. q0 + n - 1 of the encoder (see ltgnn_gru_sensor_fwd): r (B, L, S), tproj
+    [3, B * L, H] (``gru_sensor_tproj``), w_r [3, H] = W_ih[:, 0]; writes h_last (n, H) and, for training, hseq
+    (n * L, H) and gates [4, n * L, H] in the planar layout ``gru_layer_bwd`` reads."""
+    for t, nm in ((r, "r"), (tproj, "tproj"), (w_r, "w_r"), (w_hh, "w_hh"), (b_hn, "b_hn"), (h_last, "h_last")):
+        _check_act(t, nm)
+    b, l, s = r.shape
+    L = _lib.load()
+    tok = _inst.begin("gru_sensor_train" if gates is not None else "gru_sensor")
+    _lib.check(L.ltgnn_gru_sensor_fwd(_dev_index(r), b, l, s, q0, n, w_hh.shape[1], r.data_ptr(), tproj.data_ptr(),
+                                      w_r.data_ptr(), w_hh.data_ptr(), b_hn.data_ptr(),
+                                      None if hseq is None else hseq.data_ptr(), h_last.data_ptr(),
+                                      None if gates is None else gates.data_ptr(), _stream(r)))
+    _inst.end(tok)
+
+
+def _sensor_x_aug(r: torch.Tensor, tf: Optional[torch.Tensor], q0: int, n: int) -> torch.Tensor:
+    """[r | tf | 1 | 0 ...] (n * L, 32) for sequences q0 .. q0 + n - 1: the layer input with the ones column."""
+    b, l, s = r.shape
+    f = 0 if tf is None else tf.shape[-1]
+    q = torch.arange(q0, q0 + n, device=r.device)
+    bi, si = q // s, q % s
+    x = torch.zeros(n, l, 32, device=r.device, dtype=torch.float32)
+    x[:, :, 0] = r[bi, :, si]
+    if f:
+        x[:, :, 1:1 + f] = tf[bi]
+    x[:, :, 1 + f] = 1.0
+    return x.view(n * l, 32)
+
+
+class _SensorGru128(torch.autograd.Function):
+    """The shared sensor GRU at hidden 128: h_last (B, S, 128), with back-propagation through time to the four GRU
+    parameters (the inputs are data, as in ``_GruEncoder``).
+
+    Without gradients (grad mode off, or no parameter requires one): T (``gru_sensor_tproj``) and one recurrence launch,
+    nothing saved.  With gradients the sequences
+    run in slabs (``gru_sensor_slabs``): each slab's training forward saves its gates and states; the backward runs per
+    slab ``gru_layer_bwd`` from that slab's rows of dh and ``gru_layer_param_grads`` against [r | tf | 1], and adds the
+    slabs' gradients in slab order.  At B = 4096, L = 288, S = 29 the saved state alone is 87.5 GB, so the backward's
+    dG and operands (96 GB more in one piece) must be formed a slab at a time."""
+
+    @staticmethod
+    def _operands(r, tf, w_ih, w_hh, b_ih, b_hh):
+        b, l, s = r.shape
+        hd = w_hh.shape[1]
+        return (gru_sensor_tproj(tf, w_ih, b_ih, b_hh, b, l), w_ih.detach()[:, 0].contiguous(), w_hh.detach().contiguous(),
+                b_hh.detach()[2 * hd:].contiguous(), torch.empty(b, s, hd, device=r.device, dtype=torch.float32))
+
+    @staticmethod
+    def infer(r, tf, w_ih, w_hh, b_ih, b_hh):
+        tproj, w_r, w_hh_c, b_hn, h_last = _SensorGru128._operands(r, tf, w_ih, w_hh, b_ih, b_hh)
+        gru_sensor_fwd(r, tproj, w_r, w_hh_c, b_hn, 0, r.shape[0] * r.shape[2], h_last.view(-1, w_hh.shape[1]))
+        return h_last
+
+    @staticmethod
+    def forward(ctx, r, tf, w_ih, w_hh, b_ih, b_hh):
+        r = r.contiguous()
+        tf = None if tf is None else tf.contiguous()
+        if not any(ctx.needs_input_grad[2:]):   # nothing requires a gradient: backward is never reached
+            return _SensorGru128.infer(r, tf, w_ih, w_hh, b_ih, b_hh)
+        b, l, s = r.shape
+        q, hd = b * s, w_hh.shape[1]
+        tproj, w_r, w_hh_c, b_hn, h_last = _SensorGru128._operands(r, tf, w_ih, w_hh, b_ih, b_hh)
+        flat = h_last.view(q, hd)
+        slabs = gru_sensor_slabs(q, l, _dev_index(r))
+        saved = []
+        for q0, n in slabs:
+            hseq = torch.empty(n * l, hd, device=r.device, dtype=torch.float32)
+            gates = torch.empty(4, n * l, hd, device=r.device, dtype=torch.float32)
+            gru_sensor_fwd(r, tproj, w_r, w_hh_c, b_hn, q0, n, flat[q0:q0 + n], hseq, gates)
+            saved += [hseq, gates]
+        ctx.save_for_backward(r, tf, w_hh_c, *saved)
+        ctx.slabs = slabs
+        return h_last
+
+    @staticmethod
+    def backward(ctx, dh):
+        r, tf, w_hh, *saved = ctx.saved_tensors
+        l = r.shape[1]
+        f = 0 if tf is None else tf.shape[-1]
+        dh = dh.contiguous().view(-1, w_hh.shape[1])
+        grads = None
+        for i, (q0, n) in enumerate(ctx.slabs):
+            hseq, gates = saved[2 * i], saved[2 * i + 1]
+            dg = gru_layer_bwd(n, l, w_hh, gates, hseq, dh_last=dh[q0:q0 + n])
+            part = gru_layer_param_grads(dg, hseq, _sensor_x_aug(r, tf, q0, n), 1 + f, n, l)
+            del dg
+            grads = part if grads is None else [a + p for a, p in zip(grads, part)]
+        return (None, None, *grads)
+
 
 def tcn_conv(x: torch.Tensor, src: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor,
              gamma: Optional[torch.Tensor] = None, beta: Optional[torch.Tensor] = None, eps: float = 1e-5, relu: bool = True,
