@@ -319,6 +319,17 @@ int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int32_t F, int3
  */
 int ltgnn_gru_layer_fwd(int device, int64_t Q, int32_t L, int32_t H, const float* gx, const float* w_hh, const float* b_hn,
                         float* hseq, float* h_last, void* stream);
+/* gru_layer_fwd_windows: ltgnn_gru_layer_fwd on Q windows that share one input projection (overlapping windows of a
+ * series, e.g. every window of a segment): gx [3][gx_rows][H] is projected once per series row, and window q reads its
+ * step-t row at row_base[q] + t (int32 [Q]) instead of q*L + t.  h_last [Q, H] and hseq [Q, L, H] are the planar form's,
+ * bit for bit.  The caller guarantees 0 <= row_base[q] and row_base[q] + L <= gx_rows (the entry point does not read
+ * device memory).  H = 128 only, Q < 2^31 - 128 and gx_rows < 2^31 (else LTGNN_E_SHAPE); Q, L > 0, gx_rows >= L and gx,
+ * row_base, w_hh, b_hn, h_last non-NULL (else LTGNN_E_ARG); gx, w_hh, hseq, h_last 16-byte aligned and row_base 4-byte
+ * aligned (else LTGNN_E_ALIGN).  Deterministic, no allocation or host synchronisation: capturable into a CUDA graph.
+ */
+int ltgnn_gru_layer_fwd_windows(int device, int64_t Q, int32_t L, int32_t H, const float* gx, int64_t gx_rows,
+                                const int32_t* row_base, const float* w_hh, const float* b_hn, float* hseq, float* h_last,
+                                void* stream);
 
 /* ---- training of the GRU normal-state predictor (predictor.py:84-111, train_predictor.py), same file ----------------
  * gru_layer_fwd_train: ltgnn_gru_layer_fwd (same kernel, same h_last and hseq bit for bit) that also stores every step's

@@ -21,6 +21,8 @@
 // Shared memory 192 KiB + alignment; tensor memory 352 of 512 columns.  No atomics, fixed order: bitwise deterministic.
 // The same kernel runs the shared sensor encoder at hidden 128 (kSensor): there the input term is formed in the gate
 // threads from one residual and a time-feature projection shared by the window's sensors (ltgnn_gru_sensor_fwd).
+// The windowed inference form (kWindows) runs overlapping windows of a series on one shared input projection: sequence q
+// reads its step-t gx row at base[q] + t of a plane projected once per series row (ltgnn_gru_layer_fwd_windows).
 #include "umma.cuh"
 #include "rowgemm_ts.cuh"
 
@@ -66,6 +68,8 @@ struct GruLayerParams {
     uint32_t S;
     uint32_t q0;
     size_t tplane;      // B * L * H
+    // windowed form: gx is [3][gx_rows][H] (plane gx_rows * H) and sequence q reads step t from row row_base[q] + t
+    const int32_t* row_base;  // [Q]
 };
 
 // same fast forms as the sensor GRU (gru.cu)
@@ -101,7 +105,8 @@ __device__ __forceinline__ void split16_store(uint32_t t_hi, uint32_t t_lo, cons
 // kTrain: also store every step's r, z, n and hn for the backward (hseq is then required).
 // kSensor: the sensor encoder's input form (see GruLayerParams): one residual value and one T row per step instead of a
 // gx row per sequence; every output is the planar form's, row (local q) L + t.
-template <bool kTrain, bool kSensor = false>
+// kWindows (inference only): sequence q's gx rows start at row_base[q] instead of q L; hseq and h_last stay planar.
+template <bool kTrain, bool kSensor = false, bool kWindows = false>
 __global__ void __launch_bounds__(kThreads, 1)
 gru_layer_fwd_kernel(const GruLayerParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -161,6 +166,8 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
             h[j] = 0.f;
         }
         const size_t row0 = static_cast<size_t>(valid ? q : 0) * L;  // gx / hseq row of step 0
+        size_t xrow0 = row0;                                          // gx row of step 0
+        if constexpr (kWindows) xrow0 = valid ? static_cast<size_t>(__ldg(p.row_base + q)) : 0;
         float gr[16], gz[16], gn[16];
         // sensor form: the T row of step 0 (b L) and the residual of step 0 (b L S + s)
         float xr = 0.f;
@@ -180,7 +187,7 @@ gru_layer_fwd_kernel(const GruLayerParams p) {
                     load16(src + 2 * p.tplane, gn);
                     xr = __ldg(rsrc + static_cast<size_t>(t) * p.S);
                 } else {
-                    const float* src = p.gx + (row0 + t) * H + u0;
+                    const float* src = p.gx + (xrow0 + t) * H + u0;
                     load16(src, gr);
                     load16(src + p.plane, gz);
                     load16(src + 2 * p.plane, gn);
@@ -674,6 +681,31 @@ extern "C" int ltgnn_gru_sensor_fwd(int device, int64_t B, int32_t L, int32_t S,
     LTGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSensorSmem)));
     const int64_t tiles = (Q + 127) / 128;
     LTGNN_CUDA_TRY(launch_cluster(kernel, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSensorSmem,
+                                  static_cast<cudaStream_t>(stream_), kCluster, p));
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+extern "C" int ltgnn_gru_layer_fwd_windows(int device, int64_t Q, int32_t L, int32_t Hdim, const float* gx, int64_t gx_rows,
+                                           const int32_t* row_base, const float* w_hh, const float* b_hn, float* hseq,
+                                           float* h_last, void* stream_) {
+    LTGNN_REQUIRE(Q > 0 && L > 0 && gx_rows >= L, LTGNN_E_ARG, "gru_layer_fwd_windows: Q=%lld L=%d gx_rows=%lld",
+                  static_cast<long long>(Q), L, static_cast<long long>(gx_rows));
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_layer_fwd_windows: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(Q < (1ll << 31) - 128 && gx_rows < (1ll << 31), LTGNN_E_SHAPE,
+                  "gru_layer_fwd_windows: too many sequences or gx rows");
+    LTGNN_REQUIRE(gx && row_base && w_hh && b_hn && h_last, LTGNN_E_ARG, "gru_layer_fwd_windows: null tensor");
+    LTGNN_REQUIRE(aligned16(gx) && aligned16(w_hh) && aligned16(hseq) && aligned16(h_last) &&
+                  reinterpret_cast<uintptr_t>(row_base) % 4 == 0, LTGNN_E_ALIGN,
+                  "gru_layer_fwd_windows: gx, w_hh, hseq and h_last must be 16-byte aligned, row_base 4-byte aligned");
+    if (int rc = check_device(device, "gru_layer_fwd_windows")) return rc;
+    LTGNN_USE_DEVICE(device);
+    GruLayerParams p{gx, w_hh, b_hn, hseq, h_last, static_cast<uint32_t>(Q), L, static_cast<size_t>(gx_rows) * H, nullptr,
+                     nullptr, nullptr, 0u, 0u, 0, row_base};
+    auto kernel = gru_layer_fwd_kernel<false, false, true>;
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kSmem)));
+    const int64_t tiles = (Q + 127) / 128;
+    LTGNN_CUDA_TRY(launch_cluster(kernel, dim3(static_cast<unsigned>(tiles * kCluster)), dim3(kThreads), kSmem,
                                   static_cast<cudaStream_t>(stream_), kCluster, p));
     LTGNN_CUDA_TRY(cudaGetLastError());
     return LTGNN_OK;

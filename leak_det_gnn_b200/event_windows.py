@@ -17,7 +17,7 @@ from typing import List, Tuple
 import numpy as np
 import torch
 
-from .models.utils import build_residual_sequence_from_segment
+from .models.utils import build_residual_sequence_from_segment, residual_series
 
 
 @torch.no_grad()
@@ -26,7 +26,12 @@ def scenario_window_logits(predictor, detector, pressure_all, tfeat_all, l_pred:
     """All windows of one scenario.  pressure_all (T, S), tfeat_all (T, F) -- the standardised series
     event_evaluator.py:455-466 prepares.  Returns (out_end indices, logits (n_windows, C) on the CPU): window i is the
     reference's ``t0 = l_pred + i * stride``, its segment ``[t0 - l_pred, t0 + l_det)`` and its record time
-    ``df_sensor.index[out_end - 1]`` (event_evaluator.py:478-492)."""
+    ``df_sensor.index[out_end - 1]`` (event_evaluator.py:478-492).
+
+    The residual of a step does not depend on the window that reads it, so it is computed once per scenario: at
+    stride < l_det the windows read one contiguous range of steps, whose residual series (``residual_series``) every
+    window slices; at stride >= l_det no step is read twice and each window's segment goes through the residual builder
+    (the steps between windows are never computed).  The detector sees the same batches either way."""
     p = torch.as_tensor(np.asarray(pressure_all), dtype=torch.float32)
     f = torch.as_tensor(np.asarray(tfeat_all), dtype=torch.float32)
     seg_len, n_t = l_pred + l_det, p.shape[0]
@@ -34,11 +39,21 @@ def scenario_window_logits(predictor, detector, pressure_all, tfeat_all, l_pred:
     if not starts:
         return [], torch.empty(0, 0)
     idx = torch.tensor(starts)
-    seg_p = p.unfold(0, seg_len, 1).permute(0, 2, 1)             # (T - seg_len + 1, seg_len, S) strided view
-    seg_f = f.unfold(0, seg_len, 1).permute(0, 2, 1)
     predictor.eval()
     detector.eval()
     out = []
+    if stride < l_det:
+        end = starts[-1] + seg_len                                # the last step any window reads, + 1
+        p_dev, f_dev = p[:end].to(device), f[:end].to(device)
+        res = residual_series(predictor, p_dev, f_dev, l_pred)    # row i = step l_pred + i = window start i's first
+        res_w = res.unfold(0, l_det, 1)                           # (., S, l_det): window starting at row i
+        f_w = f_dev[l_pred:].unfold(0, l_det, 1)
+        for lo in range(0, len(starts), batch):
+            sel = idx[lo:lo + batch].to(device)
+            out.append(detector(res_w[sel].permute(0, 2, 1).contiguous(), f_w[sel].permute(0, 2, 1).contiguous()))
+        return [s + seg_len for s in starts], torch.cat(out).cpu()
+    seg_p = p.unfold(0, seg_len, 1).permute(0, 2, 1)             # (T - seg_len + 1, seg_len, S) strided view
+    seg_f = f.unfold(0, seg_len, 1).permute(0, 2, 1)
     for lo in range(0, len(starts), batch):
         sel = idx[lo:lo + batch]
         noisy = seg_p[sel].contiguous().to(device, non_blocking=True)

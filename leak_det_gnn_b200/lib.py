@@ -96,6 +96,8 @@ SIGNATURES = {
     "ltgnn_gru_sensor_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int64, c_int64, c_int32, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_resident_tiles": (c_int, [c_int, c_void_p]),
+    "ltgnn_gru_layer_fwd_windows": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_void_p,
+                                            c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

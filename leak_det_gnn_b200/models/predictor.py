@@ -70,6 +70,9 @@ class NormalPredictorTCN(nn.Module):
     # use the hand-written sm_100a kernels for ``forward_last`` on CUDA (csrc/tcn.cu + csrc/linear.cu) where the shapes
     # allow; False = the same cone through torch ops (cuBLAS), kept as the cross-check
     use_native = True
+    # ``forward_windows`` computes the rows overlapping windows share once (``shared_cone_plan``); False = ``forward_last``
+    # on the materialised windows, kept as the cross-check
+    share_windows = True
 
     def _native_ok(self, x: torch.Tensor) -> bool:
         blk = self.tcn[0]
@@ -86,6 +89,28 @@ class NormalPredictorTCN(nn.Module):
         if self._native_ok(x):
             return self._forward_last_native(x, x_time)
         return self._cone_torch(x, x_time)
+
+    @torch.no_grad()
+    def forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, count=None) -> torch.Tensor:
+        """``forward_last`` of every window of ``window`` steps: x (B, T, S), x_time (B, T, F) -> (B, n, S) with
+        ``out[b, j] = forward_last(x[b, j:j + window], x_time[b, j:j + window])``, n = count or T - window + 1.
+        On the native path a row of convolution i at window position p >= R_i (the cumulative left reach of convolutions
+        0..i) reads no left padding, so it is the same in every window that contains its step: it is computed once per
+        (series, step), the input projection once per series row, and only the rows near each window's left edge per
+        window (``shared_cone_plan``); the result equals ``forward_last`` on the materialised windows bit for bit."""
+        if self.training:
+            raise RuntimeError("forward_windows is the inference path of the frozen predictor (call .eval() first)")
+        b, length, _ = x.shape
+        n = _window_count(length, window, count)
+        if not (self.share_windows and self._native_ok(x)):
+            return self.forward_last(windows_of(x, window, n), windows_of(x_time, window, n)).view(b, n, -1)
+        from .. import ops
+
+        dev = x.device
+        prep = self._native_weights(dev)
+        rows = self._shared_rows(length, window, n, b, dev)
+        h = ops.linear_tc(self._native_input(x, x_time), prep["w_in"], prep["b_in"])                # (B * T, 128)
+        return self._native_stack(h, rows, prep).view(b, n, -1)
 
     def forward_cone(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
         """``forward``'s result, differentiable in train and eval mode, from the dependency cone of the last time step.
@@ -135,11 +160,23 @@ class NormalPredictorTCN(nn.Module):
         dev = x.device
         prep = self._native_weights(dev)
         rows = self._native_rows(length, b, dev)
+        h = ops.linear_tc(self._native_input(x, x_time), prep["w_in"], prep["b_in"])                # (B * L, 128)
+        return self._native_stack(h, rows, prep)
+
+    def _native_input(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
+        """cat([x, x_time]) zero-padded to the projection kernel's K = 64: (B * L, 64)."""
+        b, length, _ = x.shape
         c_in = self.num_sensors + self.time_dim
-        inp = torch.zeros(b, length, 64, device=dev, dtype=torch.float32)
+        inp = torch.zeros(b, length, 64, device=x.device, dtype=torch.float32)
         inp[:, :, :self.num_sensors] = x
         inp[:, :, self.num_sensors:c_in] = x_time
-        h = ops.linear_tc(inp.view(b * length, 64), prep["w_in"], prep["b_in"])                 # (B * L, 128)
+        return inp.view(b * length, 64)
+
+    def _native_stack(self, h: torch.Tensor, rows, prep) -> torch.Tensor:
+        """The blocks and the head on gathered rows: ``rows`` per block (src1, src2, res_row) into the previous row pool
+        (``_native_rows`` or ``_shared_rows``), whose last pool holds one row per output, in output order."""
+        from .. import ops
+
         for blk, (w1, w2), (src1, src2, keep_rows) in zip(self.tcn, prep["convs"], rows):
             y = ops.tcn_conv(h, src1, w1, blk.conv1.conv.bias, blk.norm1.weight, blk.norm1.bias, blk.norm1.eps, True)
             h = ops.tcn_conv(y, src2, w2, blk.conv2.conv.bias, blk.norm2.weight, blk.norm2.bias, blk.norm2.eps, True,
@@ -190,6 +227,21 @@ class NormalPredictorTCN(nn.Module):
             keep_rows = (win * n_in + keep.unsqueeze(0)).reshape(-1).to(torch.int32).contiguous()
             out.append((rows[0], rows[1], keep_rows))
             n_in = keep.numel()
+        if len(cache) > 8:
+            cache.clear()
+        cache[key] = out
+        return out
+
+    def _shared_rows(self, length: int, window: int, count: int, batch: int, device):
+        """``shared_cone_plan`` for ``batch`` series in the layout of ``_native_rows`` (int32 on ``device``), built on the
+        host once per shape and device: build it outside CUDA-graph capture (a graphed step's warm-up does)."""
+        cache = self.__dict__.setdefault("_shared_r", {})
+        key = (length, window, count, batch, str(device))
+        if key in cache:
+            return cache[key]
+        plan, _ = shared_cone_plan(length, window, count, batch, self.tcn[0].conv1.conv.kernel_size[0],
+                                [blk.conv1.conv.dilation[0] for blk in self.tcn])
+        out = [tuple(t.to(device=device, dtype=torch.int32).contiguous() for t in blk) for blk in plan]
         if len(cache) > 8:
             cache.clear()
         cache[key] = out
@@ -279,6 +331,9 @@ class NormalPredictorGRU(nn.Module):
     # use the hand-written sm_100a kernels for ``forward_last`` and ``forward_cone`` on CUDA where the shapes allow;
     # False = the dense cuDNN ``forward``, kept as the cross-check
     use_native = True
+    # ``forward_windows`` projects layer 0's input once per series row for all windows; False = ``forward_last`` on the
+    # materialised windows, kept as the cross-check
+    share_windows = True
 
     def _native_ok(self, x: torch.Tensor) -> bool:
         g = self.gru
@@ -298,6 +353,25 @@ class NormalPredictorGRU(nn.Module):
         prep = self._native_weights(x.device)
         h = ops.gru_predictor_fwd(x, x_time, prep["layers"])
         return ops.linear_tc(h, prep["w_out"], prep["b_out"])[:, :self.num_sensors]
+
+    @torch.no_grad()
+    def forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, count=None) -> torch.Tensor:
+        """``forward_last`` of every window of ``window`` steps: x (B, T, S), x_time (B, T, F) -> (B, n, S) with
+        ``out[b, j] = forward_last(x[b, j:j + window], x_time[b, j:j + window])``, n = count or T - window + 1.
+        Every window restarts the recurrence from a zero state, so only layer 0's input projection is shared: on the
+        native path it is computed once per series row and window (b, j) reads rows b T + j .. + window - 1 of it
+        (``ops.gru_predictor_windows``), bit for bit the result on the materialised windows."""
+        if self.training:
+            raise RuntimeError("forward_windows is the inference path of the frozen predictor (call .eval() first)")
+        b, length, _ = x.shape
+        n = _window_count(length, window, count)
+        if not (self.share_windows and self._native_ok(x)):
+            return self.forward_last(windows_of(x, window, n), windows_of(x_time, window, n)).view(b, n, -1)
+        from .. import ops
+
+        prep = self._native_weights(x.device)
+        h = ops.gru_predictor_windows(x, x_time, window, n, prep["layers"])
+        return ops.linear_tc(h, prep["w_out"], prep["b_out"])[:, :self.num_sensors].view(b, n, -1)
 
     def forward_cone(self, x: torch.Tensor, x_time: torch.Tensor) -> torch.Tensor:
         """``forward``'s result, differentiable in train and eval mode, with the module's inter-layer dropout in train mode.
@@ -351,3 +425,106 @@ def cone_positions(length: int, kernel_size: int, dilations: List[int]) -> List[
         need = {t - j * d for t in conv1 for j in range(kernel_size) if t - j * d >= 0} | need
         out.append((conv1, conv2))
     return list(reversed(out))
+
+
+def _window_count(length: int, window: int, count=None) -> int:
+    n = length - window + 1 if count is None else int(count)
+    if window < 1 or n < 1 or n + window - 1 > length:
+        raise ValueError(f"{n} windows of {window} steps do not fit a series of {length} steps")
+    return n
+
+
+def windows_of(x: torch.Tensor, window: int, count: int) -> torch.Tensor:
+    """(B, T, C) -> (B * count, window, C): window (b, j) = x[b, j:j + window] at row b * count + j (a copy)."""
+    b, _, c = x.shape
+    return x.unfold(1, window, 1)[:, :count].permute(0, 1, 3, 2).reshape(b * count, window, c)
+
+
+def cone_reach(kernel_size: int, dilations: List[int]) -> List[int]:
+    """R_i per convolution (two per block): how far left the convolutions 0..i reach together.  A row of convolution i
+    at window position p >= R_i reads no left padding, so its value depends on the series alone, not on the window.
+    For k = 3 and d = 1, 2, 4, 8: [2, 4, 8, 12, 20, 28, 44, 60]."""
+    out, r = [], 0
+    for d in dilations:
+        for _ in range(2):
+            r += (kernel_size - 1) * d
+            out.append(r)
+    return out
+
+
+def shared_cone_plan(length: int, window: int, count: int, batch: int, kernel_size: int, dilations: List[int]):
+    """Row pools of ``count`` overlapping windows of ``window`` steps per series (window (b, j) = steps j .. j + window - 1
+    of series b) that compute every window-independent row once.  The cone of each window is ``cone_positions``; its row
+    of convolution i at position p is SHARED, keyed by (series b, step j + p), when p >= R_i (``cone_reach``), and
+    WINDOWED, keyed by (window, p), otherwise.  Pool i = [shared rows, series-major then step | windowed rows,
+    window-major (b * count + j) then position]; pool -1 = the B * T input-projection rows b * T + t.
+
+    Returns (plan, shared): shared[i] = the shared rows per series of convolution i; plan per block (src1 (k, M1),
+    src2 (k, M2), res_row (M2,)) int64 on the CPU, the layout of
+    ``NormalPredictorTCN._native_rows``: src1 indexes the block input's pool (oldest tap first, -1 = left padding),
+    src2 conv1's pool and res_row the block input's pool.  The last pool holds one row per window in window order:
+    windowed when window - 1 < R_last, shared otherwise.  Built with tensor ops over (series, window, position)."""
+    if window < 1 or count < 1 or count + window - 1 > length:
+        raise ValueError(f"{count} windows of {window} steps do not fit a series of {length} steps")
+    cone = [pos for blk in cone_positions(window, kernel_size, dilations) for pos in blk]   # per convolution
+    reach = cone_reach(kernel_size, dilations)
+    i64 = torch.int64
+    bs = torch.arange(batch, dtype=i64).view(-1, 1, 1)        # (B, 1, 1)
+    js = torch.arange(count, dtype=i64).view(1, -1, 1)        # (1, n, 1)
+
+    class Pool:
+        def __init__(self, shared, windowed, r):
+            mask = torch.zeros(length, dtype=torch.bool)
+            if shared:
+                mask[(torch.tensor(shared, dtype=i64).view(-1, 1) + torch.arange(count, dtype=i64)).view(-1)] = True
+            self.steps = mask.nonzero().view(-1)                         # absolute steps of the shared rows
+            self.rank_s = torch.cumsum(mask, 0) - 1
+            self.rank_s[~mask] = -1
+            self.rank_w = torch.full((window,), -1, dtype=i64)
+            self.rank_w[torch.tensor(windowed, dtype=i64)] = torch.arange(len(windowed), dtype=i64)
+            self.win_pos = torch.tensor(windowed, dtype=i64)
+            self.n_s, self.n_w, self.r = self.steps.numel(), len(windowed), r
+
+        def at(self, p):
+            """Rows of every window (b, j) at positions p (1-D, may be < 0) -> (B, n, P); -1 for left padding."""
+            p = p.view(1, 1, -1)
+            pc = p.clamp(min=0)
+            rank = torch.where(p >= self.r, self.rank_s[js + pc], self.rank_w[pc])
+            assert bool((rank[(p >= 0).expand_as(rank)] >= 0).all()), "a tap reads a row its pool does not hold"
+            out = torch.where(p >= self.r, bs * self.n_s + rank, batch * self.n_s + (bs * count + js) * self.n_w + rank)
+            return torch.where(p < 0, torch.full_like(out, -1), out)
+
+        def at_steps(self, a):
+            """Shared rows of every series at absolute steps a (1-D) -> (B, A)."""
+            r = self.rank_s[a]
+            assert bool((r >= 0).all()), "a shared row reads a step its pool does not hold"
+            return bs.view(-1, 1) * self.n_s + r.view(1, -1)
+
+    def rows(pool_in, pos, r, d):
+        """Rows of one convolution: its pool (shared / windowed split of pos at r) and per tap its sources in pool_in."""
+        shared = [p for p in pos if p >= r]
+        windowed = [p for p in pos if p < r]
+        out = Pool(shared, windowed, r)
+        taps = []
+        for k in range(kernel_size - 1, -1, -1):                # oldest tap first: weight[:, :, 0] multiplies it
+            s_rows = pool_in.at_steps(out.steps - k * d).reshape(-1) if out.n_s else torch.empty(0, dtype=i64)
+            w_rows = pool_in.at(out.win_pos - k * d).reshape(-1)
+            taps.append(torch.cat([s_rows, w_rows]))
+        return out, torch.stack(taps)
+
+    def residual(pool_in, out):
+        s_rows = pool_in.at_steps(out.steps).reshape(-1) if out.n_s else torch.empty(0, dtype=i64)
+        return torch.cat([s_rows, pool_in.at(out.win_pos).reshape(-1)])
+
+    pool = Pool(list(range(window)), [], 0)
+    pool.steps, pool.rank_s, pool.n_s = torch.arange(length, dtype=i64), torch.arange(length, dtype=i64), length
+    plan, shared = [], []
+    for i, d in enumerate(dilations):
+        p1, src1 = rows(pool, cone[2 * i], reach[2 * i], d)
+        p2, src2 = rows(p1, cone[2 * i + 1], reach[2 * i + 1], d)
+        plan.append((src1, src2, residual(pool, p2)))
+        shared += [p1.n_s, p2.n_s]
+        pool = p2
+    # the head reads the last pool as is: one row per window, window-major
+    assert (pool.n_w, pool.n_s) == (1, 0) or (pool.n_w == 0 and torch.equal(pool.steps, torch.arange(count) + window - 1))
+    return plan, shared

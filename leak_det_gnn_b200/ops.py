@@ -939,6 +939,59 @@ def gru_predictor_fwd(x: torch.Tensor, x_time: torch.Tensor, layers) -> torch.Te
     return h_last
 
 
+def gru_layer_fwd_windows(gx: torch.Tensor, row_base: torch.Tensor, l: int, layer, seq: bool = False):
+    """Raw forward of one GRU layer over windows that share one input projection (see ltgnn_gru_layer_fwd_windows):
+    gx [3, rows, H] holds the projection of every series row once, row_base int32 (Q,) the gx row of each window's step 0.
+    The caller guarantees 0 <= row_base[q] and row_base[q] + l <= rows (the entry point cannot check device data).
+    Returns (h_last (Q, H), hseq (Q * l, H) or None): ``gru_layer_fwd``'s on the materialised windows, bit for bit."""
+    _check_act(gx, "gx")
+    _w_x, _b_x, w_hh, b_hn = layer
+    hdim = w_hh.shape[1]
+    if gx.dim() != 3 or gx.shape[0] != 3 or gx.shape[2] != hdim:
+        raise ValueError(f"gx must be (3, rows, {hdim}), got {tuple(gx.shape)}")
+    if row_base.dtype != torch.int32 or not row_base.is_cuda or not row_base.is_contiguous() or row_base.dim() != 1:
+        raise ValueError("row_base must be a contiguous 1-D int32 CUDA tensor")
+    q = row_base.numel()
+    h_last = torch.empty(q, hdim, device=gx.device, dtype=torch.float32)
+    hseq = torch.empty(q * l, hdim, device=gx.device, dtype=torch.float32) if seq else None
+    L = _lib.load()
+    tok = _inst.begin("gru_pred_layer_windows")
+    _lib.check(L.ltgnn_gru_layer_fwd_windows(_dev_index(gx), q, l, hdim, gx.data_ptr(), gx.shape[1], row_base.data_ptr(),
+                                             w_hh.data_ptr(), b_hn.data_ptr(), None if hseq is None else hseq.data_ptr(),
+                                             h_last.data_ptr(), _stream(gx)))
+    _inst.end(tok)
+    return h_last, hseq
+
+
+def gru_predictor_windows(x: torch.Tensor, x_time: torch.Tensor, window: int, count: int, layers) -> torch.Tensor:
+    """Raw stacked GRU on the ``count`` windows of ``window`` steps that start at steps 0 .. count-1 of every series:
+    x (B, T, S), x_time (B, T, F) -> the last layer's state after each window's last step, (B * count, H), window
+    (b, j) at row b * count + j.  Layer 0 projects the B * T series rows once and every window reads its rows from that
+    plane (``gru_layer_fwd_windows``); layers >= 1 run planar as in ``gru_predictor_fwd``, whose result this is bit for
+    bit on the materialised windows."""
+    b, t, s = x.shape
+    f = x_time.shape[-1]
+    k0 = layers[0][0].shape[2]
+    if s + f > k0:
+        raise ValueError(f"gru_predictor_windows: {s} + {f} inputs exceed K = {k0}")
+    if window < 1 or count < 1 or count + window - 1 > t:
+        raise ValueError(f"gru_predictor_windows: {count} windows of {window} steps do not fit {t} steps")
+    w_x, b_x, w_hh, _ = layers[0]
+    inp = torch.zeros(b * t, k0, device=x.device, dtype=torch.float32)
+    inp.view(b, t, k0)[:, :, :s] = x
+    inp.view(b, t, k0)[:, :, s:s + f] = x_time
+    gx = torch.empty(3, b * t, w_hh.shape[1], device=x.device, dtype=torch.float32)
+    for g in range(3):
+        linear_tc(inp, w_x[g], b_x[g], out=gx[g])
+    # window (b, j) starts at series row b t + j; j + window <= count - 1 + window <= t keeps every read inside the plane
+    row_base = ((torch.arange(b, device=x.device, dtype=torch.int32) * t).unsqueeze(1)
+                + torch.arange(count, device=x.device, dtype=torch.int32)).reshape(-1)
+    h_last, seq = gru_layer_fwd_windows(gx, row_base, window, layers[0], seq=len(layers) > 1)
+    for i, layer in enumerate(layers[1:], start=1):
+        h_last, seq = gru_layer_fwd(seq, b * count, window, layer, seq=i + 1 < len(layers))
+    return h_last
+
+
 
 # ----------------------------------------------------------------------------------------------
 # training of the GRU normal-state predictor (csrc/gru_pred.cu): saved-gates forward, BPTT, inter-layer dropout
