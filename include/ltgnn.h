@@ -297,6 +297,11 @@ int ltgnn_tcn_wgrad(int device, int64_t M, int32_t C, int32_t taps, const float*
  *                tensor-core GEMM instead of being saved: 8.75 GB less written and read at B*S = 118 784, L = 288.
  * gru_bwd_w:     dBfused [4H, 96] = sum_(t,q) dG^T [h_{t-1} | x | tf | 1 | 0]: columns 0..H-1 are d w_hh, H..H+F
  *                d w_ih, H+F+1 the bias gradients (rows: r, z, hn-part, in-part).  ws: ltgnn_gru_ws_floats() floats.
+ * gru_bwd_dx:    the gradient wrt the inputs from gru_bwd_dg_hn's dG: dx[q,t,:] = dG_r W_ih[r] + dG_z W_ih[z] + dG_in W_ih[n]
+ *                ([1+F] per sequence and step, fp32 FMAs in a fixed order).  dr [B, L, S] = dx[:, :, 0] at (b, t, s);
+ *                dxt [B, L, S, F] = dx[:, :, 1..F] per sequence, which the caller sums over s for d tf.  Either output may
+ *                be NULL (not both; dxt needs F > 0).  H = 64 and 1 + F <= 31 (else LTGNN_E_SHAPE); dG 16-byte aligned,
+ *                w_ih, dr and dxt 4-byte aligned (else LTGNN_E_ALIGN).  No atomics, allocation or host synchronisation.
  */
 int ltgnn_gru_fwd(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r, const float* tf,
                   const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, float* h_last,
@@ -306,6 +311,8 @@ int ltgnn_gru_bwd_dg_hn(int device, int64_t Q, int32_t L, int32_t H, const float
 int64_t ltgnn_gru_ws_floats(int device);
 int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* r, const float* tf,
                     const float* hseq, const float* dG, float* dBfused, float* ws, void* stream);
+int ltgnn_gru_bwd_dx(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t H, const float* w_ih,
+                     const float* dG, float* dr, float* dxt, void* stream);
 
 /* ---- one layer of the GRU normal-state predictor (predictor.py:84-111), forward only (csrc/gru_pred.cu) -------------
  * Q sequences of L steps, torch.nn.GRU equations and gate order (r, z, n), h_0 = 0.  The input projection is computed
@@ -374,11 +381,19 @@ int ltgnn_gru_dropout_bwd(int device, int64_t M, int32_t H, const float* dy, int
  *   gates 16-byte aligned (else LTGNN_E_ALIGN).  Deterministic, no allocation or host synchronisation: capturable.
  * gru_resident_tiles: *tiles = how many 128-sequence tiles (4-CTA clusters) of these recurrences the device runs at
  *   once (cudaOccupancyMaxActiveClusters): one wave.  Callers size their slabs in whole waves.
+ * gru_sensor_bwd_dx: ltgnn_gru_bwd_dx for the sequences q0 .. q0+Q-1 of the B*S, from ltgnn_gru_layer_bwd's dG
+ *   [4][Q*L][H] of those sequences (input planes r, z, n): writes their elements of dr [B, L, S] and dxt [B, L, S, F].
+ *   Every element is written by one thread whatever the slab split, so the caller's sum of dxt over s (after the last
+ *   slab) does not depend on it.  H = 128 and 1 + F <= 31 (else LTGNN_E_SHAPE); B, L, S, Q > 0, F >= 0, q0 >= 0,
+ *   q0 + Q <= B*S, w_ih and dG non-NULL, dr or dxt non-NULL, dxt only with F > 0 (else LTGNN_E_ARG); alignment as
+ *   ltgnn_gru_bwd_dx (else LTGNN_E_ALIGN).  No atomics, allocation or host synchronisation.
  */
 int ltgnn_gru_sensor_fwd(int device, int64_t B, int32_t L, int32_t S, int64_t q0, int64_t Q, int32_t H, const float* r,
                          const float* tproj, const float* w_r, const float* w_hh, const float* b_hn, float* hseq,
                          float* h_last, float* gates, void* stream);
 int ltgnn_gru_resident_tiles(int device, int32_t* tiles);
+int ltgnn_gru_sensor_bwd_dx(int device, int64_t B, int32_t L, int32_t S, int32_t F, int64_t q0, int64_t Q, int32_t H,
+                            const float* w_ih, const float* dG, float* dr, float* dxt, void* stream);
 
 #ifdef __cplusplus
 }

@@ -19,6 +19,7 @@
 #include "umma.cuh"
 #include "rowgemm_ts.cuh"
 #include "tgrad.cuh"
+#include "gru_dx.cuh"
 
 using namespace ltgnn;
 using namespace ltgnn::ptx;
@@ -672,4 +673,54 @@ extern "C" int ltgnn_gru_bwd_w(int device, int64_t B, int32_t L, int32_t S, int3
     int rc = tgrad::launch<2, 8, 4, 16>(device, g, x, ws, M, KA, &grid, stream, "gru_bwd_w");  // all 256 rows in one pass over X
     if (rc) return rc;
     return tgrad::gather(ws, grid, KA, 0, NG, 0, KA, dBfused, KA, 0, stream, NG);
+}
+
+// ---- input gradient (gru_dx.cuh) from the BPTT's dG: input groups r, z and in = columns 0, 1 and 3 of 4
+namespace {
+struct DgBlocked {
+    const float4* dg;  // blocked-32 [L * Qp, 4H]
+    int64_t rows;      // L * Qp
+    uint32_t Q, Qp;
+    uint64_t magic_qp;
+    __device__ __forceinline__ bool decode(int64_t row, uint32_t& q, uint32_t& t) const {
+        t = ptx::fastdiv(static_cast<uint32_t>(row), magic_qp);
+        q = static_cast<uint32_t>(row) - t * Qp;
+        return q < Q;
+    }
+    __device__ __forceinline__ float4 load(int64_t row, int g, int j4) const {
+        return ptx::ldg_stream(dg + b32(static_cast<size_t>(row), (g == 2 ? 3 : g) * (H / 4) + j4, H));
+    }
+};
+}  // namespace
+
+extern "C" int ltgnn_gru_bwd_dx(int device, int64_t B, int32_t L, int32_t S, int32_t F, int32_t Hdim, const float* w_ih,
+                                const float* dG, float* dr, float* dxt, void* stream_) {
+    LTGNN_REQUIRE(B >= 0 && L > 0 && S > 0 && F >= 0, LTGNN_E_ARG, "gru_bwd_dx: B=%lld L=%d S=%d F=%d",
+                  static_cast<long long>(B), L, S, F);
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_bwd_dx: hidden size %d not supported (64 only)", Hdim);
+    LTGNN_REQUIRE(1 + F < gru_dx::kCols, LTGNN_E_SHAPE, "gru_bwd_dx: %d time features, at most %d", F, gru_dx::kCols - 2);
+    LTGNN_REQUIRE(B * S < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_bwd_dx: too many sequences");
+    const int64_t Q = B * S, Qp = (Q + 127) / 128 * 128;
+    LTGNN_REQUIRE(Qp * L < (1ll << 31), LTGNN_E_SHAPE, "gru_bwd_dx: L*B*S=%lld rows exceed the 32-bit row index",
+                  static_cast<long long>(Qp * L));
+    if (B == 0) return LTGNN_OK;
+    LTGNN_REQUIRE(w_ih && dG && (dr || dxt) && (F > 0 || !dxt), LTGNN_E_ARG,
+                  "gru_bwd_dx: null tensor (dr or dxt required; dxt needs F > 0)");
+    LTGNN_REQUIRE(aligned16(dG) && reinterpret_cast<uintptr_t>(w_ih) % 4 == 0 && reinterpret_cast<uintptr_t>(dr) % 4 == 0 &&
+                  reinterpret_cast<uintptr_t>(dxt) % 4 == 0, LTGNN_E_ALIGN,
+                  "gru_bwd_dx: dG must be 16-byte aligned, w_ih, dr and dxt 4-byte aligned");
+    const DeviceInfo* di = device_info(device);
+    if (!di) return LTGNN_E_CUDA;
+    LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "gru_bwd_dx: device is sm_%d%d, need sm_100", di->cc_major,
+                  di->cc_minor);
+    LTGNN_USE_DEVICE(device);
+    DgBlocked lay{reinterpret_cast<const float4*>(dG), Qp * L, static_cast<uint32_t>(Q), static_cast<uint32_t>(Qp),
+                  (~0ull / static_cast<uint64_t>(Qp)) + 1};
+    auto kernel = gru_dx::gru_bwd_dx_kernel<H, DgBlocked>;
+    const size_t smem = gru_dx::smem_bytes(H);
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    kernel<<<gru_dx::grid_for(lay.rows, di->sm_count), gru_dx::kThreads, smem, static_cast<cudaStream_t>(stream_)>>>(
+        lay, w_ih, dr, dxt, static_cast<uint32_t>(S), L, F, S >= 2 ? (~0ull / static_cast<uint64_t>(S)) + 1 : 0ull);
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
 }

@@ -25,6 +25,7 @@
 // reads its step-t gx row at base[q] + t of a plane projected once per series row (ltgnn_gru_layer_fwd_windows).
 #include "umma.cuh"
 #include "rowgemm_ts.cuh"
+#include "gru_dx.cuh"
 
 using namespace ltgnn;
 using namespace ltgnn::ptx;
@@ -789,6 +790,56 @@ extern "C" int ltgnn_gru_dropout_bwd(int device, int64_t M, int32_t Hdim, const 
     gru_dropout_bwd_kernel<<<(n_words + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream_)>>>(
         reinterpret_cast<const float4*>(dy), n_parts, static_cast<size_t>(M) * (H / 4), live, keep_scale,
         reinterpret_cast<float4*>(dx), n_words);
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    return LTGNN_OK;
+}
+
+// ---- input gradient of the sensor encoder (gru_dx.cuh) from one slab's dG: input planes r, z, n = 0, 1, 2 of 4
+namespace {
+struct DgPlanarSlab {
+    const float* dg;  // [4][Q * L][H], row (q - q0) L + t
+    int64_t rows;     // Q * L
+    size_t plane;     // Q * L * H
+    uint32_t q0;
+    int L;
+    __device__ __forceinline__ bool decode(int64_t row, uint32_t& q, uint32_t& t) const {
+        const uint32_t ql = static_cast<uint32_t>(row / L);
+        t = static_cast<uint32_t>(row - static_cast<int64_t>(ql) * L);
+        q = q0 + ql;
+        return true;
+    }
+    // a thread reads its row's 512 contiguous bytes per plane: L1-allocating loads, so that the second float4 of each
+    // 32-byte sector the warp fetched is served from L1
+    __device__ __forceinline__ float4 load(int64_t row, int g, int j4) const {
+        return __ldg(reinterpret_cast<const float4*>(dg + g * plane + static_cast<size_t>(row) * H) + j4);
+    }
+};
+}  // namespace
+
+extern "C" int ltgnn_gru_sensor_bwd_dx(int device, int64_t B, int32_t L, int32_t S, int32_t F, int64_t q0, int64_t Q,
+                                       int32_t Hdim, const float* w_ih, const float* dG, float* dr, float* dxt,
+                                       void* stream_) {
+    LTGNN_REQUIRE(B > 0 && L > 0 && S > 0 && F >= 0 && q0 >= 0 && Q > 0 && q0 + Q <= B * S, LTGNN_E_ARG,
+                  "gru_sensor_bwd_dx: B=%lld L=%d S=%d F=%d q0=%lld Q=%lld", static_cast<long long>(B), L, S, F,
+                  static_cast<long long>(q0), static_cast<long long>(Q));
+    LTGNN_REQUIRE(Hdim == H, LTGNN_E_SHAPE, "gru_sensor_bwd_dx: hidden size %d not supported (128 only)", Hdim);
+    LTGNN_REQUIRE(1 + F < gru_dx::kCols, LTGNN_E_SHAPE, "gru_sensor_bwd_dx: %d time features, at most %d", F,
+                  gru_dx::kCols - 2);
+    LTGNN_REQUIRE(B * S < (1ll << 31) - 128, LTGNN_E_SHAPE, "gru_sensor_bwd_dx: too many sequences");
+    LTGNN_REQUIRE(w_ih && dG && (dr || dxt) && (F > 0 || !dxt), LTGNN_E_ARG,
+                  "gru_sensor_bwd_dx: null tensor (dr or dxt required; dxt needs F > 0)");
+    LTGNN_REQUIRE(aligned16(dG) && reinterpret_cast<uintptr_t>(w_ih) % 4 == 0 && reinterpret_cast<uintptr_t>(dr) % 4 == 0 &&
+                  reinterpret_cast<uintptr_t>(dxt) % 4 == 0, LTGNN_E_ALIGN,
+                  "gru_sensor_bwd_dx: dG must be 16-byte aligned, w_ih, dr and dxt 4-byte aligned");
+    const size_t smem = gru_dx::smem_bytes(H);
+    if (int rc = check_device(device, "gru_sensor_bwd_dx", smem)) return rc;
+    LTGNN_USE_DEVICE(device);
+    DgPlanarSlab lay{dG, Q * L, static_cast<size_t>(Q) * L * H, static_cast<uint32_t>(q0), L};
+    auto kernel = gru_dx::gru_bwd_dx_kernel<H, DgPlanarSlab>;
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    kernel<<<gru_dx::grid_for(lay.rows, device_info(device)->sm_count), gru_dx::kThreads, smem,
+             static_cast<cudaStream_t>(stream_)>>>(lay, w_ih, dr, dxt, static_cast<uint32_t>(S), L, F,
+                                                   S >= 2 ? (~0ull / static_cast<uint64_t>(S)) + 1 : 0ull);
     LTGNN_CUDA_TRY(cudaGetLastError());
     return LTGNN_OK;
 }

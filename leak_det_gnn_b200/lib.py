@@ -85,6 +85,8 @@ SIGNATURES = {
     "ltgnn_gru_ws_floats": (c_int64, [c_int]),
     "ltgnn_gru_bwd_w": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gru_bwd_dx": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                 c_void_p, c_void_p]),
     "ltgnn_gru_layer_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_void_p]),
     "ltgnn_gru_layer_fwd_train": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p,
@@ -96,6 +98,8 @@ SIGNATURES = {
     "ltgnn_gru_sensor_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int64, c_int64, c_int32, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_resident_tiles": (c_int, [c_int, c_void_p]),
+    "ltgnn_gru_sensor_bwd_dx": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int64, c_int64, c_int32, c_void_p,
+                                        c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_layer_fwd_windows": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_void_p,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),
 }

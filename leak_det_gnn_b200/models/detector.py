@@ -32,8 +32,9 @@ class SharedSensorGRUEncoder(nn.Module):
     (reference detector.py:28-73).  It feeds the hot path (SURVEY.md section 8f, rank 2): hidden size 64 runs on
     the persistent tensor-memory GRU kernel (csrc/gru.cu), hidden size 128 on the 4-CTA cluster recurrence and BPTT
     of csrc/gru_pred.cu with the time-feature projection computed once per window and step (training runs it in
-    slabs of sequences).  Other sizes, more than one layer, callers that want gradients with respect to the inputs,
-    or ``use_native = False`` take the reference's cuDNN route."""
+    slabs of sequences).  Both differentiate with respect to the parameters and to the inputs (residual and time
+    features, e.g. for saliency), each only where a gradient is asked for.  Other sizes, more than one layer, or
+    ``use_native = False`` take the reference's cuDNN route."""
 
     def __init__(self, time_dim: int = 9, hidden_size: int = 64, num_layers: int = 1, dropout: float = 0.0,
                  use_time: bool = True) -> None:
@@ -49,8 +50,7 @@ class SharedSensorGRUEncoder(nn.Module):
         if self.use_time and tfeat is None:
             raise ValueError("tfeat required when use_time=True")
         g = self.gru
-        wants_input_grad = torch.is_grad_enabled() and (r.requires_grad or (tfeat is not None and tfeat.requires_grad))
-        if (self.use_native and r.is_cuda and g.num_layers == 1 and not wants_input_grad and
+        if (self.use_native and r.is_cuda and g.num_layers == 1 and
                 ops.gru_supported(self.hidden_size, tfeat.shape[-1] if self.use_time else 0)):
             # persistent tcgen05 kernels: state in tensor memory, no per-timestep launches (csrc/gru.cu, gru_pred.cu)
             return ops.gru_encode(r, tfeat if self.use_time else None, g.weight_ih_l0, g.weight_hh_l0, g.bias_ih_l0,

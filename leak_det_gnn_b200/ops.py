@@ -816,25 +816,48 @@ def gru_fwd(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh,
     return (h_last, hseq, gates) if save else h_last
 
 
+def _dx_outputs(r: torch.Tensor, f: int, want_r: bool, want_tf: bool):
+    """(dr (B, L, S), dxt (B, L, S, F)) for ``gru_bwd_dx`` / ``gru_sensor_bwd_dx``, each only where it is asked for."""
+    dr = torch.empty_like(r) if want_r else None
+    dxt = torch.empty(*r.shape, f, device=r.device, dtype=torch.float32) if want_tf and f else None
+    return dr, dxt
+
+
+def gru_bwd_dx(dg: torch.Tensor, w_ih: torch.Tensor, r: torch.Tensor, dr: Optional[torch.Tensor],
+               dxt: Optional[torch.Tensor]) -> None:
+    """Raw input gradient at hidden 64 (see ltgnn_gru_bwd_dx) from ``ltgnn_gru_bwd_dg_hn``'s blocked-32 dG: writes
+    dr (B, L, S) and the per-sequence time-feature rows dxt (B, L, S, F) (``dxt.sum(2)`` is d tf)."""
+    b, l, s = r.shape
+    f = w_ih.shape[1] - 1
+    L = _lib.load()
+    tok = _inst.begin("gru_bwd_dx")
+    _lib.check(L.ltgnn_gru_bwd_dx(_dev_index(dg), b, l, s, f, w_ih.shape[0] // 3, w_ih.data_ptr(), dg.data_ptr(),
+                                  None if dr is None else dr.data_ptr(), None if dxt is None else dxt.data_ptr(),
+                                  _stream(dg)))
+    _inst.end(tok)
+
+
 class _GruEncoder(torch.autograd.Function):
     """h_last = GRU(cat([r_s, tf]))[:, -1] for every (window, sensor) sequence, with back-propagation through time
-    to the four GRU parameters (the inputs are data: the reference never asks for their gradient either)."""
+    to the four GRU parameters and to the inputs r and tf, each only where a gradient is asked for.  The backward runs
+    the BPTT (``ltgnn_gru_bwd_dg_hn``), then the input gradient (``ltgnn_gru_bwd_dx``) if r or tf wants one, then the
+    weight gradients (``ltgnn_gru_bwd_w``) if a parameter does: a frozen encoder pays nothing for the latter."""
 
     @staticmethod
     def forward(ctx, r, tf, w_ih, w_hh, b_ih, b_hh):
         r = r.contiguous()
         tf = None if tf is None else tf.contiguous()
         params = [t.contiguous() for t in (w_ih, w_hh, b_ih, b_hh)]
-        if any(ctx.needs_input_grad[2:]):
+        if any(ctx.needs_input_grad):
             h_last, hseq, gates = gru_fwd(r, tf, *params, save=True)
-            ctx.save_for_backward(r, tf, params[1], params[3], hseq, gates)
+            ctx.save_for_backward(r, tf, params[0], params[1], params[3], hseq, gates)
         else:  # nothing requires a gradient: backward is never reached
             h_last = gru_fwd(r, tf, *params)
         return h_last
 
     @staticmethod
     def backward(ctx, dh):
-        r, tf, w_hh, b_hh, hseq, gates = ctx.saved_tensors
+        r, tf, w_ih, w_hh, b_hh, hseq, gates = ctx.saved_tensors
         b, l, s = r.shape
         f = 0 if tf is None else tf.shape[-1]
         hd = w_hh.shape[1]
@@ -848,6 +871,12 @@ class _GruEncoder(torch.autograd.Function):
                                          hseq.data_ptr(), dh.data_ptr(), dg.data_ptr(), _stream(r)))
         _inst.end(tok)
         del gates
+        dr, dxt = _dx_outputs(r, f, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        if dr is not None or dxt is not None:
+            gru_bwd_dx(dg, w_ih, r, dr, dxt)
+        dtf = None if dxt is None else dxt.sum(2)
+        if not any(ctx.needs_input_grad[2:]):
+            return dr, dtf, None, None, None, None
         fused = torch.empty(4 * hd, 96, device=r.device, dtype=torch.float32)
         ws = torch.empty(int(L.ltgnn_gru_ws_floats(dev)), device=r.device, dtype=torch.float32)
         tok = _inst.begin("gru_bwd_w")
@@ -861,15 +890,15 @@ class _GruEncoder(torch.autograd.Function):
         dw_ih = torch.cat([rr[:, hd:kb], zz[:, hd:kb], inn[:, hd:kb]], dim=0)
         db_ih = torch.cat([rr[:, kb], zz[:, kb], inn[:, kb]], dim=0)
         db_hh = torch.cat([rr[:, kb], zz[:, kb], hn[:, kb]], dim=0)
-        return None, None, dw_ih, dw_hh, db_ih, db_hh
+        return dr, dtf, dw_ih, dw_hh, db_ih, db_hh
 
 
 def gru_encode(r: torch.Tensor, tf: Optional[torch.Tensor], w_ih, w_hh, b_ih, b_hh) -> torch.Tensor:
-    """Differentiable (wrt the parameters) shared sensor GRU: (B,L,S) [+ (B,L,F)] -> (B,S,H), H = 64 or 128."""
+    """Differentiable shared sensor GRU: (B,L,S) [+ (B,L,F)] -> (B,S,H), H = 64 or 128.  Gradients flow to the four
+    parameters and to r and tf, each only where one is asked for.  d tf is the sum over the sensors of the per-sequence
+    input gradients, taken in a fixed order once every sequence is done, so it does not depend on how the hidden-128
+    backward splits the sequences into slabs."""
     _check_act(r.contiguous(), "r")
-    if r.requires_grad or (tf is not None and tf.requires_grad):
-        raise ValueError("gru_encode: gradients with respect to the inputs are not implemented by the native GRU "
-                         "(the reference never asks for them); use the cuDNN route (use_native = False)")
     if w_hh.shape[1] == 128:
         if not torch.is_grad_enabled():   # eval, event evaluation: one launch, nothing saved
             return _SensorGru128.infer(r.contiguous(), None if tf is None else tf.contiguous(), w_ih, w_hh, b_ih, b_hh)
@@ -1254,6 +1283,20 @@ def gru_sensor_fwd(r: torch.Tensor, tproj: torch.Tensor, w_r: torch.Tensor, w_hh
     _inst.end(tok)
 
 
+def gru_sensor_bwd_dx(dg: torch.Tensor, w_ih: torch.Tensor, r: torch.Tensor, q0: int, n: int, dr: Optional[torch.Tensor],
+                      dxt: Optional[torch.Tensor]) -> None:
+    """Raw input gradient at hidden 128 of sequences q0 .. q0 + n - 1 (see ltgnn_gru_sensor_bwd_dx) from their
+    ``gru_layer_bwd`` dG [4, n * L, H]: writes their elements of dr (B, L, S) and dxt (B, L, S, F)."""
+    b, l, s = r.shape
+    f = w_ih.shape[1] - 1
+    L = _lib.load()
+    tok = _inst.begin("gru_sensor_bwd_dx")
+    _lib.check(L.ltgnn_gru_sensor_bwd_dx(_dev_index(dg), b, l, s, f, q0, n, w_ih.shape[0] // 3, w_ih.data_ptr(),
+                                         dg.data_ptr(), None if dr is None else dr.data_ptr(),
+                                         None if dxt is None else dxt.data_ptr(), _stream(dg)))
+    _inst.end(tok)
+
+
 def _sensor_x_aug(r: torch.Tensor, tf: Optional[torch.Tensor], q0: int, n: int) -> torch.Tensor:
     """[r | tf | 1 | 0 ...] (n * L, 32) for sequences q0 .. q0 + n - 1: the layer input with the ones column."""
     b, l, s = r.shape
@@ -1270,14 +1313,18 @@ def _sensor_x_aug(r: torch.Tensor, tf: Optional[torch.Tensor], q0: int, n: int) 
 
 class _SensorGru128(torch.autograd.Function):
     """The shared sensor GRU at hidden 128: h_last (B, S, 128), with back-propagation through time to the four GRU
-    parameters (the inputs are data, as in ``_GruEncoder``).
+    parameters and to the inputs r and tf, each only where a gradient is asked for.
 
-    Without gradients (grad mode off, or no parameter requires one): T (``gru_sensor_tproj``) and one recurrence launch,
+    Without gradients (grad mode off, or nothing requires one): T (``gru_sensor_tproj``) and one recurrence launch,
     nothing saved.  With gradients the sequences
     run in slabs (``gru_sensor_slabs``): each slab's training forward saves its gates and states; the backward runs per
-    slab ``gru_layer_bwd`` from that slab's rows of dh and ``gru_layer_param_grads`` against [r | tf | 1], and adds the
-    slabs' gradients in slab order.  At B = 4096, L = 288, S = 29 the saved state alone is 87.5 GB, so the backward's
-    dG and operands (96 GB more in one piece) must be formed a slab at a time."""
+    slab ``gru_layer_bwd`` from that slab's rows of dh, then ``gru_sensor_bwd_dx`` if r or tf wants a gradient and
+    ``gru_layer_param_grads`` against [r | tf | 1] if a parameter does, and adds the slabs' parameter gradients in slab
+    order.  At B = 4096, L = 288, S = 29 the saved state alone is 87.5 GB, so the backward's dG and operands (96 GB more
+    in one piece) must be formed a slab at a time.  The per-sequence time-feature gradients (F x 4 B per row, 1.2 GB
+    there) are kept for all sequences and summed over the sensors after the last slab, since a window's sensors can
+    straddle a slab boundary; the slab sizes stay those of the parameter-only backward, so asking for input gradients
+    does not change the parameter gradients' bits."""
 
     @staticmethod
     def _operands(r, tf, w_ih, w_hh, b_ih, b_hh):
@@ -1296,7 +1343,7 @@ class _SensorGru128(torch.autograd.Function):
     def forward(ctx, r, tf, w_ih, w_hh, b_ih, b_hh):
         r = r.contiguous()
         tf = None if tf is None else tf.contiguous()
-        if not any(ctx.needs_input_grad[2:]):   # nothing requires a gradient: backward is never reached
+        if not any(ctx.needs_input_grad):   # nothing requires a gradient: backward is never reached
             return _SensorGru128.infer(r, tf, w_ih, w_hh, b_ih, b_hh)
         b, l, s = r.shape
         q, hd = b * s, w_hh.shape[1]
@@ -1309,24 +1356,29 @@ class _SensorGru128(torch.autograd.Function):
             gates = torch.empty(4, n * l, hd, device=r.device, dtype=torch.float32)
             gru_sensor_fwd(r, tproj, w_r, w_hh_c, b_hn, q0, n, flat[q0:q0 + n], hseq, gates)
             saved += [hseq, gates]
-        ctx.save_for_backward(r, tf, w_hh_c, *saved)
+        ctx.save_for_backward(r, tf, w_ih.detach().contiguous(), w_hh_c, *saved)
         ctx.slabs = slabs
         return h_last
 
     @staticmethod
     def backward(ctx, dh):
-        r, tf, w_hh, *saved = ctx.saved_tensors
+        r, tf, w_ih, w_hh, *saved = ctx.saved_tensors
         l = r.shape[1]
         f = 0 if tf is None else tf.shape[-1]
         dh = dh.contiguous().view(-1, w_hh.shape[1])
-        grads = None
+        dr, dxt = _dx_outputs(r, f, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        want_w = any(ctx.needs_input_grad[2:])
+        grads = [None] * 4
         for i, (q0, n) in enumerate(ctx.slabs):
             hseq, gates = saved[2 * i], saved[2 * i + 1]
             dg = gru_layer_bwd(n, l, w_hh, gates, hseq, dh_last=dh[q0:q0 + n])
-            part = gru_layer_param_grads(dg, hseq, _sensor_x_aug(r, tf, q0, n), 1 + f, n, l)
+            if dr is not None or dxt is not None:
+                gru_sensor_bwd_dx(dg, w_ih, r, q0, n, dr, dxt)
+            if want_w:
+                part = gru_layer_param_grads(dg, hseq, _sensor_x_aug(r, tf, q0, n), 1 + f, n, l)
+                grads = part if i == 0 else [a + p for a, p in zip(grads, part)]
             del dg
-            grads = part if grads is None else [a + p for a, p in zip(grads, part)]
-        return (None, None, *grads)
+        return (dr, None if dxt is None else dxt.sum(2), *grads)
 
 
 def tcn_conv(x: torch.Tensor, src: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor,
