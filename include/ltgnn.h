@@ -395,6 +395,20 @@ int ltgnn_gru_resident_tiles(int device, int32_t* tiles);
 int ltgnn_gru_sensor_bwd_dx(int device, int64_t B, int32_t L, int32_t S, int32_t F, int64_t q0, int64_t Q, int32_t H,
                             const float* w_ih, const float* dG, float* dr, float* dxt, void* stream);
 
+/* ---- deterministic sum of gathered rows (csrc/gather_sum.cu) -------------------------------------------------------
+ * For every plane p < planes and row r < rows:
+ *   out[p * out_plane_stride + r * C + c] = sum_{e = ptr[r]} ^ {ptr[r+1] - 1} src[p * src_plane_stride + idx[e] * C + c]
+ * fp32 adds in ascending e from zero (an empty row is zeros): no atomics, bitwise deterministic.  ptr int32 [rows + 1]
+ * non-decreasing and idx int32 [ptr[rows]] are the transpose of a gather as a CSR; the caller guarantees that every idx
+ * is a row of src (the entry point does not read device memory).  The input-gradient backward of rows several readers
+ * gathered (the frozen predictor's shared windows).  C % 4 == 0 and rows < 2^31 - 1 (else LTGNN_E_SHAPE); rows >= 0,
+ * C > 0, 1 <= planes <= 65535, strides >= 0 and src, ptr, idx, out non-NULL (else LTGNN_E_ARG); src and out 16-byte
+ * aligned, the plane strides (in floats) multiples of 4, ptr and idx 4-byte aligned (else LTGNN_E_ALIGN).  No
+ * allocation or host synchronisation: capturable into a CUDA graph.
+ */
+int ltgnn_row_gather_sum(int device, int64_t rows, int32_t C, int32_t planes, const float* src, int64_t src_plane_stride,
+                         const int32_t* ptr, const int32_t* idx, float* out, int64_t out_plane_stride, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -102,6 +102,8 @@ SIGNATURES = {
                                         c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gru_layer_fwd_windows": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_void_p,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_row_gather_sum": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
+                                     c_int64, c_void_p]),
 }
 
 _lib = None

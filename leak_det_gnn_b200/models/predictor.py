@@ -9,7 +9,10 @@ rank 1).  It contains no graph layers (SURVEY F1).  ``state_dict`` keys equal th
 ``forward`` is the reference's dense evaluation (every time step of every layer); ``forward_last`` evaluates only the
 dependency cone of the last time step -- the only one the model reads (predictor.py:80): 99 instead of 288
 convolution evaluations per window -- and is what the residual builder (models/utils.py) calls.  ``forward_cone`` is
-the same cone, differentiable: what ``train_predictor_dp`` trains with.
+the same cone, differentiable: what ``train_predictor_dp`` trains with.  ``forward_windows`` evaluates every window of a
+series from rows computed once; with gradients asked for the inputs of a frozen predictor it is differentiable with
+respect to them (``differentiable_windows``), which takes the gradient of the detector's logits back to the raw
+sensor series.
 """
 from __future__ import annotations
 
@@ -18,6 +21,14 @@ from typing import List, Tuple
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+
+
+def _differentiable_windows(model: nn.Module, x: torch.Tensor, x_time: torch.Tensor) -> bool:
+    """Whether ``forward_windows(x, x_time, ...)`` returns a result differentiable with respect to x and x_time: grad mode
+    on, x or x_time requiring grad, the native shared path, and a frozen predictor (no parameter requiring grad: the
+    node computes no parameter gradient).  Otherwise ``forward_windows`` runs without gradients."""
+    return (torch.is_grad_enabled() and (x.requires_grad or x_time.requires_grad) and model.share_windows
+            and model._native_ok(x) and not any(p.requires_grad for p in model.parameters()))
 
 
 class CausalConv1d(nn.Module):
@@ -90,18 +101,35 @@ class NormalPredictorTCN(nn.Module):
             return self._forward_last_native(x, x_time)
         return self._cone_torch(x, x_time)
 
-    @torch.no_grad()
+    differentiable_windows = _differentiable_windows
+
     def forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, count=None) -> torch.Tensor:
         """``forward_last`` of every window of ``window`` steps: x (B, T, S), x_time (B, T, F) -> (B, n, S) with
         ``out[b, j] = forward_last(x[b, j:j + window], x_time[b, j:j + window])``, n = count or T - window + 1.
         On the native path a row of convolution i at window position p >= R_i (the cumulative left reach of convolutions
         0..i) reads no left padding, so it is the same in every window that contains its step: it is computed once per
         (series, step), the input projection once per series row, and only the rows near each window's left edge per
-        window (``shared_cone_plan``); the result equals ``forward_last`` on the materialised windows bit for bit."""
+        window (``shared_cone_plan``); the result equals ``forward_last`` on the materialised windows bit for bit.
+        When ``differentiable_windows`` holds, the same values come from ONE autograd node (``ops.tcn_windows``) whose
+        backward gives d x and d x_time through the shared rows (``_shared_readers``); otherwise no gradient."""
         if self.training:
             raise RuntimeError("forward_windows is the inference path of the frozen predictor (call .eval() first)")
         b, length, _ = x.shape
         n = _window_count(length, window, count)
+        if self.differentiable_windows(x, x_time):
+            from .. import ops
+
+            dev = x.device
+            norms = [(blk.conv1.conv.bias, blk.norm1.weight, blk.norm1.bias, blk.norm1.eps, blk.conv2.conv.bias,
+                      blk.norm2.weight, blk.norm2.bias, blk.norm2.eps) for blk in self.tcn]
+            return ops.tcn_windows(self._native_input(x, x_time), self._shared_rows(length, window, n, b, dev),
+                                   self._shared_readers(length, window, n, b, dev), self._native_weights(dev), norms,
+                                   self.num_sensors).view(b, n, -1)
+        with torch.no_grad():
+            return self._forward_windows(x, x_time, window, n)
+
+    def _forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, n: int) -> torch.Tensor:
+        b, length, _ = x.shape
         if not (self.share_windows and self._native_ok(x)):
             return self.forward_last(windows_of(x, window, n), windows_of(x_time, window, n)).view(b, n, -1)
         from .. import ops
@@ -247,6 +275,30 @@ class NormalPredictorTCN(nn.Module):
         cache[key] = out
         return out
 
+    def _shared_readers(self, length: int, window: int, count: int, batch: int, device):
+        """The transposes of ``_shared_rows`` for the input gradients (``shared_reader_plan``), int32 on ``device``, per
+        block (ptr1, idx1, ptr2, idx2, ptr_res, idx_res, ident1, ident2, ident_res): ident (taps, n) = tap n + r, the
+        gather of ``tcn_conv`` over the stacked per-tap sums, and ident_res = arange(n) its residual rows.  Built on the
+        host once per shape and device, like ``_shared_rows``: outside CUDA-graph capture."""
+        cache = self.__dict__.setdefault("_shared_rd", {})
+        key = (length, window, count, batch, str(device))
+        if key in cache:
+            return cache[key]
+        plan, _ = shared_cone_plan(length, window, count, batch, self.tcn[0].conv1.conv.kernel_size[0],
+                                   [blk.conv1.conv.dilation[0] for blk in self.tcn])
+        out = []
+        n_in = batch * length
+        for (src1, _, res_row), csr in zip(plan, shared_reader_plan(plan, n_in)):
+            ks, n_mid = src1.shape
+            ident = [torch.arange(ks * n, dtype=torch.int64).view(ks, n) for n in (n_in, n_mid)]
+            out.append(tuple(t.to(device=device, dtype=torch.int32).contiguous()
+                             for t in (*csr, *ident, torch.arange(n_in))))
+            n_in = res_row.numel()
+        if len(cache) > 8:
+            cache.clear()
+        cache[key] = out
+        return out
+
     def _native_inverse(self, length: int, batch: int, device):
         """Inverses of ``_native_rows`` for the input gradients: per block (inv1, inv2, keep_inv), inv int32 (taps, rows
         of the convolution's input) = the output row that reads input row r through that tap, or -1; keep_inv int32
@@ -354,17 +406,36 @@ class NormalPredictorGRU(nn.Module):
         h = ops.gru_predictor_fwd(x, x_time, prep["layers"])
         return ops.linear_tc(h, prep["w_out"], prep["b_out"])[:, :self.num_sensors]
 
-    @torch.no_grad()
+    differentiable_windows = _differentiable_windows
+
     def forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, count=None) -> torch.Tensor:
         """``forward_last`` of every window of ``window`` steps: x (B, T, S), x_time (B, T, F) -> (B, n, S) with
         ``out[b, j] = forward_last(x[b, j:j + window], x_time[b, j:j + window])``, n = count or T - window + 1.
         Every window restarts the recurrence from a zero state, so only layer 0's input projection is shared: on the
         native path it is computed once per series row and window (b, j) reads rows b T + j .. + window - 1 of it
-        (``ops.gru_predictor_windows``), bit for bit the result on the materialised windows."""
+        (``ops.gru_predictor_windows``), bit for bit the result on the materialised windows.  When
+        ``differentiable_windows`` holds, the same values come from ONE autograd node (``ops.gru_windows``) whose
+        backward gives d x and d x_time (layer 0's gradient summed over the windows into series rows, ``_window_readers``);
+        otherwise no gradient."""
         if self.training:
             raise RuntimeError("forward_windows is the inference path of the frozen predictor (call .eval() first)")
         b, length, _ = x.shape
         n = _window_count(length, window, count)
+        if self.differentiable_windows(x, x_time):
+            from .. import ops
+
+            prep = self._native_weights(x.device)
+            k0 = prep["layers"][0][0].shape[2]
+            inp = torch.zeros(b, length, k0, device=x.device, dtype=torch.float32)
+            inp[:, :, :self.num_sensors] = x
+            inp[:, :, self.num_sensors:self.num_sensors + self.time_dim] = x_time
+            return ops.gru_windows(inp.view(b * length, k0), window, self._window_readers(length, window, n, b, x.device),
+                                   prep, self.num_sensors).view(b, n, -1)
+        with torch.no_grad():
+            return self._forward_windows(x, x_time, window, n)
+
+    def _forward_windows(self, x: torch.Tensor, x_time: torch.Tensor, window: int, n: int) -> torch.Tensor:
+        b, length, _ = x.shape
         if not (self.share_windows and self._native_ok(x)):
             return self.forward_last(windows_of(x, window, n), windows_of(x_time, window, n)).view(b, n, -1)
         from .. import ops
@@ -410,6 +481,23 @@ class NormalPredictorGRU(nn.Module):
         prep = {"layers": layers, "w_out": w_out, "b_out": b_out}
         cache.update(ver=ver, prep=prep)
         return prep
+
+    def _window_readers(self, length: int, window: int, count: int, batch: int, device):
+        """(gather, ptr, idx) on ``device``: gather int64 (B * count * window,) = the series row b T + j + p of window row
+        (b count + j) window + p, and its transpose ``window_reader_csr`` as int32.  Built on the host once per shape and
+        device: outside CUDA-graph capture."""
+        cache = self.__dict__.setdefault("_window_rd", {})
+        key = (length, window, count, batch, str(device))
+        if key in cache:
+            return cache[key]
+        bs = torch.arange(batch).view(-1, 1, 1)
+        gather = (bs * length + torch.arange(count).view(1, -1, 1) + torch.arange(window).view(1, 1, -1)).reshape(-1)
+        ptr, idx = window_reader_csr(length, window, count, batch)
+        out = (gather.to(device), ptr.to(device=device, dtype=torch.int32), idx.to(device=device, dtype=torch.int32))
+        if len(cache) > 8:
+            cache.clear()
+        cache[key] = out
+        return out
 
 
 def cone_positions(length: int, kernel_size: int, dilations: List[int]) -> List[Tuple[List[int], List[int]]]:
@@ -528,3 +616,42 @@ def shared_cone_plan(length: int, window: int, count: int, batch: int, kernel_si
     # the head reads the last pool as is: one row per window, window-major
     assert (pool.n_w, pool.n_s) == (1, 0) or (pool.n_w == 0 and torch.equal(pool.steps, torch.arange(count) + window - 1))
     return plan, shared
+
+
+def reader_csr(keys: torch.Tensor, vals: torch.Tensor, n_rows: int):
+    """The transpose of a gather as a CSR: row r lists vals[e] for every e with keys[e] == r, in the order of e; keys < 0
+    (left padding) are not listed.  keys, vals 1-D int64 -> (ptr (n_rows + 1,), idx) int64 on the CPU."""
+    ok = keys >= 0
+    keys, vals = keys[ok], vals[ok]
+    ptr = torch.zeros(n_rows + 1, dtype=torch.int64)
+    ptr[1:] = torch.cumsum(torch.bincount(keys, minlength=n_rows), 0)
+    return ptr, vals[torch.sort(keys, stable=True).indices]
+
+
+def shared_reader_plan(plan, n_input_rows: int):
+    """Who reads each row of ``shared_cone_plan``'s pools, for the input gradients: per block (ptr1, idx1, ptr2, idx2,
+    ptr_res, idx_res) int64 CSRs.  Convolution c's CSR has one row per (tap, row of its input pool), tap n_src + r, listing
+    in ascending order the output rows m with src[tap, m] == r; the residual's has one row per block input row, listing
+    the m with res_row[m] == r.  These maps are not injective: a shared row near a window's left edge is read through
+    one tap by windowed rows of several neighbouring windows.  ``n_input_rows``: pool -1's rows, B * T."""
+    out = []
+    n_in = n_input_rows
+    for src1, src2, res_row in plan:
+        csr = []
+        for src, n_src in ((src1, n_in), (src2, src1.shape[1])):
+            ks, m = src.shape
+            keys = torch.where(src >= 0, src + torch.arange(ks, dtype=torch.int64).view(-1, 1) * n_src, -1)
+            csr += reader_csr(keys.reshape(-1), torch.arange(m, dtype=torch.int64).repeat(ks), ks * n_src)
+        csr += reader_csr(res_row, torch.arange(res_row.numel(), dtype=torch.int64), n_in)
+        out.append(tuple(csr))
+        n_in = res_row.numel()
+    return out
+
+
+def window_reader_csr(length: int, window: int, count: int, batch: int):
+    """The windows that read each series row: the CSR over series rows b T + t listing the window rows
+    (b count + j) window + (t - j), 0 <= t - j < window, in ascending j.  int64 (ptr, idx) on the CPU."""
+    bs = torch.arange(batch).view(-1, 1, 1)
+    js = torch.arange(count).view(1, -1, 1)
+    ps = torch.arange(window).view(1, 1, -1)
+    return reader_csr((bs * length + js + ps).reshape(-1), ((bs * count + js) * window + ps).reshape(-1), batch * length)

@@ -17,6 +17,12 @@ def _shares_windows(predictor: Any) -> bool:
             and not predictor.training and not torch.is_grad_enabled())
 
 
+def _differentiates_windows(predictor: Any, noisy_seg: torch.Tensor, time_seg: torch.Tensor) -> bool:
+    """A frozen predictor in eval mode whose ``forward_windows`` is differentiable with respect to these inputs."""
+    diff = getattr(predictor, "differentiable_windows", None)
+    return diff is not None and not predictor.training and diff(noisy_seg, time_seg)
+
+
 def build_residual_sequence_from_segment(predictor: Any, noisy_seg: torch.Tensor, time_seg: torch.Tensor, l_pred: int,
                                          l_det: int, device: Optional[Any] = None) -> torch.Tensor:
     """Residual sequence for the detector from a (l_pred + l_det)-step segment: same arguments, result and window
@@ -27,7 +33,10 @@ def build_residual_sequence_from_segment(predictor: Any, noisy_seg: torch.Tensor
     are one strided view of the segment, and a frozen TCN predictor is evaluated only on the dependency cone of its
     last time step (``NormalPredictorTCN.forward_last``: 99 instead of 288 convolution evaluations per window).
     A predictor with ``forward_windows`` and ``share_windows`` on runs the l_det windows of every segment in one call that
-    computes what they share once (no window is materialised), with the same result bit for bit."""
+    computes what they share once (no window is materialised), with the same result bit for bit.  It does so under
+    autograd too when the segment requires grad and the predictor is frozen (``differentiable_windows``): the residual
+    is then differentiable with respect to ``noisy_seg`` and ``time_seg`` through the shared windows; with
+    ``share_windows`` off the dense ``predictor(x, t)`` on the materialised windows gives the same gradients."""
     squeeze_back = noisy_seg.dim() == 2
     if squeeze_back:
         noisy_seg, time_seg = noisy_seg.unsqueeze(0), time_seg.unsqueeze(0)
@@ -36,7 +45,7 @@ def build_residual_sequence_from_segment(predictor: Any, noisy_seg: torch.Tensor
     if device is not None:
         noisy_seg, time_seg = noisy_seg.to(device), time_seg.to(device)
 
-    if _shares_windows(predictor):
+    if _shares_windows(predictor) or _differentiates_windows(predictor, noisy_seg, time_seg):
         y_hat = predictor.forward_windows(noisy_seg, time_seg, l_pred, count=l_det)              # (B, l_det, S)
         residual = noisy_seg[:, l_pred:, :] - y_hat
         return residual.squeeze(0) if squeeze_back else residual

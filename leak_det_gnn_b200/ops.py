@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -1091,6 +1091,19 @@ def gru_dropout_bwd(parts: torch.Tensor, live: Optional[torch.Tensor], drop_p: f
     return dx
 
 
+def gru_input_grad(dg: torch.Tensor, w_x: torch.Tensor) -> torch.Tensor:
+    """``sum_g dG[g] @ W_x[g]`` over the input planes r, z, n: dG (>= 3, M, H), W_x (3, H, K) (layer 0's
+    ``gru_predictor_weights`` entry, K zero-padded) -> (M, K).  One ``linear_tc`` per plane; the planes are added in
+    index order by ``gru_dropout_bwd`` over a 128-wide view of the K-wide parts (the tail past M K is zero)."""
+    m, k = dg.shape[1], w_x.shape[2]
+    n = m * k
+    flat = torch.empty(3, (n + 127) // 128 * 128, device=dg.device, dtype=torch.float32)
+    flat[:, n:] = 0.0
+    for g in range(3):
+        linear_tc(dg[g], w_x[g], transposed=True, out=flat[g, :n])
+    return gru_dropout_bwd(flat.view(3, -1, 128), None, 0.0).view(-1)[:n].view(m, k)
+
+
 def unpack_gru_live(live: torch.Tensor) -> torch.Tensor:
     """int32 (M, H / 32) -> bool (M, H): the units ``gru_dropout`` kept (tests and debugging)."""
     bits = (live.unsqueeze(-1) >> torch.arange(32, device=live.device, dtype=torch.int32)) & 1
@@ -1126,7 +1139,7 @@ def gru_layer_param_grads(dg: torch.Tensor, hseq: torch.Tensor, x_aug: torch.Ten
 
 class _GruPredictor(torch.autograd.Function):
     """The GRU predictor -- every layer and the head on the last step -- as ONE autograd node: gradients for all GRU and
-    head parameters (the inputs are data).
+    head parameters, and for the input rows when they require grad (``gru_input_grad`` of layer 0's dG).
 
     Forward per layer: input projection (``linear_tc``, b_hr and b_hz folded), the recurrence saving its gates, and for
     every layer but the last the inter-layer dropout.  Backward per layer, top down: BPTT -> dG; dW_hh and d b_hh from
@@ -1168,6 +1181,7 @@ class _GruPredictor(torch.autograd.Function):
                               *[lv for lv in lives if lv is not None])
         ctx.q, ctx.l, ctx.c_in, ctx.n_sensors, ctx.n_layers, ctx.p = q, l, c_in, n_sensors, n_layers, p
         ctx.has_live = [lv is not None for lv in lives]
+        ctx.w_x0 = layers[0][0]                     # layer 0's W_ih per gate group, zero-padded to the input's width
         return pred
 
     @staticmethod
@@ -1183,13 +1197,15 @@ class _GruPredictor(torch.autograd.Function):
         dp[:, :s] = dpred
         t_head = wgrad(dp, _ones_aug(h_last, hdim + 32))
         dh_last = linear_tc(dp[:, :w_out.shape[0]].contiguous(), w_out, transposed=True)
-        dh_seq = None
+        dh_seq = d_inp = None
         grads = [None] * (4 * n)
         for i in range(n - 1, -1, -1):
             x, hseq, gates, w_hh, w_ih3 = saved[i]
             dg = gru_layer_bwd(q, l, w_hh, gates, hseq, dh_last=dh_last, dh_seq=dh_seq)
             if i == 0:
                 grads[0:4] = gru_layer_param_grads(dg, hseq, x, ctx.c_in, q, l)   # layer 0's input carries the ones
+                if ctx.needs_input_grad[0]:
+                    d_inp = gru_input_grad(dg, ctx.w_x0)
             else:
                 grads[4 * i:4 * i + 4] = gru_layer_param_grads(dg, hseq, _ones_aug(x, hdim + 32), hdim, q, l)
             if i > 0:
@@ -1199,7 +1215,8 @@ class _GruPredictor(torch.autograd.Function):
                 dh_seq = gru_dropout_bwd(parts, lives[i - 1], ctx.p)
                 dh_last = None
             del dg
-        return (None, None, None, None, None, None, *grads, t_head[:s, :hdim].contiguous(), t_head[:s, hdim].contiguous())
+        return (d_inp, None, None, None, None, None, *grads, t_head[:s, :hdim].contiguous(),
+                t_head[:s, hdim].contiguous())
 
 
 def gru_predictor_cone(x: torch.Tensor, x_time: torch.Tensor, drop_p: float, params) -> torch.Tensor:
@@ -1492,7 +1509,8 @@ def tcn_wgrad(dz: torch.Tensor, x: torch.Tensor, src: torch.Tensor) -> torch.Ten
 
 class _TcnCone(torch.autograd.Function):
     """The TCN predictor's cone as ONE autograd node: input projection -> per block two training convolutions (the
-    second with the residual) -> head on the last position; gradients for all parameters (the inputs are data).
+    second with the residual) -> head on the last position; gradients for all parameters, and for the input rows when
+    they require grad (the input projection's ``dh`` times its padded weight).
 
     Backward per convolution: epilogue backward (dz and the LayerNorm / bias column sums), weight gradient over the
     gathered rows, input gradient as the forward's gathered GEMM with the inverse index and the per-tap transposed
@@ -1527,14 +1545,14 @@ class _TcnCone(torch.autograd.Function):
         b_out = torch.zeros(n_pad, device=inp.device, dtype=torch.float32)
         b_out[:n_sensors] = b_head
         pred = linear_tc(h, w_out, b_out)[:, :n_sensors]
-        ctx.save_for_backward(inp, h, w_out, *saved)
+        ctx.save_for_backward(inp, h, w_out, w_in_p, *saved)
         ctx.rows, ctx.inv, ctx.n_blk, ctx.c_in, ctx.n_sensors = rows, inv, n_blk, c_in, n_sensors
         ctx.scale = 1.0 / (1.0 - p)
         return pred
 
     @staticmethod
     def backward(ctx, dpred):
-        inp, h_last, w_out, *saved = ctx.saved_tensors
+        inp, h_last, w_out, w_in_p, *saved = ctx.saved_tensors
         s, c = ctx.n_sensors, h_last.shape[1]
         bsz = h_last.shape[0]
         dp = torch.zeros(bsz, 64, device=dpred.device, dtype=torch.float32)   # wgrad_tc takes 64 or 128 output rows
@@ -1561,7 +1579,8 @@ class _TcnCone(torch.autograd.Function):
         t_in = wgrad(dh, inp)
         d_w_in = t_in[:, :ctx.c_in].unsqueeze(-1)
         d_b_in = t_in[:, ctx.c_in].contiguous()
-        return (None, None, None, None, None, None, d_w_in, d_b_in, *grads, t_head[:s, :c].contiguous(),
+        d_inp = linear_tc(dh, w_in_p, transposed=True) if ctx.needs_input_grad[0] else None
+        return (d_inp, None, None, None, None, None, d_w_in, d_b_in, *grads, t_head[:s, :c].contiguous(),
                 t_head[:s, c].contiguous())
 
 
@@ -1579,3 +1598,155 @@ def tcn_cone(x: torch.Tensor, x_time: torch.Tensor, rows, inv, drop_p: float, ep
     inp.view(b, length, kp)[:, :, s:c_in] = x_time
     inp[:, c_in] = 1.0
     return _TcnCone.apply(inp, rows, inv, s, float(drop_p), float(eps), *params)
+
+
+# ----------------------------------------------------------------------------------------------
+# input gradients of the frozen predictor's shared windows (``forward_windows`` under autograd): the rows several windows
+# read receive the sum of their readers' gradients (csrc/gather_sum.cu)
+# ----------------------------------------------------------------------------------------------
+def row_gather_sum(src: torch.Tensor, ptr: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
+    """Raw deterministic sum of gathered rows (see ltgnn_row_gather_sum): src (R, C) or planes (P, R, C) fp32 CUDA, C % 4
+    == 0; ptr int32 (rows + 1,), idx int32 a CSR whose every entry is a row of src (the host plans build them so) ->
+    (rows, C) or (P, rows, C), ``out[.., r] = sum_{e = ptr[r]} ^ {ptr[r+1] - 1} src[.., idx[e]]`` in ascending e."""
+    _check_act(src, "src")
+    for t, nm in ((ptr, "ptr"), (idx, "idx")):
+        if t.dtype != torch.int32 or not t.is_cuda or not t.is_contiguous() or t.dim() != 1:
+            raise ValueError(f"{nm} must be a contiguous 1-D int32 CUDA tensor")
+    if src.dim() not in (2, 3):
+        raise ValueError(f"src must be (rows, C) or (planes, rows, C), got {tuple(src.shape)}")
+    planes = src.shape[0] if src.dim() == 3 else 1
+    r_in, c = src.shape[-2], src.shape[-1]
+    rows = ptr.numel() - 1
+    if idx.numel() == 0:                            # no row has a reader: the sums are zeros
+        return torch.zeros(*src.shape[:-2], rows, c, device=src.device, dtype=torch.float32)
+    out = torch.empty(*src.shape[:-2], rows, c, device=src.device, dtype=torch.float32)
+    L = _lib.load()
+    tok = _inst.begin("row_gather_sum")
+    _lib.check(L.ltgnn_row_gather_sum(_dev_index(src), rows, c, planes, src.data_ptr(), r_in * c, ptr.data_ptr(),
+                                      idx.data_ptr(), out.data_ptr(), rows * c, _stream(src)))
+    _inst.end(tok)
+    return out
+
+
+class _TcnWindows(torch.autograd.Function):
+    """Every window of the frozen TCN predictor from the shared plan (``NormalPredictorTCN.forward_windows``) as ONE
+    autograd node, differentiable with respect to its input rows only.
+
+    Forward: ``_native_stack`` with each convolution through ``tcn_conv_train`` at drop_p = 0 (the same values bit for
+    bit), saving z, the row statistics and the live mask.  Backward per block, from the last: epilogue backward -> dz;
+    per tap the gather-sum of dz into the rows of the convolution's input pool (the reader CSRs: a shared row is read
+    through one tap by several windows); one ``tcn_conv`` over the stacked per-tap sums with an identity gather and the
+    per-tap transposed weights; the block input also receives the gather-sum of the block output's gradient through the
+    residual CSR.  Last, the input projection's transpose.  No weight gradient is computed."""
+
+    @staticmethod
+    def forward(ctx, inp, rows, readers, prep, norms, n_sensors):
+        h = linear_tc(inp, prep["w_in"], prep["b_in"])
+        saved, lives = [], []
+        for (w1, w2), (src1, src2, keep), (b1, g1, e1, eps1, b2, g2, e2, eps2) in zip(prep["convs"], rows, norms):
+            y1, z1, s1, l1 = tcn_conv_train(h, src1, w1, b1, g1, e1, eps1)
+            h, z2, s2, l2 = tcn_conv_train(y1, src2, w2, b2, g2, e2, eps2, res=h, res_row=keep)
+            saved += [z1, s1, l1, z2, s2, l2]
+            lives += [l1, l2]
+        if DEBUG_CAPTURE is not None:
+            DEBUG_CAPTURE["tcn_lives"] = lives
+        ctx.save_for_backward(*saved)
+        ctx.readers, ctx.prep, ctx.norms, ctx.n_sensors = readers, prep, norms, n_sensors
+        return linear_tc(h, prep["w_out"], prep["b_out"])[:, :n_sensors]
+
+    @staticmethod
+    def backward(ctx, dpred):
+        saved, prep = ctx.saved_tensors, ctx.prep
+        w_out = prep["w_out"]
+        dp = torch.zeros(dpred.shape[0], w_out.shape[0], device=dpred.device, dtype=torch.float32)
+        dp[:, :ctx.n_sensors] = dpred
+        dh = linear_tc(dp, w_out, transposed=True)
+        zero_bias = torch.zeros(dh.shape[1], device=dh.device, dtype=torch.float32)
+        for i in range(len(prep["convs"]) - 1, -1, -1):
+            z1, s1, l1, z2, s2, l2 = saved[6 * i:6 * i + 6]
+            w1, w2 = prep["convs"][i]
+            g1, g2 = ctx.norms[i][1], ctx.norms[i][5]
+            ptr1, idx1, ptr2, idx2, ptr_r, idx_r, ident1, ident2, ident_r = ctx.readers[i]
+            dz2 = tcn_ln_bwd(dh, l2, z2, s2, g2, 1.0)[0]
+            dy1 = tcn_conv(row_gather_sum(dz2, ptr2, idx2), ident2, w2.transpose(1, 2).contiguous(), zero_bias,
+                           relu=False)
+            dz1 = tcn_ln_bwd(dy1, l1, z1, s1, g1, 1.0)[0]
+            dh = tcn_conv(row_gather_sum(dz1, ptr1, idx1), ident1, w1.transpose(1, 2).contiguous(), zero_bias,
+                          relu=False, res=row_gather_sum(dh, ptr_r, idx_r), res_row=ident_r)
+        return linear_tc(dh, prep["w_in"], transposed=True), None, None, None, None, None
+
+
+def tcn_windows(inp: torch.Tensor, rows, readers, prep, norms, n_sensors: int) -> torch.Tensor:
+    """Differentiable ``forward_windows`` of a frozen TCN predictor: inp (B * T, 64) the zero-padded input rows ->
+    (B * count, n_sensors).  ``rows`` / ``readers``: NormalPredictorTCN._shared_rows / _shared_readers; ``prep``: its
+    _native_weights; ``norms``: per block (conv1 bias, norm1 weight, bias, eps, conv2 bias, norm2 weight, bias, eps)."""
+    _check_act(inp.detach(), "inp")
+    return _TcnWindows.apply(inp, rows, readers, prep, norms, n_sensors)
+
+
+class _GruWindows(torch.autograd.Function):
+    """Every window of the frozen GRU predictor (``NormalPredictorGRU.forward_windows``) as ONE autograd node,
+    differentiable with respect to its input rows only.
+
+    Forward: layer 0 projects the B * T series rows once (as ``gru_predictor_windows``), each window's rows of that
+    projection are gathered into the planar form and every layer runs ``gru_layer_fwd_train`` (the inference recurrence's
+    values bit for bit), saving its gates.  Backward: BPTT per layer, top down (upper layers take sum_g dG[g] W_ih[g]);
+    layer 0's dG planes r, z, n are gather-summed over the windows into series rows (the window CSR), and one
+    ``gru_input_grad`` on B * T rows instead of B * count * window gives the input rows' gradient."""
+
+    @staticmethod
+    def forward(ctx, inp, window, readers, prep, n_sensors):
+        gather, ptr, idx = readers
+        layers = prep["layers"]
+        w_x, b_x, w_hh, b_hn = layers[0]
+        hdim = w_hh.shape[1]
+        q = gather.numel() // window
+        gx = torch.empty(3, inp.shape[0], hdim, device=inp.device, dtype=torch.float32)
+        for g in range(3):
+            linear_tc(inp, w_x[g], b_x[g], out=gx[g])
+        gx = gx.index_select(1, gather)                         # (3, Q * window, H): window (b, j) at rows of b T + j ..
+        saved = []
+        for i, (w_x, b_x, w_hh, b_hn) in enumerate(layers):
+            if i > 0:
+                gx = torch.empty(3, q * window, hdim, device=inp.device, dtype=torch.float32)
+                for g in range(3):
+                    linear_tc(hseq, w_x[g], b_x[g], out=gx[g])
+            h_last, hseq, gates = gru_layer_fwd_train(gx, q, window, w_hh, b_hn)
+            del gx
+            saved += [hseq, gates]
+        ctx.save_for_backward(*saved)
+        ctx.window, ctx.readers, ctx.prep, ctx.n_sensors = window, readers, prep, n_sensors
+        return linear_tc(h_last, prep["w_out"], prep["b_out"])[:, :n_sensors]
+
+    @staticmethod
+    def backward(ctx, dpred):
+        saved, prep, l = ctx.saved_tensors, ctx.prep, ctx.window
+        _, ptr, idx = ctx.readers
+        layers = prep["layers"]
+        w_out = prep["w_out"]
+        q = dpred.shape[0]
+        dp = torch.zeros(q, w_out.shape[0], device=dpred.device, dtype=torch.float32)
+        dp[:, :ctx.n_sensors] = dpred
+        dh_last, dh_seq = linear_tc(dp, w_out, transposed=True), None
+        for i in range(len(layers) - 1, -1, -1):
+            w_x, _, w_hh, _ = layers[i]
+            hseq, gates = saved[2 * i], saved[2 * i + 1]
+            dg = gru_layer_bwd(q, l, w_hh, gates, hseq, dh_last=dh_last, dh_seq=dh_seq)
+            if i > 0:
+                parts = torch.empty(3, q * l, w_hh.shape[1], device=dg.device, dtype=torch.float32)
+                for g in range(3):
+                    linear_tc(dg[g], w_x[g], transposed=True, out=parts[g])
+                dh_seq, dh_last = gru_dropout_bwd(parts, None, 0.0), None
+                del parts
+            else:
+                d_inp = gru_input_grad(row_gather_sum(dg[:3], ptr, idx), w_x)
+            del dg
+        return d_inp, None, None, None, None
+
+
+def gru_windows(inp: torch.Tensor, window: int, readers, prep, n_sensors: int) -> torch.Tensor:
+    """Differentiable ``forward_windows`` of a frozen GRU predictor: inp (B * T, 64) the zero-padded input rows ->
+    (B * count, n_sensors).  ``readers``: NormalPredictorGRU._window_readers (the forward gather of the window rows and
+    its transpose as a CSR); ``prep``: its _native_weights."""
+    _check_act(inp.detach(), "inp")
+    return _GruWindows.apply(inp, window, readers, prep, n_sensors)
