@@ -112,6 +112,40 @@ int ltgnn_spmm_fused(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const
                      float gate_scale, float* colsum, float* ws, uint32_t* live_out, const uint32_t* live_in,
                      void* stream);
 
+/* ---- weighted adjacency: per-call edge weights (PyG's GCNConv edge_weight) ------------------------------------
+ * ltgnn_spmm_fused_vals: ltgnn_spmm_fused (and ltgnn_spmm through algo, with no fused part) with the entry values
+ *   read from vals[b * vals_stride + k] instead of the handle: vals [1 or B][nnz] in the order of the chosen orientation
+ *   (A_hat's rows for transpose = 0, A_hat^T's for transpose = 1), vals_stride 0 (one set shared by every window) or
+ *   nnz.  Column indices and the summation order are the handle's.  algo as in ltgnn_spmm (a fused call honours
+ *   LTGNN_SPMM_GATHER).
+ * ltgnn_edge_norm_fwd: PyG gcn_norm(edge_index, w, add_self_loops=True) of Bw sets of edge weights w [Bw][E]
+ *   (w_stride 0 = one set read for every row of the output, or E): ent_edge [nnz] / t_ent_edge [nnz] give for every
+ *   entry of A_hat / A_hat^T the edge it comes from (an appended self loop: the position of the loop it replaces, or -1
+ *   for weight 1).  Writes dis [Bw][N] = deg^-1/2 (inf -> 0; deg summed in row order, self loop last), vals [Bw][nnz]
+ *   (A_hat order) and t_vals [Bw][nnz] (A_hat^T order), each (dis[src] * w) * dis[dst].
+ * ltgnn_edge_norm_bwd: dw [Bw][E] from dvals [Bw][nnz] (A_hat order) through the normalisation above; t_perm [nnz]:
+ *   A_hat position of each A_hat^T entry; ddeg: workspace of Bw * N floats.  Edges no entry comes from (a node's
+ *   earlier duplicate self loops) get 0.
+ * ltgnn_gcn_adj_grad: dA[b][k] (+)= sum_d Gg[b, row_k, d] XW[b, col_k, d] over A_hat's entries (A_hat order): the
+ *   gradient of Y = A_hat XW with respect to the entry values.  Gg = G gated as in ltgnn_spmm_fused (gate or live_in,
+ *   times gate_scale; both NULL: G itself).  accumulate = 1 adds to dA (several layers sharing one adjacency).
+ *   dA_sum (NULL or [nnz]): weights shared by every window -- dA is then scratch, written afresh, and dA_sum (+)= the
+ *   sum of its B rows (fixed two-stage order).
+ *   D % 4 == 0 and D <= 256.  All four: fixed summation order, no atomics, no allocation, no host synchronisation.
+ */
+int ltgnn_spmm_fused_vals(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float* X, float* Y,
+                          const float* vals, int64_t vals_stride, int algo, const float* bias, int relu, float drop_p,
+                          uint64_t drop_seed, const float* gate, float gate_scale, float* colsum, float* ws,
+                          uint32_t* live_out, const uint32_t* live_in, void* stream);
+int ltgnn_edge_norm_fwd(ltgnn_graph_t g, int64_t Bw, int32_t n_edges, const float* w, int64_t w_stride,
+                        const int32_t* ent_edge, const int32_t* t_ent_edge, float* dis, float* vals, float* t_vals,
+                        void* stream);
+int ltgnn_edge_norm_bwd(ltgnn_graph_t g, int64_t Bw, int32_t n_edges, const float* w, int64_t w_stride,
+                        const int32_t* ent_edge, const int32_t* t_ent_edge, const int32_t* t_perm, const float* dis,
+                        const float* dvals, float* ddeg, float* dw, void* stream);
+int ltgnn_gcn_adj_grad(ltgnn_graph_t g, int64_t B, int32_t D, const float* G, const float* gate, const uint32_t* live_in,
+                       float gate_scale, const float* XW, float* dA, int accumulate, float* dA_sum, void* stream);
+
 /* ---- dense row-wise layer on tensor cores --------------------------------------------------
  * Y[M,N] = gate( act( X[M,K] op(W) + bias[N] ) )
  *   op(W) = W^T with W [N,K] row-major (w_transposed = 0, torch.nn.Linear layout)

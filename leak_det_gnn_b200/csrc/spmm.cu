@@ -55,6 +55,9 @@ struct StagedParams {
     // 1-bit-per-element form of the gate: word (b, slice, node), bit 8 c + q <-> element (b, node, 32 slice + 4 q + c)
     uint32_t* live_out;       // written by the output epilogue (kEpi), or nullptr
     const uint32_t* live_in;  // read by the input gate (kGate) instead of `gate`, or nullptr
+    // per-call entry values (kVals): entry k of window b weighs vals[b * vals_stride + k] instead of the handle's value
+    const float* vals;
+    int64_t vals_stride;  // 0: one set shared by every window
 };
 
 __device__ __forceinline__ void fma2(float4& acc, float w, const float4& x) {
@@ -67,7 +70,7 @@ __device__ __forceinline__ void fma2(float4& acc, float w, const float4& x) {
 
 __device__ __forceinline__ void consumer_bar() { asm volatile("bar.sync 1, %0;" ::"n"(kConsumerWarps * 32) : "memory"); }
 
-template <bool kEpi, bool kGate>
+template <bool kEpi, bool kGate, bool kVals = false>
 __global__ void __launch_bounds__(kStagedThreads, 1)
 spmm_staged_kernel(const __grid_constant__ CUtensorMap tmap, const StagedParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -181,6 +184,9 @@ spmm_staged_kernel(const __grid_constant__ CUtensorMap tmap, const StagedParams 
         }
 
         float4* y = reinterpret_cast<float4*>(p.Y) + base4;
+        const float* vb = kVals ? p.vals + b * p.vals_stride : nullptr;
+        // an entry's weight: the handle's packed value, or the per-call one (same summation order either way)
+        auto wt = [&](const int2 c, int k) { return kVals ? __ldg(vb + k) : __int_as_float(c.y); };
         float4 bias4 = make_float4(0.f, 0.f, 0.f, 0.f);
         if (kEpi && p.bias) bias4 = __ldg(reinterpret_cast<const float4*>(p.bias) + sl * (kSliceFloats / 4) + q);
 
@@ -204,16 +210,16 @@ spmm_staged_kernel(const __grid_constant__ CUtensorMap tmap, const StagedParams 
                 const int2 c1 = s_colval[k1++];
                 const float4 x0 = xs[c0.x * 8];
                 const float4 x1 = xs[c1.x * 8];
-                fma2(a0, __int_as_float(c0.y), x0);
-                fma2(a1, __int_as_float(c1.y), x1);
+                fma2(a0, wt(c0, k0 - 1), x0);
+                fma2(a1, wt(c1, k1 - 1), x1);
             }
             for (; k0 < e0; ++k0) {
                 const int2 c0 = s_colval[k0];
-                fma2(a0, __int_as_float(c0.y), xs[c0.x * 8]);
+                fma2(a0, wt(c0, k0), xs[c0.x * 8]);
             }
             for (; k1 < e1; ++k1) {
                 const int2 c1 = s_colval[k1];
-                fma2(a1, __int_as_float(c1.y), xs[c1.x * 8]);
+                fma2(a1, wt(c1, k1), xs[c1.x * 8]);
             }
             if (kEpi) {
                 a0.x = __fadd_rn(a0.x, bias4.x); a0.y = __fadd_rn(a0.y, bias4.y);
@@ -291,13 +297,13 @@ __global__ void colsum_reduce_kernel(const float* __restrict__ ws, float* __rest
 // form live_in [B, D/32, N] (4 bytes per neighbour and 32-feature slice instead of a second 16-byte gather per float4).
 // live_out: the same record of y > 0, written by the q == 0 lane of every 8-lane slice group (word layout of new_live_mask:
 // bit 8 c + q <-> element 4 q + c of the slice).  Lanes of a warp stay together (the ballots need all 32).
-template <bool kEpi, bool kGate>
+template <bool kEpi, bool kGate, bool kVals = false>
 __global__ void __launch_bounds__(256)
 spmm_gather_kernel(const int32_t* __restrict__ rowptr, const int2* __restrict__ colval, const float4* __restrict__ X,
                    float4* __restrict__ Y, int32_t n, int32_t d4, int64_t total, const float4* __restrict__ bias, int relu,
                    uint32_t drop_thresh, float keep_scale, uint64_t drop_seed_arg, const uint64_t* seed_src,
                    const float4* __restrict__ gate, float gate_scale, uint32_t* __restrict__ live_out,
-                   const uint32_t* __restrict__ live_in) {
+                   const uint32_t* __restrict__ live_in, const float* __restrict__ vals, int64_t vals_stride) {
     const uint64_t drop_seed = launch_seed(drop_seed_arg, seed_src);
     const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
     const int lane = threadIdx.x & 31, n_slices = d4 >> 3;
@@ -312,6 +318,8 @@ spmm_gather_kernel(const int32_t* __restrict__ rowptr, const int2* __restrict__ 
         const float4* gb = (kGate && gate) ? gate + b * n * d4 + c4 : nullptr;
         const uint32_t* lb = (kGate && live_in) ? live_in + (b * n_slices + (c4 >> 3)) * n : nullptr;
         const int q = c4 & 7;
+        const float* vb = kVals ? vals + b * vals_stride : nullptr;
+        auto wt = [&](const int2 c, int kk) { return kVals ? __ldg(vb + kk) : __int_as_float(c.y); };
         auto fetch = [&](int col) {
             float4 x = __ldg(xb + static_cast<int64_t>(col) * d4);
             if (kGate) {
@@ -336,12 +344,12 @@ spmm_gather_kernel(const int32_t* __restrict__ rowptr, const int2* __restrict__ 
                 const int2 c1 = __ldg(colval + k + 1);
                 const float4 x0 = fetch(c0.x);
                 const float4 x1 = fetch(c1.x);
-                fma2(acc, __int_as_float(c0.y), x0);
-                fma2(acc, __int_as_float(c1.y), x1);
+                fma2(acc, wt(c0, k), x0);
+                fma2(acc, wt(c1, k + 1), x1);
             }
             if (k < end) {
                 const int2 c0 = __ldg(colval + k);
-                fma2(acc, __int_as_float(c0.y), fetch(c0.x));
+                fma2(acc, wt(c0, k), fetch(c0.x));
             }
             if (kEpi) {
                 if (bias) {
@@ -448,6 +456,8 @@ struct FusedArgs {
     float* ws = nullptr;
     uint32_t* live_out = nullptr;
     const uint32_t* live_in = nullptr;
+    const float* vals = nullptr;  // per-call entry values [1 or B][nnz], in the order of the chosen orientation
+    int64_t vals_stride = 0;
 };
 
 int spmm_impl(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float* X, float* Y, int algo,
@@ -475,7 +485,7 @@ int spmm_impl(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float*
 
     const StagedPlan pl = plan_staged(g, D);
     const bool fused = epi || gated;
-    const bool want_staged = (algo == LTGNN_SPMM_STAGED) || (fused && pl.ok) ||
+    const bool want_staged = (algo == LTGNN_SPMM_STAGED) || (fused && pl.ok && algo != LTGNN_SPMM_GATHER) ||
                              (algo == LTGNN_SPMM_AUTO && pl.ok && pl.n_stages >= 2);
     if (algo == LTGNN_SPMM_STAGED)
         LTGNN_REQUIRE(pl.ok, LTGNN_E_SHAPE, "%s: the STAGED kernel needs D %% 32 == 0 and a 32-feature slice of the "
@@ -526,6 +536,8 @@ int spmm_impl(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float*
         p.colsum_ws = f.colsum ? f.ws : nullptr;
         p.live_out = f.live_out;
         p.live_in = f.live_in;
+        p.vals = f.vals;
+        p.vals_stride = f.vals_stride;
         LTGNN_REQUIRE(!f.live_in || g->n <= kMaxGateRows * kConsumerWarps * 4, LTGNN_E_SHAPE,
                       "%s: the 1-bit gate supports graphs up to %d nodes", who, kMaxGateRows * kConsumerWarps * 4);
         // a CTA must keep one feature slice for its whole life when it accumulates column sums
@@ -541,7 +553,10 @@ int spmm_impl(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float*
             return LTGNN_OK;
         };
         int rc;
-        if (gated) rc = epi ? launch(spmm_staged_kernel<true, true>) : launch(spmm_staged_kernel<false, true>);
+        if (f.vals) {
+            if (gated) rc = epi ? launch(spmm_staged_kernel<true, true, true>) : launch(spmm_staged_kernel<false, true, true>);
+            else rc = epi ? launch(spmm_staged_kernel<true, false, true>) : launch(spmm_staged_kernel<false, false, true>);
+        } else if (gated) rc = epi ? launch(spmm_staged_kernel<true, true>) : launch(spmm_staged_kernel<false, true>);
         else rc = epi ? launch(spmm_staged_kernel<true, false>) : launch(spmm_staged_kernel<false, false>);
         if (rc) return rc;
         if (f.colsum) {
@@ -561,12 +576,15 @@ int spmm_impl(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float*
         kern<<<static_cast<int>(blocks), 256, 0, stream>>>(
             g->rowptr[transpose], g->colval[transpose], reinterpret_cast<const float4*>(X), reinterpret_cast<float4*>(Y),
             g->n, D / 4, total, reinterpret_cast<const float4*>(f.bias), f.relu, thresh, keep, f.drop_seed, seed_source(),
-            reinterpret_cast<const float4*>(f.gate), f.gate_scale, f.live_out, f.live_in);
+            reinterpret_cast<const float4*>(f.gate), f.gate_scale, f.live_out, f.live_in, f.vals, f.vals_stride);
         LTGNN_CUDA_TRY(cudaGetLastError());
         return LTGNN_OK;
     };
     int rc;
-    if (gated) rc = epi ? launch_g(spmm_gather_kernel<true, true>) : launch_g(spmm_gather_kernel<false, true>);
+    if (f.vals) {
+        if (gated) rc = epi ? launch_g(spmm_gather_kernel<true, true, true>) : launch_g(spmm_gather_kernel<false, true, true>);
+        else rc = epi ? launch_g(spmm_gather_kernel<true, false, true>) : launch_g(spmm_gather_kernel<false, false, true>);
+    } else if (gated) rc = epi ? launch_g(spmm_gather_kernel<true, true>) : launch_g(spmm_gather_kernel<false, true>);
     else rc = epi ? launch_g(spmm_gather_kernel<true, false>) : launch_g(spmm_gather_kernel<false, false>);
     if (rc) return rc;
     if (f.colsum) {
@@ -610,4 +628,29 @@ extern "C" int ltgnn_spmm_fused(ltgnn_graph_t g, int transpose, int64_t B, int32
     f.colsum = colsum;
     f.ws = ws;
     return spmm_impl(g, transpose, B, D, X, Y, LTGNN_SPMM_AUTO, f, static_cast<cudaStream_t>(stream_), "spmm_fused");
+}
+
+extern "C" int ltgnn_spmm_fused_vals(ltgnn_graph_t g, int transpose, int64_t B, int32_t D, const float* X, float* Y,
+                                     const float* vals, int64_t vals_stride, int algo, const float* bias, int relu,
+                                     float drop_p, uint64_t drop_seed, const float* gate, float gate_scale, float* colsum,
+                                     float* ws, uint32_t* live_out, const uint32_t* live_in, void* stream_) {
+    LTGNN_REQUIRE(vals != nullptr, LTGNN_E_ARG, "spmm_fused_vals: null vals");
+    LTGNN_REQUIRE(g == nullptr || vals_stride == 0 || vals_stride == g->nnz, LTGNN_E_ARG,
+                  "spmm_fused_vals: vals_stride %lld must be 0 (shared) or nnz", static_cast<long long>(vals_stride));
+    LTGNN_REQUIRE(algo == LTGNN_SPMM_AUTO || algo == LTGNN_SPMM_STAGED || algo == LTGNN_SPMM_GATHER, LTGNN_E_ARG,
+                  "spmm_fused_vals: unknown algo %d", algo);
+    FusedArgs f;
+    f.live_out = live_out;
+    f.live_in = live_in;
+    f.bias = bias;
+    f.relu = relu;
+    f.drop_p = drop_p;
+    f.drop_seed = drop_seed;
+    f.gate = gate;
+    f.gate_scale = gate_scale;
+    f.colsum = colsum;
+    f.ws = ws;
+    f.vals = vals;
+    f.vals_stride = vals_stride;
+    return spmm_impl(g, transpose, B, D, X, Y, algo, f, static_cast<cudaStream_t>(stream_), "spmm_fused_vals");
 }

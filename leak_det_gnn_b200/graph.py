@@ -183,6 +183,10 @@ class GCNCsr:
     ``t_rowptr/t_col/t_val`` : CSR of A_hat^T (the "CSC transpose"): row = source,
                           entries ordered by edge position, used by every backward.
     ``t_perm``          : position in the forward arrays of each transposed entry.
+    ``edge/t_edge``     : for every entry of the two orders, the position in the input ``edge_index`` of the edge it
+                          comes from; an appended self loop holds the position of the self loop it replaces (the
+                          last one, if a node had several), or -1 where the node had none (weight 1).  This is what
+                          maps per-call ``edge_weight`` values (``num_edges`` of them) onto the entries.
     """
 
     num_nodes: int
@@ -193,6 +197,9 @@ class GCNCsr:
     t_col: np.ndarray
     t_val: np.ndarray
     t_perm: np.ndarray  # int32 [nnz]
+    edge: np.ndarray  # int32 [nnz]
+    t_edge: np.ndarray  # int32 [nnz]
+    num_edges: int
 
     @property
     def nnz(self) -> int:
@@ -231,6 +238,13 @@ def build_gcn_csr(edge_index: torch.Tensor, num_nodes: int) -> GCNCsr:
     if edge_index.numel() and (int(edge_index.min()) < 0 or int(edge_index.max()) >= num_nodes):
         raise ValueError("edge_index entries out of range for num_nodes")
     ei, norm = gcn_norm_edges(edge_index, num_nodes)
+    # source edge of each normalised edge: kept non-loop edges in order, then per node its last removed loop or -1
+    e_in = edge_index.detach().to("cpu", torch.long)
+    pos = torch.arange(e_in.size(1), dtype=torch.long)
+    is_loop = e_in[0] == e_in[1]
+    loop_src = torch.full((num_nodes,), -1, dtype=torch.long)
+    loop_src[e_in[0, is_loop]] = pos[is_loop]  # CPU index_put: the last duplicate wins, as PyG's loop_attr assignment
+    ent_src_edge = torch.cat([pos[~is_loop], loop_src]).numpy()
     src = ei[0].numpy()
     dst = ei[1].numpy()
     w = norm.numpy()
@@ -249,4 +263,5 @@ def build_gcn_csr(edge_index: torch.Tensor, num_nodes: int) -> GCNCsr:
     pos_in_fwd = np.empty(nnz, dtype=np.int64)
     pos_in_fwd[order_f] = np.arange(nnz)
     t_perm = pos_in_fwd[order_t].astype(np.int32)
-    return GCNCsr(int(num_nodes), rowptr, col, val, t_rowptr, t_col, t_val, t_perm)
+    return GCNCsr(int(num_nodes), rowptr, col, val, t_rowptr, t_col, t_val, t_perm, ent_src_edge[order_f].astype(np.int32),
+                  ent_src_edge[order_t].astype(np.int32), int(edge_index.size(1)))

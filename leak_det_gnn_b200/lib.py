@@ -31,6 +31,15 @@ SIGNATURES = {
     "ltgnn_spmm_ws_floats": (c_int64, [c_void_p]),
     "ltgnn_spmm_fused": (c_int, [c_void_p, c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int, c_float,
                                  c_uint64, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_spmm_fused_vals": (c_int, [c_void_p, c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_int,
+                                      c_void_p, c_int, c_float, c_uint64, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p]),
+    "ltgnn_edge_norm_fwd": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p]),
+    "ltgnn_edge_norm_bwd": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_gcn_adj_grad": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                                   c_int, c_void_p, c_void_p]),
     "ltgnn_linear": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
                              c_float, c_void_p, c_void_p]),
     "ltgnn_wgrad_ws_floats": (c_int64, [c_int, c_int32, c_int32]),

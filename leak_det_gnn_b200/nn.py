@@ -10,6 +10,11 @@ zero).  ``forward`` accepts
 * ``conv(x, edge_index)`` with a ``(2, E)`` int64 tensor, PyG's own signature: the graph over
   ``x.size(0)`` nodes is normalised on the host once per distinct ``edge_index`` content
   (the cache keeps its own copy and compares contents) and then runs the same kernels as one big window.
+
+Both take PyG's third argument ``edge_weight``: one weight per edge of ``edge_index`` (the graph's, or the replicated
+one's), or with a ``PipeGraph`` also (B, E), one row per window.  The weights are normalised on the device on every call
+(``gcn_norm`` with self loops; a node's existing self loop keeps its weight, an added one weighs 1) and are
+differentiable.
 """
 from __future__ import annotations
 
@@ -78,10 +83,11 @@ class GCNConv(nn.Module):
         if self.bias is not None:
             nn.init.zeros_(self.bias)
 
-    def forward(self, x: torch.Tensor, graph: Union[PipeGraph, torch.Tensor]) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, graph: Union[PipeGraph, torch.Tensor],
+                edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
         if isinstance(graph, torch.Tensor):
             graph = _graph_from_edge_index(graph, x.shape[0] if x.dim() == 2 else x.shape[-2])
-        return ops.gcn_conv(x, graph, self.lin.weight, self.bias)
+        return ops.gcn_conv(x, graph, self.lin.weight, self.bias, edge_weight)
 
     def extra_repr(self) -> str:
         return f"{self.in_channels}, {self.out_channels}"

@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -42,6 +42,7 @@ class PipeGraph:
         self.num_nodes = int(num_nodes)
         self.csr: GCNCsr = build_gcn_csr(edge_index, self.num_nodes)
         self._handles: Dict[int, ctypes.c_void_p] = {}
+        self._edge_maps: Dict[int, tuple] = {}
         self._lock = threading.Lock()
 
     @property
@@ -64,6 +65,24 @@ class PipeGraph:
                                                     _ptr(c.t_rowptr), _ptr(c.t_col), _ptr(c.t_val), ctypes.byref(out)))
                     self._handles[idx] = h = out
         return h
+
+    @property
+    def num_edges(self) -> int:
+        """Edges of the ``edge_index`` the graph was built from: the length of an ``edge_weight`` row."""
+        return self.csr.num_edges
+
+    def edge_maps(self, device: torch.device):
+        """(edge, t_edge, t_perm) of :class:`~leak_det_gnn_b200.graph.GCNCsr` as int32 tensors on ``device``, uploaded
+        once: what the device normalisation of per-call edge weights reads."""
+        self.handle(device)
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        hit = self._edge_maps.get(idx)
+        if hit is None:
+            c = self.csr
+            hit = tuple(torch.from_numpy(np.ascontiguousarray(a)).to(torch.device("cuda", idx))
+                        for a in (c.edge, c.t_edge, c.t_perm))
+            self._edge_maps[idx] = hit
+        return hit
 
     def __del__(self) -> None:  # best effort; the handle only owns ~40 KB of device memory
         try:
@@ -202,11 +221,12 @@ def unpack_live_mask(live: torch.Tensor) -> torch.Tensor:
 def spmm_fused(graph: PipeGraph, x: torch.Tensor, transpose: bool = False, bias: Optional[torch.Tensor] = None,
                relu: bool = False, drop_p: float = 0.0, drop_seed: int = 0, gate: Optional[torch.Tensor] = None,
                gate_scale: float = 1.0, want_colsum: bool = False, live_out: Optional[torch.Tensor] = None,
-               live_in: Optional[torch.Tensor] = None):
+               live_in: Optional[torch.Tensor] = None, vals: Optional[torch.Tensor] = None, algo: int = _lib.SPMM_AUTO):
     """Raw fused aggregation (see ltgnn_spmm_fused): ``dropout(relu(A (x * gatemask) + bias))``.
     Returns ``y`` or ``(y, colsum)`` when ``want_colsum`` (column sums of the gated input).
     ``live_out`` / ``live_in``: int32 (B, D/32, N) tensors holding ``y > 0`` / the gate as one bit per element
-    (see :func:`new_live_mask`)."""
+    (see :func:`new_live_mask`).  ``vals``: per-call entry values (1 or B, nnz) in the order of the chosen orientation
+    (:func:`edge_norm`) instead of the graph's own (ltgnn_spmm_fused_vals; ``algo`` forces a kernel there)."""
     _check_act(x, "x")
     n, d = graph.num_nodes, x.shape[-1]
     if x.numel() % (n * d) != 0:
@@ -222,6 +242,12 @@ def spmm_fused(graph: PipeGraph, x: torch.Tensor, transpose: bool = False, bias:
         if lv is not None and (lv.dtype != torch.int32 or not lv.is_cuda or not lv.is_contiguous()
                                or tuple(lv.shape) != (b, d // 32, n)):
             raise ValueError(f"{nm} must be a contiguous int32 CUDA tensor of shape {(b, d // 32, n)}")
+    if vals is not None:
+        _check_act(vals, "vals")
+        if vals.dim() != 2 or vals.shape[1] != graph.nnz or vals.shape[0] not in (1, b):
+            raise ValueError(f"vals must be (1, {graph.nnz}) or ({b}, {graph.nnz}), got {tuple(vals.shape)}")
+        if vals.device != x.device:
+            raise ValueError("vals must be on the device of x")
     y = torch.empty_like(x)
     L = _lib.load()
     h = graph.handle(x.device)
@@ -231,6 +257,18 @@ def spmm_fused(graph: PipeGraph, x: torch.Tensor, transpose: bool = False, bias:
             raise ValueError("want_colsum needs a gate")
         colsum = torch.empty(d, device=x.device, dtype=torch.float32)
         ws = torch.empty(int(L.ltgnn_spmm_ws_floats(h)), device=x.device, dtype=torch.float32)
+    if vals is not None:
+        tok = _inst.begin("spmm_vals_bwd" if transpose else "spmm_vals_fwd")
+        _lib.check(L.ltgnn_spmm_fused_vals(h, int(bool(transpose)), b, d, x.data_ptr(), y.data_ptr(), vals.data_ptr(),
+                                           0 if vals.shape[0] == 1 else graph.nnz, int(algo),
+                                           None if bias is None else bias.data_ptr(), int(relu), float(drop_p),
+                                           int(drop_seed) & (2**64 - 1), None if gate is None else gate.data_ptr(),
+                                           float(gate_scale), None if colsum is None else colsum.data_ptr(),
+                                           None if ws is None else ws.data_ptr(),
+                                           None if live_out is None else live_out.data_ptr(),
+                                           None if live_in is None else live_in.data_ptr(), _stream(x)))
+        _inst.end(tok)
+        return (y, colsum) if want_colsum else y
     tok = _inst.begin("spmm_fused_bwd" if transpose else "spmm_fused_fwd")
     _lib.check(L.ltgnn_spmm_fused(h, int(bool(transpose)), b, d, x.data_ptr(), y.data_ptr(),
                                   None if bias is None else bias.data_ptr(), int(relu), float(drop_p),
@@ -416,6 +454,115 @@ def node_init_bwd(h_s, slot, weight, dx0, x0, gate_scale, live=None):
 
 
 # ----------------------------------------------------------------------------------------------
+# per-call edge weights: PyG's gcn_norm on the device and the gradient with respect to the adjacency values
+# ----------------------------------------------------------------------------------------------
+def _check_edge_weight(graph: PipeGraph, w: torch.Tensor, b: int) -> None:
+    if not isinstance(w, torch.Tensor):
+        raise ValueError("edge_weight must be a tensor")
+    e = graph.num_edges
+    if not (tuple(w.shape) == (e,) or (w.dim() == 2 and tuple(w.shape) == (b, e))):
+        raise ValueError(f"edge_weight must be ({e},) (shared by every window) or ({b}, {e}) (one row per window), "
+                         f"got {tuple(w.shape)}")
+    if not w.is_cuda:
+        raise ValueError("edge_weight must be a CUDA tensor (libltgnn has no CPU path)")
+    if w.dtype != torch.float32:
+        raise ValueError(f"edge_weight must be float32, got {w.dtype}")
+
+
+def edge_norm(graph: PipeGraph, w: torch.Tensor):
+    """Raw device normalisation (see ltgnn_edge_norm_fwd): edge weights (E,) or (Bw, E) in ``edge_index`` order ->
+    ``(vals, t_vals, dis)``: the entry values of A_hat and of A_hat^T, (1 or Bw, nnz) each, and deg^-1/2 (1 or Bw, N)."""
+    _check_act(w, "edge_weight")
+    w2 = w.view(1, -1) if w.dim() == 1 else w
+    if w2.dim() != 2 or w2.shape[1] != graph.num_edges:
+        raise ValueError(f"edge_weight rows must hold {graph.num_edges} values, got {tuple(w.shape)}")
+    bw = w2.shape[0]
+    ent, t_ent, _ = graph.edge_maps(w.device)
+    vals = torch.empty(bw, graph.nnz, device=w.device, dtype=torch.float32)
+    t_vals = torch.empty_like(vals)
+    dis = torch.empty(bw, graph.num_nodes, device=w.device, dtype=torch.float32)
+    tok = _inst.begin("edge_norm_fwd")
+    _lib.check(_lib.load().ltgnn_edge_norm_fwd(graph.handle(w.device), bw, graph.num_edges, w2.data_ptr(), graph.num_edges,
+                                               ent.data_ptr(), t_ent.data_ptr(), dis.data_ptr(), vals.data_ptr(),
+                                               t_vals.data_ptr(), _stream(w)))
+    _inst.end(tok)
+    return vals, t_vals, dis
+
+
+def edge_norm_bwd(graph: PipeGraph, w: torch.Tensor, dis: torch.Tensor, dvals: torch.Tensor) -> torch.Tensor:
+    """Raw backward of :func:`edge_norm`: d vals (Bw, nnz) in A_hat order -> d edge_weight of ``w``'s shape."""
+    w2 = w.view(1, -1) if w.dim() == 1 else w
+    dvals = dvals.contiguous()
+    ent, t_ent, t_perm = graph.edge_maps(w.device)
+    bw = w2.shape[0]
+    ddeg = torch.empty(bw, graph.num_nodes, device=w.device, dtype=torch.float32)
+    dw = torch.empty(bw, graph.num_edges, device=w.device, dtype=torch.float32)
+    tok = _inst.begin("edge_norm_bwd")
+    _lib.check(_lib.load().ltgnn_edge_norm_bwd(graph.handle(w.device), bw, graph.num_edges, w2.data_ptr(), graph.num_edges,
+                                               ent.data_ptr(), t_ent.data_ptr(), t_perm.data_ptr(), dis.data_ptr(),
+                                               dvals.data_ptr(), ddeg.data_ptr(), dw.data_ptr(), _stream(w)))
+    _inst.end(tok)
+    return dw.view(w.shape)
+
+
+def gcn_adj_grad(graph: PipeGraph, g: torch.Tensor, xw: torch.Tensor, gate: Optional[torch.Tensor] = None,
+                 live_in: Optional[torch.Tensor] = None, gate_scale: float = 1.0, out: Optional[torch.Tensor] = None,
+                 shared: bool = False, accumulate: bool = False) -> torch.Tensor:
+    """Raw adjacency-value gradient (see ltgnn_gcn_adj_grad): ``dA[b, k] = <Gg[b, row_k], xw[b, col_k]>`` over A_hat's
+    entries, Gg = g gated by ``gate`` / ``live_in`` times ``gate_scale``.  Returns (B, nnz), or with ``shared`` the sum
+    over windows (1, nnz); ``accumulate`` adds into ``out``."""
+    _check_act(g, "g")
+    _check_act(xw, "xw")
+    n, d = graph.num_nodes, g.shape[-1]
+    if xw.shape != g.shape or g.numel() % (n * d) != 0:
+        raise ValueError(f"g {tuple(g.shape)} and xw {tuple(xw.shape)} must be the same whole number of {n}-node graphs")
+    b = g.numel() // (n * d)
+    if gate is not None:
+        _check_act(gate, "gate")
+    rows = 1 if shared else b
+    if out is None:
+        out = torch.empty(rows, graph.nnz, device=g.device, dtype=torch.float32)
+    elif tuple(out.shape) != (rows, graph.nnz):
+        raise ValueError(f"out must be {(rows, graph.nnz)}")
+    scratch = torch.empty(b, graph.nnz, device=g.device, dtype=torch.float32) if shared else out
+    tok = _inst.begin("gcn_adj_grad")
+    _lib.check(_lib.load().ltgnn_gcn_adj_grad(graph.handle(g.device), b, d, g.data_ptr(),
+                                              None if gate is None else gate.data_ptr(),
+                                              None if live_in is None else live_in.data_ptr(), float(gate_scale),
+                                              xw.data_ptr(), scratch.data_ptr(), int(bool(accumulate)),
+                                              out.data_ptr() if shared else None, _stream(g)))
+    _inst.end(tok)
+    return out
+
+
+class _EdgeNorm(torch.autograd.Function):
+    """edge_weight -> (vals, t_vals): the normalised entry values in both orders.  The layers report the gradient of
+    the adjacency through ``vals`` (A_hat order); ``t_vals`` is the same matrix transposed, for their backward."""
+
+    @staticmethod
+    def forward(ctx, w, graph):
+        w = w.contiguous()
+        vals, t_vals, dis = edge_norm(graph, w)
+        ctx.mark_non_differentiable(t_vals)
+        ctx.save_for_backward(w, dis)
+        ctx.graph = graph
+        return vals, t_vals
+
+    @staticmethod
+    def backward(ctx, dvals, _dt_vals):
+        w, dis = ctx.saved_tensors
+        if dvals is None:
+            return None, None
+        return edge_norm_bwd(ctx.graph, w, dis, dvals), None
+
+
+def normalized_edge_values(graph: PipeGraph, edge_weight: torch.Tensor, b: int):
+    """Differentiable ``(vals, t_vals)`` of ``edge_weight`` ((E,) or (b, E)) for the weighted layers."""
+    _check_edge_weight(graph, edge_weight, b)
+    return _EdgeNorm.apply(edge_weight, graph)
+
+
+# ----------------------------------------------------------------------------------------------
 # operator-level autograd: GCNConv  (reference call site models/detector.py:199)
 # ----------------------------------------------------------------------------------------------
 class _GcnConv(torch.autograd.Function):
@@ -423,37 +570,55 @@ class _GcnConv(torch.autograd.Function):
     dW = G^T x, dx = G W, db = column sums of dout."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, graph):
+    def forward(ctx, x, weight, bias, graph, vals=None, t_vals=None):
         x = x.contiguous()
         n = graph.num_nodes
         xw = _linear_any(x, weight)
         xw3 = xw.view(-1, n, xw.shape[-1])
-        if bias is not None and _staged_ok(graph, xw.shape[-1]):
+        if vals is not None:  # weighted adjacency: the per-call values (bias fused where the STAGED kernel takes it)
+            fuse = bias is not None and _staged_ok(graph, xw.shape[-1])
+            y = spmm_fused(graph, xw3, bias=bias if fuse else None, vals=vals)
+            if bias is not None and not fuse:
+                y += bias
+        elif bias is not None and _staged_ok(graph, xw.shape[-1]):
             y = spmm_fused(graph, xw3, bias=bias)
         else:
             y = spmm(graph, xw3)
             if bias is not None:
                 y += bias
-        ctx.save_for_backward(x, weight)
-        ctx.graph, ctx.has_bias = graph, bias is not None
+        keep_xw = vals is not None and ctx.needs_input_grad[4]
+        ctx.save_for_backward(x, weight, t_vals, xw3 if keep_xw else None)
+        ctx.graph, ctx.has_bias, ctx.shared = graph, bias is not None, vals is not None and vals.shape[0] == 1
         return y.view(*x.shape[:-1], xw.shape[-1])
 
     @staticmethod
     def backward(ctx, dy):
-        x, weight = ctx.saved_tensors
+        x, weight, t_vals, xw3 = ctx.saved_tensors
         dy = dy.contiguous()
-        g = spmm(ctx.graph, dy.view(-1, ctx.graph.num_nodes, dy.shape[-1]), transpose=True).view(dy.shape)
+        dy3 = dy.view(-1, ctx.graph.num_nodes, dy.shape[-1])
+        if t_vals is None:
+            g = spmm(ctx.graph, dy3, transpose=True).view(dy.shape)
+        else:
+            g = spmm_fused(ctx.graph, dy3, transpose=True, vals=t_vals).view(dy.shape)
         dw = wgrad(g, x) if ctx.needs_input_grad[1] else None
         dx = _linear_any(g, weight, transposed=True) if ctx.needs_input_grad[0] else None
         db = dy.reshape(-1, dy.shape[-1]).sum(0) if ctx.has_bias and ctx.needs_input_grad[2] else None
-        return dx, dw, db, None
+        dvals = gcn_adj_grad(ctx.graph, dy3, xw3, shared=ctx.shared) if xw3 is not None else None
+        return dx, dw, db, None, dvals, None
 
 
-def gcn_conv(x: torch.Tensor, graph: PipeGraph, weight: torch.Tensor, bias: Optional[torch.Tensor]) -> torch.Tensor:
+def gcn_conv(x: torch.Tensor, graph: PipeGraph, weight: torch.Tensor, bias: Optional[torch.Tensor],
+             edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
     """``A_hat (x W^T) + b`` -- the operator ``torch_geometric.nn.GCNConv.forward`` computes
-    (reference call site models/detector.py:199).  x: (B, N, Din) or (B*N, Din), fp32 CUDA."""
+    (reference call site models/detector.py:199).  x: (B, N, Din) or (B*N, Din), fp32 CUDA.  ``edge_weight``: PyG's
+    per-edge weights in ``edge_index`` order, (E,) shared by every window or (B, E), normalised on the device
+    (gcn_norm with self loops) on each call and differentiable; ``None`` runs the graph's own normalised adjacency."""
     _check_act(x.contiguous(), "x")
-    return _GcnConv.apply(x, weight, bias, graph)
+    if edge_weight is None:
+        return _GcnConv.apply(x, weight, bias, graph)
+    b = x.numel() // (graph.num_nodes * x.shape[-1])
+    vals, t_vals = normalized_edge_values(graph, edge_weight, b)
+    return _GcnConv.apply(x, weight, bias, graph, vals, t_vals)
 
 
 class _MeanPool(torch.autograd.Function):
@@ -712,7 +877,7 @@ class _GnnBody(torch.autograd.Function):
     bias gradient in one staged kernel, weight gradient, input gradient on tensor cores."""
 
     @staticmethod
-    def forward(ctx, h_s, slot, graph, drop_p, training, w0, b0, *conv_params):
+    def forward(ctx, h_s, slot, graph, drop_p, training, vals, t_vals, w0, b0, *conv_params):
         h_s = h_s.contiguous()
         n = graph.num_nodes
         p = float(drop_p) if training else 0.0
@@ -726,9 +891,13 @@ class _GnnBody(torch.autograd.Function):
         lives = [live_for(w0.shape[0])]
         x = node_init_fwd(h_s, slot, n, w0, b0, p, new_dropout_seed() if p > 0 else 0, live_out=lives[0])
         xs = [x]
+        # weighted adjacency: every layer runs ltgnn_linear + the weighted aggregation; XW of each layer is kept for the
+        # adjacency-value gradient when one is asked for
+        keep_xw = vals is not None and ctx.needs_input_grad[5]
+        xws = []
         for l in range(n_layers):
             w, b = conv_params[2 * l], conv_params[2 * l + 1]
-            if FUSED_LAYER and w.is_contiguous() and gcn_layer_supported(graph, x, w):
+            if vals is None and FUSED_LAYER and w.is_contiguous() and gcn_layer_supported(graph, x, w):
                 lives.append(live_for(w.shape[0]))
                 x = gcn_layer_fwd(graph, x, w, bias=b, relu=True, drop_p=p, drop_seed=new_dropout_seed() if p > 0 else 0,
                                   live_out=lives[-1])
@@ -741,14 +910,17 @@ class _GnnBody(torch.autograd.Function):
             lives.append(live_for(d_out) if _staged_ok(graph, d_out)
                          else (new_live_mask(bsz, n, d_out, h_s.device) if need_grad and d_out % 32 == 0 else None))
             x = spmm_fused(graph, xw.view(bsz, n, -1), bias=b, relu=True, drop_p=p,
-                           drop_seed=new_dropout_seed() if p > 0 else 0, live_out=lives[-1])
+                           drop_seed=new_dropout_seed() if p > 0 else 0, live_out=lives[-1], vals=vals)
+            if keep_xw:
+                xws.append(xw.view(bsz, n, -1))
             del xw
             xs.append(x)
         ctx.lives = lives
         if DEBUG_CAPTURE is not None:
             DEBUG_CAPTURE["lives"] = lives
             DEBUG_CAPTURE["xs"] = xs   # the gates of the layers without a live mask (None in `lives`)
-        ctx.save_for_backward(h_s, slot, w0, *conv_params[0::2], *xs)
+        ctx.save_for_backward(h_s, slot, w0, *conv_params[0::2], *xs, t_vals, *xws)
+        ctx.shared = vals is not None and vals.shape[0] == 1
         # the kernels draw 16 random bits per element: keep probability 1 - round(p * 2^16) / 2^16
         ctx.graph, ctx.n_layers, ctx.scale = graph, n_layers, 1.0 / (1.0 - int(p * 65536.0 + 0.5) / 65536.0)
         return xs[-1]
@@ -759,28 +931,38 @@ class _GnnBody(torch.autograd.Function):
         L_ = ctx.n_layers
         h_s, slot, w0 = saved[0], saved[1], saved[2]
         ws_ = saved[3:3 + L_]
-        xs = saved[3 + L_:]
+        xs = saved[3 + L_:3 + 2 * L_ + 1]
+        t_vals, xws = saved[3 + 2 * L_ + 1], saved[3 + 2 * L_ + 2:]
         graph, scale = ctx.graph, ctx.scale
         g = dx.contiguous()
         grads = [None] * (2 * L_)
+        dvals = None
         for l in range(L_ - 1, -1, -1):
             x_out, x_in, w = xs[l + 1], xs[l], ws_[l]
             live = ctx.lives[l + 1]
+            if xws:  # d A_hat of this layer, gated exactly as the aggregation below gates g; layers add up
+                dvals = gcn_adj_grad(graph, g, xws[l], gate=x_out if live is None else None, live_in=live,
+                                     gate_scale=scale, out=dvals, shared=ctx.shared, accumulate=dvals is not None)
             gz, db = spmm_fused(graph, g, transpose=True, gate=x_out if live is None else None, live_in=live,
-                                gate_scale=scale, want_colsum=True)
+                                gate_scale=scale, want_colsum=True, vals=t_vals)
             grads[2 * l] = wgrad(gz, x_in)
             grads[2 * l + 1] = db
             g = _linear_any(gz, w, transposed=True)
             del gz
         dhs, dw0, db0 = node_init_bwd(h_s, slot, w0, g, xs[0], scale, live=ctx.lives[0])
-        return (dhs, None, None, None, None, dw0, db0, *grads)
+        return (dhs, None, None, None, None, dvals, None, dw0, db0, *grads)
 
 
 def gnn_body(h_s: torch.Tensor, slot: torch.Tensor, graph: PipeGraph, drop_p: float, training: bool,
-             w0: torch.Tensor, b0: torch.Tensor, conv_params) -> torch.Tensor:
-    """Sensor embeddings (B,S,ds) -> node states after the last GCN layer (B,N,D)."""
+             w0: torch.Tensor, b0: torch.Tensor, conv_params, edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Sensor embeddings (B,S,ds) -> node states after the last GCN layer (B,N,D).  ``edge_weight``: (E,) or (B, E)
+    weights of the graph's edges, normalised once on the device and used by every layer (as PyG passes one
+    ``edge_weight`` to every conv); differentiable.  ``None``: the graph's own adjacency, on the one-kernel layers."""
     _check_act(h_s.contiguous(), "h_s")
-    return _GnnBody.apply(h_s, slot, graph, drop_p, training, w0, b0, *conv_params)
+    vals = t_vals = None
+    if edge_weight is not None:
+        vals, t_vals = normalized_edge_values(graph, edge_weight, h_s.shape[0])
+    return _GnnBody.apply(h_s, slot, graph, drop_p, training, vals, t_vals, w0, b0, *conv_params)
 
 
 # ----------------------------------------------------------------------------------------------
