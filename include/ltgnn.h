@@ -146,6 +146,35 @@ int ltgnn_edge_norm_bwd(ltgnn_graph_t g, int64_t Bw, int32_t n_edges, const floa
 int ltgnn_gcn_adj_grad(ltgnn_graph_t g, int64_t B, int32_t D, const float* G, const float* gate, const uint32_t* live_in,
                        float gate_scale, const float* XW, float* dA, int accumulate, float* dA_sum, void* stream);
 
+/* ---- explainer edge masks (PyG's MessagePassing.explain_message, GNNExplainer) --------------------------------------
+ * ltgnn_edge_mask_fwd: vals [B][nnz] (A_hat order) and t_vals [B][nnz] (A_hat^T order) = base * f, f = mask[b][edge(k)]
+ *   for an off-diagonal entry k and 1 for gcn_norm's self loops: the mask scales the message after the normalisation.
+ *   mask [1 or B][E] (mask_stride 0 or E); base / t_base [1 or B][nnz] in the two orders (base_stride 0 or nnz), e.g.
+ *   ltgnn_edge_norm_fwd's vals / t_vals, or both NULL for the handle's own values.  ent_edge / t_ent_edge as in
+ *   ltgnn_edge_norm_fwd.
+ * ltgnn_edge_mask_bwd: from dvals [B][nnz] (A_hat order): dmask [B][E] = dvals[k] * base[k] at edge(k) (0 for edges no
+ *   entry comes from: input self loops); dbase (NULL, or [B][nnz] with per-call base) = dvals * f.  dmask_sum /
+ *   dbase_sum (NULL or [E] / [nnz]): a mask / base shared by every window -- the row results are then scratch and the
+ *   sums of their B rows (fixed two-stage order) are written there.
+ * ltgnn_explain_step: one GNNExplainer epoch (PyG 2.x, edge_mask_type='object', edge_reduction='sum') on the mask
+ *   logits m [B][E] of s = sigmoid(m) [B][E], from g = d loss / d s [B][E]:
+ *     dm = g s(1-s) + hard [edge_size + edge_ent / n_hard[b] * dH/ds] s(1-s),
+ *     H(s) = -s log(s + 1e-15) - (1-s) log(1-s + 1e-15), the entropy term 0 for a window without hard entries;
+ *   then torch.optim.Adam (lr, beta1, beta2, eps; state exp_avg / exp_avg_sq [B][E]; *step = steps taken, read and then
+ *   incremented on the device, so a captured epoch replays with the right bias corrections) and the new m and s.
+ *   record = 1 (epoch 0): no regulariser; writes hard [B][E] (bytes, dm != 0) and n_hard [B] (int32 counts).
+ *   All three: no atomics, no allocation, no host synchronisation.
+ */
+int ltgnn_edge_mask_fwd(ltgnn_graph_t g, int64_t B, int32_t n_edges, const float* mask, int64_t mask_stride,
+                        const float* base, const float* t_base, int64_t base_stride, const int32_t* ent_edge,
+                        const int32_t* t_ent_edge, float* vals, float* t_vals, void* stream);
+int ltgnn_edge_mask_bwd(ltgnn_graph_t g, int64_t B, int32_t n_edges, const float* mask, int64_t mask_stride,
+                        const float* base, int64_t base_stride, const int32_t* ent_edge, const float* dvals, float* dmask,
+                        float* dmask_sum, float* dbase, float* dbase_sum, void* stream);
+int ltgnn_explain_step(int device, int64_t B, int32_t E, const float* g, float* m, float* s, float* exp_avg,
+                       float* exp_avg_sq, uint8_t* hard, int32_t* n_hard, int32_t* step, double lr, double beta1,
+                       double beta2, double eps, float edge_size, float edge_ent, int record, void* stream);
+
 /* ---- dense row-wise layer on tensor cores --------------------------------------------------
  * Y[M,N] = gate( act( X[M,K] op(W) + bias[N] ) )
  *   op(W) = W^T with W [N,K] row-major (w_transposed = 0, torch.nn.Linear layout)

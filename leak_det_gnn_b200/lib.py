@@ -6,7 +6,7 @@ There is deliberately no fallback: if the shared library is missing or a call fa
 from __future__ import annotations
 
 import ctypes
-from ctypes import POINTER, c_char_p, c_float, c_int, c_int32, c_int64, c_size_t, c_uint64, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_uint64, c_void_p
 from pathlib import Path
 
 _PKG = Path(__file__).resolve().parent
@@ -40,6 +40,13 @@ SIGNATURES = {
                                     c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gcn_adj_grad": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
                                    c_int, c_void_p, c_void_p]),
+    "ltgnn_edge_mask_fwd": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_edge_mask_bwd": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
+                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_explain_step": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_double, c_double, c_double, c_double, c_float, c_float, c_int,
+                                   c_void_p]),
     "ltgnn_linear": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
                              c_float, c_void_p, c_void_p]),
     "ltgnn_wgrad_ws_floats": (c_int64, [c_int, c_int32, c_int32]),

@@ -137,18 +137,20 @@ class LeakDetector(nn.Module):
             self._dev_cache[key] = hit
         return hit
 
-    def gnn_stack(self, h_s: torch.Tensor, edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def gnn_stack(self, h_s: torch.Tensor, edge_weight: Optional[torch.Tensor] = None,
+                  edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Sensor embeddings (B, S, d_s) -> logits (B, P+1): reference detector.py:178-218, the
         message-passing hot path (SURVEY.md section 8a rows a4-a12).  ``edge_weight``: optional weights of the edges
         of ``edge_index_single`` -- (E,) shared by every window or (B, E) -- used by every GCN layer, as PyG's
         ``conv(x, edge_index, edge_weight)``; edges ``2p`` and ``2p + 1`` are the two directions of link ``p``.  Their
-        gradient is the per-pipe attribution of a logit (INTEGRATION section 2)."""
+        gradient is the per-pipe attribution of a logit (INTEGRATION section 2).  ``edge_mask``: PyG's explainer
+        edge mask, same shapes, on every GCN layer's messages after the normalisation (see :mod:`..explain`)."""
         if not h_s.is_cuda:
             raise ValueError("LeakDetector runs on CUDA only (sm_100a kernels; no CPU fallback)")
         slot, _, ends32, incidence = self._index_tensors(h_s.device)
         conv_params = [t for conv in self.convs for t in (conv.lin.weight, conv.bias)]
         x = ops.gnn_body(h_s, slot, self.pipe_graph, self.dropout.p, self.training, self.sensor_to_node.weight,
-                         self.sensor_to_node.bias, conv_params, edge_weight=edge_weight)
+                         self.sensor_to_node.bias, conv_params, edge_weight=edge_weight, edge_mask=edge_mask)
         lin1, lin2 = self.edge_head.mlp[0], self.edge_head.mlp[3]
         # pipe head (features formed on the fly, tcgen05) + mean pool; the H -> 1 layer's bias and the tiny no-leak MLP
         # on the pooled (B, D) vector stay in torch.  Node widths other than 64 / 128 raise inside ops.heads.
@@ -158,6 +160,6 @@ class LeakDetector(nn.Module):
         return torch.cat([pipe_logits, noleak_logit], dim=-1)
 
     def forward(self, residual: torch.Tensor, tfeat: Optional[torch.Tensor] = None,
-                edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+                edge_weight: Optional[torch.Tensor] = None, edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         h_s = self.sensor_encoder(residual, tfeat)
-        return self.gnn_stack(h_s, edge_weight)
+        return self.gnn_stack(h_s, edge_weight, edge_mask)

@@ -14,7 +14,8 @@ zero).  ``forward`` accepts
 Both take PyG's third argument ``edge_weight``: one weight per edge of ``edge_index`` (the graph's, or the replicated
 one's), or with a ``PipeGraph`` also (B, E), one row per window.  The weights are normalised on the device on every call
 (``gcn_norm`` with self loops; a node's existing self loop keeps its weight, an added one weighs 1) and are
-differentiable.
+differentiable.  ``edge_mask`` (same shapes) is PyG's explainer mask: it scales each edge's message after the
+normalisation, leaves the added self loops unmasked, and is differentiable (``explain_message`` of PyG 2.x).
 """
 from __future__ import annotations
 
@@ -84,10 +85,10 @@ class GCNConv(nn.Module):
             nn.init.zeros_(self.bias)
 
     def forward(self, x: torch.Tensor, graph: Union[PipeGraph, torch.Tensor],
-                edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+                edge_weight: Optional[torch.Tensor] = None, edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         if isinstance(graph, torch.Tensor):
             graph = _graph_from_edge_index(graph, x.shape[0] if x.dim() == 2 else x.shape[-2])
-        return ops.gcn_conv(x, graph, self.lin.weight, self.bias, edge_weight)
+        return ops.gcn_conv(x, graph, self.lin.weight, self.bias, edge_weight, edge_mask)
 
     def extra_repr(self) -> str:
         return f"{self.in_channels}, {self.out_channels}"

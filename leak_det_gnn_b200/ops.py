@@ -17,7 +17,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad"]
+__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad", "edge_mask_fwd", "explain_step"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -456,17 +456,23 @@ def node_init_bwd(h_s, slot, weight, dx0, x0, gate_scale, live=None):
 # ----------------------------------------------------------------------------------------------
 # per-call edge weights: PyG's gcn_norm on the device and the gradient with respect to the adjacency values
 # ----------------------------------------------------------------------------------------------
-def _check_edge_weight(graph: PipeGraph, w: torch.Tensor, b: int) -> None:
+def _check_edge_weight(graph: PipeGraph, w: torch.Tensor, b: int, name: str = "edge_weight") -> None:
     if not isinstance(w, torch.Tensor):
-        raise ValueError("edge_weight must be a tensor")
+        raise ValueError(f"{name} must be a tensor")
     e = graph.num_edges
     if not (tuple(w.shape) == (e,) or (w.dim() == 2 and tuple(w.shape) == (b, e))):
-        raise ValueError(f"edge_weight must be ({e},) (shared by every window) or ({b}, {e}) (one row per window), "
+        raise ValueError(f"{name} must be ({e},) (shared by every window) or ({b}, {e}) (one row per window), "
                          f"got {tuple(w.shape)}")
     if not w.is_cuda:
-        raise ValueError("edge_weight must be a CUDA tensor (libltgnn has no CPU path)")
+        raise ValueError(f"{name} must be a CUDA tensor (libltgnn has no CPU path)")
     if w.dtype != torch.float32:
-        raise ValueError(f"edge_weight must be float32, got {w.dtype}")
+        raise ValueError(f"{name} must be float32, got {w.dtype}")
+
+
+def _check_edge_mask(graph: PipeGraph, m: torch.Tensor, b: int) -> None:
+    _check_edge_weight(graph, m, b, "edge_mask")
+    if not m.is_contiguous():
+        raise ValueError("edge_mask must be contiguous")
 
 
 def edge_norm(graph: PipeGraph, w: torch.Tensor):
@@ -556,10 +562,131 @@ class _EdgeNorm(torch.autograd.Function):
         return edge_norm_bwd(ctx.graph, w, dis, dvals), None
 
 
-def normalized_edge_values(graph: PipeGraph, edge_weight: torch.Tensor, b: int):
-    """Differentiable ``(vals, t_vals)`` of ``edge_weight`` ((E,) or (b, E)) for the weighted layers."""
-    _check_edge_weight(graph, edge_weight, b)
-    return _EdgeNorm.apply(edge_weight, graph)
+def edge_mask_fwd(graph: PipeGraph, mask: torch.Tensor, base: Optional[torch.Tensor] = None,
+                  t_base: Optional[torch.Tensor] = None):
+    """Raw message mask (see ltgnn_edge_mask_fwd): mask (E,) or (Bm, E) in ``edge_index`` order on the entry values
+    ``base`` / ``t_base`` ((1 or Bv, nnz) in A_hat / A_hat^T order, e.g. :func:`edge_norm`'s) or on the graph's own
+    (both ``None``) -> masked ``(vals, t_vals)``, (max(Bm, Bv), nnz) each; gcn_norm's self loops keep factor 1."""
+    _check_act(mask, "edge_mask")
+    m2 = mask.view(1, -1) if mask.dim() == 1 else mask
+    if m2.dim() != 2 or m2.shape[1] != graph.num_edges:
+        raise ValueError(f"edge_mask rows must hold {graph.num_edges} values, got {tuple(mask.shape)}")
+    rows = m2.shape[0]
+    if base is not None:
+        _check_act(base, "base")
+        _check_act(t_base, "t_base")
+        if base.shape != t_base.shape or base.dim() != 2 or base.shape[1] != graph.nnz:
+            raise ValueError(f"base and t_base must both be (rows, {graph.nnz})")
+        if 1 not in (rows, base.shape[0]) and rows != base.shape[0]:
+            raise ValueError(f"edge_mask rows ({rows}) and base rows ({base.shape[0]}) do not broadcast")
+        rows = max(rows, base.shape[0])
+    ent, t_ent, _ = graph.edge_maps(mask.device)
+    vals = torch.empty(rows, graph.nnz, device=mask.device, dtype=torch.float32)
+    t_vals = torch.empty_like(vals)
+    tok = _inst.begin("edge_mask_fwd")
+    _lib.check(_lib.load().ltgnn_edge_mask_fwd(graph.handle(mask.device), rows, graph.num_edges, m2.data_ptr(),
+                                               0 if m2.shape[0] == 1 else graph.num_edges,
+                                               None if base is None else base.data_ptr(),
+                                               None if t_base is None else t_base.data_ptr(),
+                                               0 if base is None or base.shape[0] == 1 else graph.nnz, ent.data_ptr(),
+                                               t_ent.data_ptr(), vals.data_ptr(), t_vals.data_ptr(), _stream(mask)))
+    _inst.end(tok)
+    return vals, t_vals
+
+
+def edge_mask_bwd(graph: PipeGraph, mask: torch.Tensor, dvals: torch.Tensor, base: Optional[torch.Tensor] = None,
+                  want_base: bool = False):
+    """Raw backward of :func:`edge_mask_fwd`: d vals (rows, nnz) in A_hat order -> ``(d mask, d base)`` of the shapes of
+    ``mask`` and ``base`` (``d base`` only with ``want_base``, else ``None``); an operand with one row shared by
+    several output rows gets the sum over them."""
+    m2 = mask.view(1, -1) if mask.dim() == 1 else mask
+    dvals = dvals.contiguous()
+    rows, e, nnz = dvals.shape[0], graph.num_edges, graph.nnz
+    dev = mask.device
+    dmask = torch.empty(rows, e, device=dev, dtype=torch.float32)
+    dmask_sum = torch.empty(1, e, device=dev, dtype=torch.float32) if m2.shape[0] < rows else None
+    dbase = dbase_sum = None
+    if want_base:
+        dbase = torch.empty(rows, nnz, device=dev, dtype=torch.float32)
+        dbase_sum = torch.empty(1, nnz, device=dev, dtype=torch.float32) if base.shape[0] < rows else None
+    ent, _, _ = graph.edge_maps(dev)
+    tok = _inst.begin("edge_mask_bwd")
+    _lib.check(_lib.load().ltgnn_edge_mask_bwd(graph.handle(dev), rows, e, m2.data_ptr(), 0 if m2.shape[0] == 1 else e,
+                                               None if base is None else base.data_ptr(),
+                                               0 if base is None or base.shape[0] == 1 else nnz, ent.data_ptr(),
+                                               dvals.data_ptr(), dmask.data_ptr(),
+                                               None if dmask_sum is None else dmask_sum.data_ptr(),
+                                               None if dbase is None else dbase.data_ptr(),
+                                               None if dbase_sum is None else dbase_sum.data_ptr(), _stream(dvals)))
+    _inst.end(tok)
+    dmask = (dmask if dmask_sum is None else dmask_sum).view(mask.shape)
+    if want_base:
+        dbase = (dbase if dbase_sum is None else dbase_sum).view(base.shape)
+    return dmask, dbase
+
+
+class _EdgeMask(torch.autograd.Function):
+    """(edge_mask, vals, t_vals) -> masked (vals, t_vals): PyG's explainer mask on each message after the normalisation.
+    ``vals`` / ``t_vals`` ``None``: the graph's own values.  Differentiable in the mask and in ``vals`` (and so, through
+    :class:`_EdgeNorm`, in ``edge_weight``)."""
+
+    @staticmethod
+    def forward(ctx, mask, vals, t_vals, graph):
+        mvals, mt_vals = edge_mask_fwd(graph, mask, vals, t_vals)
+        ctx.mark_non_differentiable(mt_vals)
+        ctx.save_for_backward(mask, vals)
+        ctx.graph = graph
+        return mvals, mt_vals
+
+    @staticmethod
+    def backward(ctx, dvals, _dt_vals):
+        mask, vals = ctx.saved_tensors
+        if dvals is None:
+            return None, None, None, None
+        dmask, dbase = edge_mask_bwd(ctx.graph, mask, dvals, vals, want_base=ctx.needs_input_grad[1])
+        return dmask, dbase, None, None
+
+
+def normalized_edge_values(graph: PipeGraph, edge_weight: Optional[torch.Tensor], b: int,
+                           edge_mask: Optional[torch.Tensor] = None):
+    """Differentiable ``(vals, t_vals)`` of ``edge_weight`` ((E,) or (b, E); ``None``: the graph's own normalisation)
+    for the weighted layers, each message scaled by ``edge_mask`` ((E,) or (b, E)) when one is given.  Both are
+    validated before anything is launched."""
+    if edge_weight is not None:
+        _check_edge_weight(graph, edge_weight, b)
+    if edge_mask is not None:
+        _check_edge_mask(graph, edge_mask, b)
+    vals = t_vals = None
+    if edge_weight is not None:
+        vals, t_vals = _EdgeNorm.apply(edge_weight, graph)
+    if edge_mask is not None:
+        vals, t_vals = _EdgeMask.apply(edge_mask, vals, t_vals, graph)
+    return vals, t_vals
+
+
+def explain_step(g: torch.Tensor, m: torch.Tensor, s: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor,
+                 hard: torch.Tensor, n_hard: torch.Tensor, step: torch.Tensor, record: bool, lr: float = 0.01,
+                 edge_size: float = 0.005, edge_ent: float = 1.0, betas=(0.9, 0.999), eps: float = 1e-8) -> None:
+    """One GNNExplainer epoch on (B, E) mask logits, in place (see ltgnn_explain_step): ``g`` = d loss / d ``s``,
+    ``s`` = sigmoid(``m``); Adam state ``exp_avg`` / ``exp_avg_sq`` and the int32 step count ``step`` (1,) on the device;
+    ``record`` (epoch 0): no regulariser, writes the hard mask ``hard`` (bool (B, E)) and its counts ``n_hard``
+    (int32 (B,)); later epochs regularise on them."""
+    for t, nm in ((g, "g"), (m, "m"), (s, "s"), (exp_avg, "exp_avg"), (exp_avg_sq, "exp_avg_sq")):
+        _check_act(t, nm)
+        if t.dim() != 2 or t.shape != m.shape:
+            raise ValueError(f"explain_step: {nm} must be (B, E) like m {tuple(m.shape)}")
+    b, e = m.shape
+    if hard.dtype != torch.bool or hard.shape != m.shape or not hard.is_contiguous():
+        raise ValueError("explain_step: hard must be a contiguous bool tensor shaped like m")
+    for t, nm, shape in ((n_hard, "n_hard", (b,)), (step, "step", (1,))):
+        if t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_cuda:
+            raise ValueError(f"explain_step: {nm} must be an int32 CUDA tensor of shape {shape}")
+    tok = _inst.begin("explain_step")
+    _lib.check(_lib.load().ltgnn_explain_step(_dev_index(m), b, e, g.data_ptr(), m.data_ptr(), s.data_ptr(),
+                                              exp_avg.data_ptr(), exp_avg_sq.data_ptr(), hard.data_ptr(), n_hard.data_ptr(),
+                                              step.data_ptr(), float(lr), float(betas[0]), float(betas[1]), float(eps),
+                                              float(edge_size), float(edge_ent), int(bool(record)), _stream(m)))
+    _inst.end(tok)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -608,16 +735,18 @@ class _GcnConv(torch.autograd.Function):
 
 
 def gcn_conv(x: torch.Tensor, graph: PipeGraph, weight: torch.Tensor, bias: Optional[torch.Tensor],
-             edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+             edge_weight: Optional[torch.Tensor] = None, edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
     """``A_hat (x W^T) + b`` -- the operator ``torch_geometric.nn.GCNConv.forward`` computes
     (reference call site models/detector.py:199).  x: (B, N, Din) or (B*N, Din), fp32 CUDA.  ``edge_weight``: PyG's
     per-edge weights in ``edge_index`` order, (E,) shared by every window or (B, E), normalised on the device
-    (gcn_norm with self loops) on each call and differentiable; ``None`` runs the graph's own normalised adjacency."""
+    (gcn_norm with self loops) on each call and differentiable; ``None`` runs the graph's own normalised adjacency.
+    ``edge_mask``: PyG's explainer mask, same shapes, scaling each edge's message after the normalisation (the self
+    loops gcn_norm adds are not masked; an input self loop's value has no effect); differentiable."""
     _check_act(x.contiguous(), "x")
-    if edge_weight is None:
+    if edge_weight is None and edge_mask is None:
         return _GcnConv.apply(x, weight, bias, graph)
     b = x.numel() // (graph.num_nodes * x.shape[-1])
-    vals, t_vals = normalized_edge_values(graph, edge_weight, b)
+    vals, t_vals = normalized_edge_values(graph, edge_weight, b, edge_mask)
     return _GcnConv.apply(x, weight, bias, graph, vals, t_vals)
 
 
@@ -733,6 +862,8 @@ class _Heads(torch.autograd.Function):
                                             _stream(x)))
         _inst.end(tok)
         del ws
+        if not any(ctx.needs_input_grad[4:7]):  # frozen head
+            return dx, None, None, None, None, None, None, None, None
         # parameter gradients: dW1 on tensor cores with operands formed on the fly; db1 and dw2 from the same accumulators
         dw1 = torch.empty_like(w1)
         db1 = torch.empty(h, device=x.device, dtype=torch.float32)
@@ -823,18 +954,20 @@ class _HeadsWide(torch.autograd.Function):
                                         gq.data_ptr(), cs.data_ptr(), ws.data_ptr(), _stream(x)))
         _inst.end(tok)
         # parameter gradients: T[t] = gq^T F[t] on the tensor cores; dW1, db1, dw2 follow from T and cs (the hidden layer is
-        # linear in W1, b1 under the gate -- no second pass over the hidden activations)
-        t3 = torch.empty(3, h, d, device=x.device, dtype=torch.float32)
-        for t in range(3):
-            wgrad(gq, feat[t], out=t3[t])
-        dw1 = torch.empty_like(w1)
-        db1 = torch.empty(h, device=x.device, dtype=torch.float32)
-        dw2 = torch.empty(1, h, device=x.device, dtype=torch.float32)
-        w1c, b1c = w1.detach().contiguous(), b1.detach().contiguous()
-        tok = _inst.begin("head_wide_finish")
-        _lib.check(L.ltgnn_head_wide_finish(dev, h, d, t3.data_ptr(), w1c.data_ptr(), b1c.data_ptr(), w2v.data_ptr(),
-                                            cs.data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), _stream(x)))
-        _inst.end(tok)
+        # linear in W1, b1 under the gate -- no second pass over the hidden activations).  Skipped for a frozen head.
+        dw1 = db1 = dw2 = None
+        if any(ctx.needs_input_grad[4:7]):
+            t3 = torch.empty(3, h, d, device=x.device, dtype=torch.float32)
+            for t in range(3):
+                wgrad(gq, feat[t], out=t3[t])
+            dw1 = torch.empty_like(w1)
+            db1 = torch.empty(h, device=x.device, dtype=torch.float32)
+            dw2 = torch.empty(1, h, device=x.device, dtype=torch.float32)
+            w1c, b1c = w1.detach().contiguous(), b1.detach().contiguous()
+            tok = _inst.begin("head_wide_finish")
+            _lib.check(L.ltgnn_head_wide_finish(dev, h, d, t3.data_ptr(), w1c.data_ptr(), b1c.data_ptr(), w2v.data_ptr(),
+                                                cs.data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), _stream(x)))
+            _inst.end(tok)
         dfeat = torch.empty_like(feat)
         for t in range(3):
             linear_tc(dh, w3[t], transposed=True, out=dfeat[t])                        # dF_t = dh W1[:, tD:(t+1)D]
@@ -934,6 +1067,12 @@ class _GnnBody(torch.autograd.Function):
         xs = saved[3 + L_:3 + 2 * L_ + 1]
         t_vals, xws = saved[3 + 2 * L_ + 1], saved[3 + 2 * L_ + 2:]
         graph, scale = ctx.graph, ctx.scale
+        need = ctx.needs_input_grad
+        # below[l]: the gradient at layer l's input is needed -- by node init (h_s, w0, b0), by a lower layer's
+        # parameters, or by a lower layer's d A_hat (which reads it at that layer's output).  A frozen stack skips the rest.
+        below = [need[0] or need[7] or need[8]]
+        for l in range(1, L_):
+            below.append(below[-1] or need[7 + 2 * l] or need[8 + 2 * l] or bool(xws))
         g = dx.contiguous()
         grads = [None] * (2 * L_)
         dvals = None
@@ -943,25 +1082,37 @@ class _GnnBody(torch.autograd.Function):
             if xws:  # d A_hat of this layer, gated exactly as the aggregation below gates g; layers add up
                 dvals = gcn_adj_grad(graph, g, xws[l], gate=x_out if live is None else None, live_in=live,
                                      gate_scale=scale, out=dvals, shared=ctx.shared, accumulate=dvals is not None)
-            gz, db = spmm_fused(graph, g, transpose=True, gate=x_out if live is None else None, live_in=live,
-                                gate_scale=scale, want_colsum=True, vals=t_vals)
-            grads[2 * l] = wgrad(gz, x_in)
-            grads[2 * l + 1] = db
+            want_w, want_b = need[9 + 2 * l], need[10 + 2 * l]
+            if not (want_w or want_b or below[l]):
+                break
+            gz = spmm_fused(graph, g, transpose=True, gate=x_out if live is None else None, live_in=live,
+                            gate_scale=scale, want_colsum=want_b, vals=t_vals)
+            if want_b:
+                gz, grads[2 * l + 1] = gz
+            if want_w:
+                grads[2 * l] = wgrad(gz, x_in)
+            if not below[l]:
+                break
             g = _linear_any(gz, w, transposed=True)
             del gz
-        dhs, dw0, db0 = node_init_bwd(h_s, slot, w0, g, xs[0], scale, live=ctx.lives[0])
+        dhs = dw0 = db0 = None
+        if below[0]:
+            dhs, dw0, db0 = node_init_bwd(h_s, slot, w0, g, xs[0], scale, live=ctx.lives[0])
         return (dhs, None, None, None, None, dvals, None, dw0, db0, *grads)
 
 
 def gnn_body(h_s: torch.Tensor, slot: torch.Tensor, graph: PipeGraph, drop_p: float, training: bool,
-             w0: torch.Tensor, b0: torch.Tensor, conv_params, edge_weight: Optional[torch.Tensor] = None) -> torch.Tensor:
+             w0: torch.Tensor, b0: torch.Tensor, conv_params, edge_weight: Optional[torch.Tensor] = None,
+             edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Sensor embeddings (B,S,ds) -> node states after the last GCN layer (B,N,D).  ``edge_weight``: (E,) or (B, E)
     weights of the graph's edges, normalised once on the device and used by every layer (as PyG passes one
-    ``edge_weight`` to every conv); differentiable.  ``None``: the graph's own adjacency, on the one-kernel layers."""
+    ``edge_weight`` to every conv); differentiable.  ``edge_mask``: (E,) or (B, E) explainer mask on every layer's
+    messages after the normalisation (as PyG's ``set_masks`` puts one mask on every conv); differentiable.  Both
+    ``None``: the graph's own adjacency, on the one-kernel layers."""
     _check_act(h_s.contiguous(), "h_s")
     vals = t_vals = None
-    if edge_weight is not None:
-        vals, t_vals = normalized_edge_values(graph, edge_weight, h_s.shape[0])
+    if edge_weight is not None or edge_mask is not None:
+        vals, t_vals = normalized_edge_values(graph, edge_weight, h_s.shape[0], edge_mask)
     return _GnnBody.apply(h_s, slot, graph, drop_p, training, vals, t_vals, w0, b0, *conv_params)
 
 
