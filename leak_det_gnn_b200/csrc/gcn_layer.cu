@@ -351,6 +351,20 @@ gcn_layer_fwd_kernel(const Params p) {
 
 inline uint32_t align_up(uint32_t x, uint32_t a) { return (x + a - 1) / a * a; }
 
+// Shared memory a launch may ask for: the opt-in limit bounds dynamic + static bytes, and the kernel's barriers are
+// static.  0 if the kernel's attributes cannot be read.
+inline uint32_t dynamic_smem_limit(int smem_optin) {
+    static const int static_bytes = [] {
+        cudaFuncAttributes a{};
+        if (cudaFuncGetAttributes(&a, gcn_layer_fwd_kernel) != cudaSuccess) {
+            (void)cudaGetLastError();
+            return -1;
+        }
+        return static_cast<int>(a.sharedSizeBytes);
+    }();
+    return static_bytes < 0 || static_bytes >= smem_optin ? 0u : static_cast<uint32_t>(smem_optin - static_bytes);
+}
+
 }  // namespace gl
 }  // namespace
 
@@ -361,7 +375,7 @@ extern "C" int ltgnn_gcn_layer_supported(ltgnn_graph_t g, int32_t K, int32_t D) 
     if (T > gl::kMaxTiles || T * D + 2 * gl::kSlotCols > 512) return 0;  // accumulators + at least two A slots
     const uint32_t fixed = gl::align_up(2u * D * K * 4 + gl::align_up(static_cast<uint32_t>(g->n) * 128, 128) +
                                             gl::align_up(4u * (g->n + 1), 16) + 8u * g->nnz, 1024);
-    return 1024 + fixed + gl::kLdWarps * 2 * patch::kPatchBytes <= static_cast<uint32_t>(g->smem_optin);
+    return 1024 + fixed + gl::kLdWarps * 2 * patch::kPatchBytes <= gl::dynamic_smem_limit(g->smem_optin);
 }
 
 extern "C" int ltgnn_gcn_layer_fwd(ltgnn_graph_t g, int64_t B, int32_t K, int32_t D, const float* X, const float* W,
@@ -404,7 +418,7 @@ extern "C" int ltgnn_gcn_layer_fwd(ltgnn_graph_t g, int64_t B, int32_t K, int32_
     p.off_rowptr = p.off_stage + gl::align_up(static_cast<uint32_t>(g->n) * 128, 128);
     p.off_colval = p.off_rowptr + gl::align_up(4u * (g->n + 1), 16);
     p.off_ring = gl::align_up(p.off_colval + 8u * g->nnz, 1024);  // patches address chunks by XOR: keep them aligned
-    const uint32_t room = static_cast<uint32_t>(g->smem_optin) - 1024 - p.off_ring;
+    const uint32_t room = gl::dynamic_smem_limit(g->smem_optin) - 1024 - p.off_ring;
     p.depth = room >= gl::kLdWarps * 4 * patch::kPatchBytes ? 4 : 2;  // 64 KB (or 32 KB) of loads in flight
     const size_t smem = 1024 + p.off_ring + static_cast<size_t>(gl::kLdWarps) * p.depth * patch::kPatchBytes;
     LTGNN_CUDA_TRY(cudaFuncSetAttribute(gl::gcn_layer_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
