@@ -17,6 +17,7 @@ from typing import List, Tuple
 import numpy as np
 import torch
 
+from . import ops
 from .models.utils import build_residual_sequence_from_segment, residual_series
 
 
@@ -83,7 +84,7 @@ class GraphedDetector:
                 self.detector(self.residual, self.tfeat)
         torch.cuda.current_stream(dev).wait_stream(side)
         self.graph = torch.cuda.CUDAGraph()
-        with torch.no_grad(), torch.cuda.graph(self.graph):
+        with torch.no_grad(), ops.capture(self.graph):
             self.logits = self.detector(self.residual, self.tfeat)
 
     @torch.no_grad()

@@ -97,7 +97,7 @@ def explain_edges(detector, residual: torch.Tensor, tfeat: Optional[torch.Tensor
         torch.cuda.current_stream(h_s.device).wait_stream(side)
         if epochs > 1:
             graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
+            with ops.capture(graph):
                 st.epoch(*args, False, *hyper)
             for _ in range(int(epochs) - 1):
                 graph.replay()

@@ -76,14 +76,15 @@ class GraphedStep:
         self.graph_a = torch.cuda.CUDAGraph()
         self.graph_b = torch.cuda.CUDAGraph() if self.split and self.has_update else None
         counted = _inst.launches
-        with torch.cuda.graph(self.graph_a):
+        with ops.capture(self.graph_a):
             self._forward_backward()
             if not self.split:
                 self._update()
         if self.graph_b is not None:
-            with torch.cuda.graph(self.graph_b, pool=self.graph_a.pool()):
+            with ops.capture(self.graph_b, pool=self.graph_a.pool()):
                 self._update()
         self.kernels_per_replay = _inst.launches - counted       # libltgnn launches recorded into the graph(s)
+        ops._release_retired()                                   # graph handles collected during the capture
         # undo the warm-up steps: parameters back, optimiser moments and step counts to zero (addresses unchanged)
         with torch.no_grad():
             for p, k in zip(module.parameters(), keep):

@@ -6,7 +6,9 @@ device pointers and the current torch stream.  Non-CUDA / non-fp32 inputs are a
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
+import gc
 import threading
 from typing import Dict, Optional
 
@@ -17,7 +19,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad", "edge_mask_fwd", "explain_step"]
+__all__ = ["PipeGraph", "capture", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad", "edge_mask_fwd", "explain_step"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -28,6 +30,37 @@ DEBUG_CAPTURE: Optional[dict] = None
 
 def _ptr(a: np.ndarray) -> ctypes.c_void_p:
     return a.ctypes.data_as(ctypes.c_void_p)
+
+
+@contextlib.contextmanager
+def capture(graph: torch.cuda.CUDAGraph, pool=None):
+    """``torch.cuda.graph(graph, pool)`` with Python's cycle collector kept out of the capture.  A finaliser that frees
+    device memory or destroys a CUDA graph -- a dead PipeGraph's handle, the graphs of a dead training step -- is not
+    permitted while a capture is underway and invalidates it, and torch no longer collects before capturing.  So dead
+    cycles are finalised first, and no collection runs until the capture has ended."""
+    gc.collect()
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph, pool=pool):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
+
+
+# Graph handles of PipeGraphs finalised during a capture (by a caller's own torch.cuda.graph, or by reference count
+# inside one), waiting for ltgnn_graph_destroy: its cudaFree is not permitted during a capture.  They are released at
+# the next release point with no capture underway on this thread.
+_RETIRED: list = []
+
+
+def _release_retired() -> None:
+    if not _RETIRED or torch.cuda.is_current_stream_capturing():
+        return
+    L = _lib.load()
+    while _RETIRED:
+        L.ltgnn_graph_destroy(_RETIRED.pop())
 
 
 class PipeGraph:
@@ -55,6 +88,7 @@ class PipeGraph:
         idx = device.index if device.index is not None else torch.cuda.current_device()
         h = self._handles.get(idx)
         if h is None:
+            _release_retired()
             with self._lock:
                 h = self._handles.get(idx)
                 if h is None:
@@ -86,9 +120,9 @@ class PipeGraph:
 
     def __del__(self) -> None:  # best effort; the handle only owns ~40 KB of device memory
         try:
-            L = _lib.load()
-            for h in self._handles.values():
-                L.ltgnn_graph_destroy(h)
+            _RETIRED.extend(self._handles.values())
+            self._handles.clear()
+            _release_retired()
         except Exception:
             pass
 

@@ -127,3 +127,61 @@ def test_graphed_step_draws_fresh_dropout_masks(graph_golden):
     a, b = losses(), losses()
     assert len(set(a)) == 4, a
     assert a == b
+
+
+
+def test_capture_keeps_the_cycle_collector_out():
+    """ops.capture (used by the graphed steps and the explainer) finalises dead cycles before capturing -- here one
+    holding a captured CUDA graph, whose destruction is not permitted during a capture -- and runs no collection
+    until the capture has ended."""
+    import gc
+    import weakref
+
+    from leak_det_gnn_b200 import ops
+
+    class Holder:
+        pass
+
+    x = torch.arange(8.0, device="cuda")
+    dead = Holder()
+    dead.graph = torch.cuda.CUDAGraph()
+    with ops.capture(dead.graph):
+        x.add_(1.0)
+    dead.cycle = dead
+    gone = weakref.ref(dead)
+    del dead
+    cg = torch.cuda.CUDAGraph()
+    with ops.capture(cg):
+        state = (gone() is None, gc.isenabled())
+        y = x * 2
+    assert state == (True, False) and gc.isenabled()
+    x.fill_(3.0)
+    cg.replay()
+    torch.cuda.synchronize()
+    assert torch.equal(y, torch.full_like(x, 6.0))
+
+
+def test_pipe_graph_finalised_during_a_capture_is_released_after_it():
+    """A PipeGraph finalised inside a caller's own capture keeps its device arrays until no capture is underway:
+    cudaFree is not permitted during a capture and would invalidate it."""
+    import gc
+
+    from leak_det_gnn_b200 import ops
+
+    dev = torch.device("cuda")
+    dead = ops.PipeGraph(torch.tensor([[0, 1], [1, 0]]), 2)
+    hv = dead.handle(dev).value
+    x = torch.arange(8.0, device=dev)
+    gc.collect()
+    cg = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(cg):
+        y = x * 2
+        del dead                         # finalised here, by reference count
+        parked = [h.value for h in ops._RETIRED]
+    x.fill_(3.0)
+    cg.replay()
+    torch.cuda.synchronize()
+    assert hv in parked and torch.equal(y, torch.full_like(x, 6.0))
+    live = ops.PipeGraph(torch.tensor([[0, 1], [1, 0]]), 2)
+    live.handle(dev)                     # the next handle, outside any capture, releases the parked one
+    assert not ops._RETIRED
