@@ -175,6 +175,31 @@ int ltgnn_explain_step(int device, int64_t B, int32_t E, const float* g, float* 
                        float* exp_avg_sq, uint8_t* hard, int32_t* n_hard, int32_t* step, double lr, double beta1,
                        double beta2, double eps, float edge_size, float edge_ent, int record, void* stream);
 
+/* ---- PGExplainer's edge network (PyG 2.x, torch_geometric/explain/algorithm/pg_explainer.py) ----------------
+ * The MLP Linear(2D, 64) -> ReLU -> Linear(64, 1) on [z[src] | z[dst]], factored per node: pq [B*N][128] = [P | Q]
+ * = z [W1a; W1b]^T (one ltgnn_linear), then per edge e of window b (src / dst [E] int32 node indices)
+ *   pre = (P[b, src[e]] + Q[b, dst[e]]) + b1,  logit = w2 . relu(pre) + *b2   (b1, w2 [64] and b2 [1] on the device).
+ * ltgnn_pg_edge_fwd: inv_t NULL (explaining): mask [B][E] = sigmoid(logit), nothing else written.
+ *   inv_t (device scalar 1 / T, training): the concrete sample s [B][E] = (log eps - log(1 - eps) + logit) * (1 / T),
+ *   eps = (1 - 2 bias) U + bias, U in [0, 1) from Philox keyed by seed (+ the ltgnn_seed_source word when one is set)
+ *   and the edge's index b * E + e; mask = sigmoid(s); gate [B][E][2] uint32: bit l of word j = (pre of unit 2l + j
+ *   > 0); uniform (NULL or [B][E]) receives U.  bias in [0, 0.5]; 0.5 is noise-free.
+ * ltgnn_pg_edge_bwd: from dmask [B][E] (the gradient at fwd's mask) and fwd's mask, gate and inv_t:
+ *   dlogit = dmask s(1 - s) / T,  gh[u] = dlogit w2[u] [pre_u > 0];  R [B*N][128]: R[b, n, :64] = sum of gh over the
+ *   edges with src = n, R[b, n, 64:] over those with dst = n, in ascending edge order (out_ptr / out_edge [N+1] / [E]:
+ *   the edges by source, in_ptr / in_edge by target, each ascending) -- d pq; dparams [129] = d b1 [64] | d w2 [64] |
+ *   d b2 (relu(pre) recomputed in the forward's order), per-CTA partials (ws: ltgnn_pg_edge_bwd_ws_floats floats)
+ *   summed in a fixed order.  Both: no atomics, no allocation, no host synchronisation; any N (gathers through L2).
+ */
+int ltgnn_pg_edge_fwd(int device, int64_t B, int32_t N, int32_t E, const int32_t* src, const int32_t* dst,
+                      const float* pq, const float* b1, const float* w2, const float* b2, const float* inv_t, float bias,
+                      uint64_t seed, float* mask, float* s, uint32_t* gate, float* uniform, void* stream);
+int64_t ltgnn_pg_edge_bwd_ws_floats(int device);
+int ltgnn_pg_edge_bwd(int device, int64_t B, int32_t N, int32_t E, const int32_t* out_ptr, const int32_t* out_edge,
+                      const int32_t* in_ptr, const int32_t* in_edge, const int32_t* dst, const float* pq, const float* b1,
+                      const float* w2, const float* inv_t, const float* mask, const float* dmask, const uint32_t* gate,
+                      float* R, float* dparams, float* ws, void* stream);
+
 /* ---- dense row-wise layer on tensor cores --------------------------------------------------
  * Y[M,N] = gate( act( X[M,K] op(W) + bias[N] ) )
  *   op(W) = W^T with W [N,K] row-major (w_transposed = 0, torch.nn.Linear layout)

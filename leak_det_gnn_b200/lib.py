@@ -47,6 +47,12 @@ SIGNATURES = {
     "ltgnn_explain_step": (c_int, [c_int, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p, c_void_p, c_double, c_double, c_double, c_double, c_float, c_float, c_int,
                                    c_void_p]),
+    "ltgnn_pg_edge_fwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_void_p, c_float, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ltgnn_pg_edge_bwd_ws_floats": (c_int64, [c_int]),
+    "ltgnn_pg_edge_bwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_void_p]),
     "ltgnn_linear": (c_int, [c_int, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
                              c_float, c_void_p, c_void_p]),
     "ltgnn_wgrad_ws_floats": (c_int64, [c_int, c_int32, c_int32]),

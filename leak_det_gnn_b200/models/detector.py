@@ -159,6 +159,21 @@ class LeakDetector(nn.Module):
         noleak_logit = self.noleak_head(pooled).unsqueeze(-1)
         return torch.cat([pipe_logits, noleak_logit], dim=-1)
 
+    def embeddings(self, h_s: torch.Tensor) -> torch.Tensor:
+        """Sensor embeddings (B, S, d_s) -> node embeddings (B, N, D): PyG's ``get_embeddings(model, ...)[-1]``, the
+        last GCN layer's output ``A_hat (x W^T) + b`` before the ReLU and dropout that follow it, computed in eval mode
+        without gradient and without a mask -- what PGExplainer's edge network reads (see :mod:`..explain`)."""
+        if not h_s.is_cuda:
+            raise ValueError("LeakDetector runs on CUDA only (sm_100a kernels; no CPU fallback)")
+        slot = self._index_tensors(h_s.device)[0]
+        conv_params = [t for conv in self.convs[:-1] for t in (conv.lin.weight, conv.bias)]
+        last = self.convs[-1]
+        with torch.no_grad():
+            x = ops.gnn_body(h_s, slot, self.pipe_graph, 0.0, False, self.sensor_to_node.weight,
+                             self.sensor_to_node.bias, conv_params)
+            xw = ops._linear_any(x, last.lin.weight)
+            return ops.spmm_fused(self.pipe_graph, xw.view(x.shape[0], x.shape[1], -1), bias=last.bias)
+
     def forward(self, residual: torch.Tensor, tfeat: Optional[torch.Tensor] = None,
                 edge_weight: Optional[torch.Tensor] = None, edge_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
         h_s = self.sensor_encoder(residual, tfeat)

@@ -19,7 +19,7 @@ from . import instrument as _inst
 from . import lib as _lib
 from .graph import GCNCsr, build_gcn_csr
 
-__all__ = ["PipeGraph", "capture", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad", "edge_mask_fwd", "explain_step"]
+__all__ = ["PipeGraph", "capture", "device_seed", "spmm", "spmm_fused", "aggregate", "linear_tc", "wgrad", "gcn_conv", "mean_pool", "gnn_body", "heads", "heads_supported", "heads_wide_supported", "pipe_incidence", "gru_encode", "gru_supported", "tcn_cone", "gru_predictor_fwd", "gru_predictor_cone", "row_gather_sum", "tcn_windows", "gru_windows", "edge_norm", "gcn_adj_grad", "edge_mask_fwd", "explain_step", "pg_edge_index", "pg_edge_mask"]
 
 
 # Test hook: when set to a dict, the autograd nodes drop the masks they saved into it (``lives``: the 1-bit ReLU-and-
@@ -721,6 +721,154 @@ def explain_step(g: torch.Tensor, m: torch.Tensor, s: torch.Tensor, exp_avg: tor
                                               step.data_ptr(), float(lr), float(betas[0]), float(betas[1]), float(eps),
                                               float(edge_size), float(edge_ent), int(bool(record)), _stream(m)))
     _inst.end(tok)
+
+
+# ----------------------------------------------------------------------------------------------
+# PGExplainer's edge network (csrc/pg_explain.cu): [P | Q] = z [W1a; W1b]^T on the tensor cores, then per edge
+# sigmoid(w2 . relu(P[src] + Q[dst] + b1) + b2), with PyG's concrete sample in training
+# ----------------------------------------------------------------------------------------------
+PG_HIDDEN = 64  # PyG's PGExplainer MLP: Linear(2D, 64) -> ReLU -> Linear(64, 1)
+
+
+def pg_edge_index(edge_index: torch.Tensor, num_nodes: int, device: torch.device) -> tuple:
+    """``(src, dst, out_ptr, out_edge, in_ptr, in_edge)`` int32 on ``device``: each edge's end nodes, and the edges
+    grouped by source and by target, ascending within a node -- what ltgnn_pg_edge_fwd / _bwd read.  Host work, once
+    per graph."""
+    ei = edge_index.detach().cpu().numpy().astype(np.int64)
+    if ei.ndim != 2 or ei.shape[0] != 2 or (ei.size and (ei.min() < 0 or ei.max() >= num_nodes)):
+        raise ValueError(f"edge_index must be (2, E) with node indices in [0, {num_nodes})")
+    out = [ei[0], ei[1]]
+    for row in (ei[0], ei[1]):
+        ptr = np.zeros(num_nodes + 1, dtype=np.int64)
+        np.cumsum(np.bincount(row, minlength=num_nodes), out=ptr[1:])
+        out += [ptr, np.argsort(row, kind="stable")]
+    return tuple(torch.from_numpy(np.ascontiguousarray(a, dtype=np.int32)).to(device) for a in out)
+
+
+def _check_pg_mlp(d: int, w1, b1, w2, b2) -> None:
+    want = ((w1, (PG_HIDDEN, 2 * d), "mlp.0.weight"), (b1, (PG_HIDDEN,), "mlp.0.bias"), (w2, (1, PG_HIDDEN), "mlp.2.weight"),
+            (b2, (1,), "mlp.2.bias"))
+    for t, shape, nm in want:
+        _check_act(t, nm)
+        if tuple(t.shape) != shape:
+            raise ValueError(f"{nm} must be {shape} for node width {d}, got {tuple(t.shape)}")
+
+
+def pg_edge_fwd(pq: torch.Tensor, idx: tuple, b1: torch.Tensor, w2: torch.Tensor, b2: torch.Tensor,
+                inv_t: Optional[torch.Tensor] = None, bias: float = 0.01, seed: int = 0,
+                uniform: Optional[torch.Tensor] = None):
+    """Raw edge network (see ltgnn_pg_edge_fwd) on ``pq`` (B, N, 128) = [P | Q] with ``idx`` from
+    :func:`pg_edge_index`.  ``inv_t`` ``None``: returns the mask sigmoid(logit) (B, E).  ``inv_t`` (a one-element
+    device tensor 1 / T): returns ``(mask, s, gate)`` of the concrete sample, ``uniform`` (B, E) receiving the draws."""
+    b, n = pq.shape[0], pq.shape[1]
+    e = idx[0].numel()
+    mask = torch.empty(b, e, device=pq.device, dtype=torch.float32)
+    s = gate = None
+    if inv_t is not None:
+        s = torch.empty_like(mask)
+        gate = torch.empty(b, e, 2, device=pq.device, dtype=torch.int32)
+    tok = _inst.begin("pg_edge_fwd")
+    _lib.check(_lib.load().ltgnn_pg_edge_fwd(_dev_index(pq), b, n, e, idx[0].data_ptr(), idx[1].data_ptr(), pq.data_ptr(),
+                                             b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),
+                                             None if inv_t is None else inv_t.data_ptr(), float(bias),
+                                             int(seed) & (2**64 - 1), mask.data_ptr(), None if s is None else s.data_ptr(),
+                                             None if gate is None else gate.data_ptr(),
+                                             None if uniform is None else uniform.data_ptr(), _stream(pq)))
+    _inst.end(tok)
+    return mask if inv_t is None else (mask, s, gate)
+
+
+def pg_edge_bwd(pq: torch.Tensor, idx: tuple, b1: torch.Tensor, w2: torch.Tensor, inv_t: torch.Tensor,
+                mask: torch.Tensor, dmask: torch.Tensor, gate: torch.Tensor):
+    """Raw backward of :func:`pg_edge_fwd` in training (see ltgnn_pg_edge_bwd): d mask (B, E) -> ``(R, dparams)``,
+    R = d[P | Q] (B, N, 128) and dparams (129,) = d b1 | d w2 | d b2."""
+    b, n = pq.shape[0], pq.shape[1]
+    e = idx[0].numel()
+    dev = _dev_index(pq)
+    L = _lib.load()
+    r = torch.empty_like(pq)
+    dparams = torch.empty(2 * PG_HIDDEN + 1, device=pq.device, dtype=torch.float32)
+    ws = torch.empty(int(L.ltgnn_pg_edge_bwd_ws_floats(dev)), device=pq.device, dtype=torch.float32)
+    tok = _inst.begin("pg_edge_bwd")
+    _lib.check(L.ltgnn_pg_edge_bwd(dev, b, n, e, idx[2].data_ptr(), idx[3].data_ptr(), idx[4].data_ptr(),
+                                   idx[5].data_ptr(), idx[1].data_ptr(), pq.data_ptr(), b1.data_ptr(), w2.data_ptr(),
+                                   inv_t.data_ptr(), mask.data_ptr(), dmask.data_ptr(), gate.data_ptr(), r.data_ptr(),
+                                   dparams.data_ptr(), ws.data_ptr(), _stream(pq)))
+    _inst.end(tok)
+    return r, dparams
+
+
+class _PgProject(torch.autograd.Function):
+    """(z, W1) -> [P | Q] = z [W1a; W1b]^T, (B, N, 128): PyG's first MLP layer on [z[src] | z[dst]] without its bias,
+    factored per node (W1a acts on the source half).  Backward: d W1 only (z is the frozen detector's embedding), from
+    R^T z on the tensor cores, re-laid out as PyG's (64, 2D)."""
+
+    @staticmethod
+    def forward(ctx, z, w1):
+        d = z.shape[-1]
+        w_stack = torch.cat([w1[:, :d], w1[:, d:]], 0).contiguous()
+        ctx.save_for_backward(z)
+        return linear_tc(z, w_stack)
+
+    @staticmethod
+    def backward(ctx, dpq):
+        (z,) = ctx.saved_tensors
+        dw = wgrad(dpq.contiguous(), z)
+        return None, torch.cat([dw[:PG_HIDDEN], dw[PG_HIDDEN:]], 1)
+
+
+class _PgEdge(torch.autograd.Function):
+    """([P | Q], b1, w2, b2) -> (mask, s) of the concrete sample; differentiable in the mask (s is returned for
+    inspection).  Backward: ltgnn_pg_edge_bwd -> d[P | Q], d b1, d w2, d b2."""
+
+    @staticmethod
+    def forward(ctx, pq, b1, w2, b2, idx, inv_t, bias, seed):
+        uniform = None
+        if DEBUG_CAPTURE is not None:
+            uniform = torch.empty(pq.shape[0], idx[0].numel(), device=pq.device, dtype=torch.float32)
+            DEBUG_CAPTURE["pg_uniform"] = uniform
+        mask, s, gate = pg_edge_fwd(pq, idx, b1, w2, b2, inv_t, bias, seed, uniform)
+        if DEBUG_CAPTURE is not None:
+            DEBUG_CAPTURE["pg_gate"] = gate
+        ctx.mark_non_differentiable(s)
+        ctx.save_for_backward(pq, b1, w2, inv_t, mask, gate)
+        ctx.idx = idx
+        return mask, s
+
+    @staticmethod
+    def backward(ctx, dmask, _ds):
+        pq, b1, w2, inv_t, mask, gate = ctx.saved_tensors
+        if dmask is None:
+            return (None,) * 8
+        r, dp = pg_edge_bwd(pq, ctx.idx, b1, w2, inv_t, mask, dmask.contiguous(), gate)
+        return r, dp[:PG_HIDDEN], dp[PG_HIDDEN:2 * PG_HIDDEN].view(1, PG_HIDDEN), dp[2 * PG_HIDDEN:], None, None, None, None
+
+
+def pg_edge_mask(z: torch.Tensor, idx: tuple, w1: torch.Tensor, b1: torch.Tensor, w2: torch.Tensor, b2: torch.Tensor,
+                 inv_t: Optional[torch.Tensor] = None, bias: float = 0.01, seed: int = 0):
+    """PGExplainer's edge mask from node embeddings ``z`` (B, N, D) over the edges of ``idx`` (:func:`pg_edge_index`)
+    with the MLP ``Linear(2D, 64) -> ReLU -> Linear(64, 1)`` (``w1`` (64, 2D), ``b1`` (64,), ``w2`` (1, 64), ``b2``
+    (1,)).  ``inv_t`` ``None``: explaining, returns sigmoid(logit) (B, E).  ``inv_t`` (one-element CUDA tensor, 1 / T):
+    training, returns ``(mask, s)`` with s = (log eps - log(1 - eps) + logit) / T, eps = (1 - 2 bias) U + bias, mask =
+    sigmoid(s), differentiable in the MLP's parameters.  Every input is checked before anything is launched."""
+    _check_act(z, "z")
+    if z.dim() != 3 or z.shape[-1] % 32 or not 0 < z.shape[-1] <= 192:
+        raise ValueError(f"z must be (B, N, D) with D a multiple of 32 up to 192, got {tuple(z.shape)}")
+    _check_pg_mlp(z.shape[-1], w1, b1, w2, b2)
+    if len(idx) != 6 or any(t.dtype != torch.int32 or t.device != z.device for t in idx):
+        raise ValueError("idx must be pg_edge_index(...) on the device of z")
+    if idx[2].numel() != z.shape[1] + 1:
+        raise ValueError(f"idx is for a {idx[2].numel() - 1}-node graph, z has {z.shape[1]} nodes")
+    if inv_t is not None:
+        _check_act(inv_t, "inv_t")
+        if inv_t.numel() != 1:
+            raise ValueError("inv_t must be a one-element tensor")
+    if not 0.0 <= float(bias) <= 0.5:
+        raise ValueError(f"bias must lie in [0, 0.5], got {bias}")
+    pq = _PgProject.apply(z, w1)
+    if inv_t is None:
+        return pg_edge_fwd(pq, idx, b1, w2, b2)
+    return _PgEdge.apply(pq, b1, w2, b2, idx, inv_t, float(bias), int(seed))
 
 
 # ----------------------------------------------------------------------------------------------
