@@ -241,6 +241,16 @@ int ltgnn_node_init_bwd(int device, int64_t B, int32_t N, int32_t S, int32_t ds,
                         const int32_t* slot, const float* W, const float* dX0, const float* X0,
                         const uint32_t* live_in, float gate_scale, float* dhs, float* dW, float* dbias, float* ws,
                         void* stream);
+/* bwd_from_layer: the same three gradients for dX0 = G1 W1, the input gradient of the first GCN layer -- G1 [B,N,K] its
+ *      aggregated output gradient, W1 [K, D] its weight (GCNConv.lin.weight) -- without forming dX0: the tensor-core GEMM
+ *      gates it with live_in (required) in its epilogue and keeps only the column sums and the sensor rows.  dhs and dW
+ *      carry the bits of ltgnn_node_init_bwd on the same dX0; dbias differs by summation order.  K a multiple of 32 up to
+ *      128, D 64 or 128, B*N < 2^31 - 128.  ws: ltgnn_node_init_ws_floats() floats.  Deterministic.
+ */
+int ltgnn_node_init_bwd_from_layer(int device, int64_t B, int32_t N, int32_t S, int32_t ds, int32_t D, int32_t K,
+                                   const float* hs, const int32_t* slot, const float* W, const float* G1,
+                                   const float* W1, const uint32_t* live_in, float gate_scale, float* dhs, float* dW,
+                                   float* dbias, float* ws, void* stream);
 
 /* ---- one GCN layer forward as ONE kernel (detector.py:198-201: conv -> relu -> dropout) ---------
  * Y = dropout(relu(A_hat (X W^T) + bias)) with the dense product on tcgen05 and never written to HBM: the window's

@@ -97,6 +97,93 @@ struct StoreEpilogue {
 };
 
 
+// Epilogue of the first GCN layer's input-gradient GEMM dX0 = G1 W1 when node init's backward is its only reader: of dX0
+// that backward needs just the gated column sums (-> d bias) and the gated sensor rows (-> dz [B, S, D]), so dX0 itself is
+// never stored.  Gate exactly as gate_extract_kernel<true> (node_init.cu): live bit ? v * gate_scale : 0, with element j
+// of a 32-column slice at bit 8 (j & 3) + (j >> 2) of the word [b][D/32][node].  Works in row form (lane = row): column
+// sums accumulate per lane pair (the first round of a shuffle tree per tile: 16 sums per 32 columns, so that two blocks
+// fit the kernel's 128 registers) over its rows, and are reduced once at the end (warp_sums: the rest of the tree; the
+// kernel then adds its warps in a fixed order into part[cta][D]) -- no atomics, the same bits on every run.
+struct GateSumEpilogue {
+    float* dz;             // [B, S, n]: gated gradient of the sensor rows
+    float* part;           // [CTAs, n]: column-sum partials
+    const uint32_t* live;  // [B, n/32, N]
+    const int32_t* slot;   // [N]: sensor slot of node i, or -1
+    float gate_scale;
+    int n;                 // D: 64 or 128 (one or two 32-column blocks per epilogue warp)
+    uint32_t N, S;
+    struct Cursor {        // per thread, carried over its tiles
+        uint32_t b, node;  // its row as (window, node), advanced without a division per tile
+        float sum[2][16];  // column sums of its blocks c_first, c_first + c_stride: column j + 16 (lane >> 4)
+    };
+    __device__ __forceinline__ void start(Cursor& cur, uint32_t row) const {
+        cur.b = row / N;
+        cur.node = row - cur.b * N;
+#pragma unroll
+        for (int k = 0; k < 2; ++k)
+#pragma unroll
+            for (int j = 0; j < 16; ++j) cur.sum[k][j] = 0.f;
+    }
+    __device__ __forceinline__ void advance(Cursor& cur, uint32_t rows) const {
+        cur.node += rows;
+        while (cur.node >= N) {
+            cur.node -= N;
+            ++cur.b;
+        }
+    }
+    template <class Pull>
+    __device__ __forceinline__ void operator()(Cursor& cur, bool valid, Pull&& pull, int lane, int c_first,
+                                               int c_stride) const {
+        const int sl = valid ? __ldg(slot + cur.node) : -1;
+        const bool up = lane & 16;
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const int c0 = c_first + k * c_stride;
+            if (c0 >= n) break;
+            float v[32];
+            pull(c0, v, 32);
+            const uint32_t w = valid ? __ldg(live + (static_cast<size_t>(cur.b) * (n >> 5) + (c0 >> 5)) * N + cur.node) : 0u;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = (w >> (8 * (j & 3) + (j >> 2))) & 1u ? v[j] * gate_scale : 0.f;
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const float send = up ? v[j] : v[j + 16], keep = up ? v[j + 16] : v[j];
+                cur.sum[k][j] += keep + __shfl_xor_sync(0xffffffffu, send, 16);
+            }
+            if (sl >= 0) {
+                float4* o = reinterpret_cast<float4*>(dz + (static_cast<size_t>(cur.b) * S + sl) * n + c0);
+#pragma unroll
+                for (int j = 0; j < 8; ++j) o[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+            }
+        }
+    }
+    // the warp's column sums: out[32 k + l] = column l of block k, summed over the 32 lanes.  Each round of the tree
+    // halves the columns a lane holds: it keeps the half selected by its lane bit and adds the partner's copy of it.
+    __device__ __forceinline__ void warp_sums(Cursor& cur, int lane, int c_first, int c_stride, float* out) const {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            if (c_first + k * c_stride >= n) break;
+            float* s = cur.sum[k];
+#pragma unroll
+            for (int o = 8; o >= 1; o >>= 1) {
+                const bool up = lane & o;
+#pragma unroll
+                for (int j = 0; j < o; ++j) {
+                    const float send = up ? s[j] : s[j + o], keep = up ? s[j + o] : s[j];
+                    s[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+                }
+            }
+            out[32 * k + lane] = s[0];
+        }
+    }
+};
+
+// dX = G W (W [K, N] row-major, N = ep.n) on linear.cu's tensor-memory row GEMM with a GateSumEpilogue; *parts: the number
+// of rows of ep.part written (one per CTA).  K a multiple of 32 up to 128; M < 2^31 - 128.
+int linear_gate_sums(int device, int64_t M, int K, const float* G, const float* W, const GateSumEpilogue& ep, int* parts,
+                     cudaStream_t stream);
+
+
 // ---- plain row-major operands, optionally two matrices stacked side by side to fill the 128 accumulator rows
 struct StackedRows {
     static constexpr bool kRowFast = false;

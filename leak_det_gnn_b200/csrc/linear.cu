@@ -25,7 +25,8 @@ namespace {
 //   warp  4     MMA       elected lane, 3xTF32
 //   warps 5-12  EPILOGUE  StoreEpilogue (bias / ReLU / gate, coalesced stores through the patch); two warps per TMEM
 //                         lane quadrant share the 32-column blocks -- a device-side timeline showed the epilogue, not
-//                         the loads or the MMAs, setting the pace (3 300 clocks per tile with 4 warps)
+//                         the loads or the MMAs, setting the pace (3 300 clocks per tile with 4 warps).  Or
+//                         GateSumEpilogue (node init's backward from the first layer's gradient: no product stored)
 // ---------------------------------------------------------------------------------------------------------
 namespace lt {
 using namespace ltgnn::ptx;
@@ -33,9 +34,11 @@ using namespace ltgnn::umma;
 constexpr int kLdWarps = 4, kMmaWarp = 4, kEpWarps = 8, kThreads = (kLdWarps + 1 + kEpWarps) * 32;  // 13 warps: 128 regs
 constexpr int kSlots = 4, kSlotCols = 64;
 
+template <class Epi>
 __global__ void __launch_bounds__(kThreads, 1)
-linear_ts_kernel(const float4* __restrict__ X, const StoreEpilogue epilogue, const float* __restrict__ W, int ldw,
+linear_ts_kernel(const float4* __restrict__ X, const Epi epilogue, const float* __restrict__ W, int ldw,
                  int transposed, uint32_t M, int K, int N, int depth) {
+    constexpr bool kSums = std::is_same<Epi, GateSumEpilogue>::value;
     extern __shared__ uint8_t smem_raw[];
     __shared__ uint64_t bar_full[kSlots], bar_empty[kSlots], bar_tfull[2], bar_tempty[2];
     __shared__ uint32_t tmem_base_s;
@@ -167,21 +170,42 @@ linear_ts_kernel(const float4* __restrict__ X, const StoreEpilogue epilogue, con
         }
     } else {
         const int q = warp & 3, half = (warp - kMmaWarp - 1) >> 2;  // TMEM lane quadrant = warp % 4
-        const patch::Patch pt(scratch + (kLdWarps * depth + warp - kMmaWarp - 1) * patch::kPatchBytes, lane);
+        uint8_t* const patch_mem = scratch + (kLdWarps * depth + warp - kMmaWarp - 1) * patch::kPatchBytes;
+        const patch::Patch pt(patch_mem, lane);
+        GateSumEpilogue::Cursor cur;
+        if constexpr (kSums) epilogue.start(cur, t_begin * 128 + q * 32 + lane);
         for (uint32_t t = 0; t < t_end - t_begin; ++t) {
             const uint32_t a = t & 1;
             mbar_wait_relaxed(&bar_tfull[a], (t >> 1) & 1);
             fence_after_sync();
             const uint32_t taddr = acc_base + a * 128 + (static_cast<uint32_t>(q * 32) << 16);
             const uint32_t row = (t_begin + t) * 128 + q * 32 + lane;
-            epilogue(row, M, 0, [&](int c0, float* v, int w) { if (w == 32) tmem_ld32(taddr + c0, v); else tmem_ld16(taddr + c0, v); }, pt, lane, 32 * half, 64);
+            auto pull = [&](int c0, float* v, int w) { if (w == 32) tmem_ld32(taddr + c0, v); else tmem_ld16(taddr + c0, v); };
+            if constexpr (kSums) {
+                epilogue(cur, row < M, pull, lane, 32 * half, 64);
+                epilogue.advance(cur, 128);
+            } else {
+                epilogue(row, M, 0, pull, pt, lane, 32 * half, 64);
+            }
             fence_before_sync();
             __syncwarp();
             if (lane == 0) mbar_arrive(&bar_tempty[a]);
         }
+        if constexpr (kSums) epilogue.warp_sums(cur, lane, 32 * half, 64, reinterpret_cast<float*>(patch_mem));
     }
     fence_before_sync();
     __syncthreads();
+    if constexpr (kSums) {
+        // this CTA's column sums: block c / 32 was handled by the four epilogue warps (one per lane quadrant) with
+        // half = block & 1, as entry block >> 1 of their lists; added in warp order
+        if (tid < N) {
+            const int blk = tid >> 5, half = blk & 1;
+            float s = 0.f;
+            for (int e = 4 * half; e < 4 * half + 4; ++e)
+                s += reinterpret_cast<const float*>(scratch + (kLdWarps * depth + e) * patch::kPatchBytes)[32 * (blk >> 1) + (tid & 31)];
+            epilogue.part[static_cast<size_t>(blockIdx.x) * N + tid] = s;
+        }
+    }
     if (warp == kMmaWarp) {
         fence_after_sync();
         tmem_dealloc(tmem_base, 512);
@@ -189,7 +213,39 @@ linear_ts_kernel(const float4* __restrict__ X, const StoreEpilogue epilogue, con
 }
 }  // namespace lt
 
+// the tensor-memory form for the streaming shapes: K % 32 == 0, K <= 128, N % 32 == 0, N <= 128, M < 2^31 - 128
+template <class Epi>
+int launch_ts(int device, int64_t M, int K, int N, const float* X, const float* W, int w_transposed, const Epi& ep,
+              int* grid_out, cudaStream_t stream) {
+    const DeviceInfo* di = device_info(device);
+    if (!di) return LTGNN_E_CUDA;
+    LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "linear: device is sm_%d%d, need sm_100", di->cc_major,
+                  di->cc_minor);
+    const size_t wbytes = 2ull * N * K * 4;
+    const int depth = 1024 + wbytes + (lt::kLdWarps * 8 + lt::kEpWarps) * patch::kPatchBytes <= static_cast<size_t>(di->smem_optin) ? 8 : 4;
+    const size_t smem = 1024 + wbytes + (lt::kLdWarps * depth + lt::kEpWarps) * patch::kPatchBytes;
+    LTGNN_REQUIRE(smem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "linear: %zu B of shared memory", smem);
+    LTGNN_USE_DEVICE(device);
+    LTGNN_CUDA_TRY(cudaFuncSetAttribute(lt::linear_ts_kernel<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(smem)));
+    const int64_t tiles = (M + 127) / 128;
+    const int grid = static_cast<int>(tiles < di->sm_count ? tiles : di->sm_count);
+    lt::linear_ts_kernel<Epi><<<grid, lt::kThreads, smem, stream>>>(reinterpret_cast<const float4*>(X), ep, W,
+                                                                    w_transposed ? N : K, w_transposed,
+                                                                    static_cast<uint32_t>(M), K, N, depth);
+    LTGNN_CUDA_TRY(cudaGetLastError());
+    if (grid_out) *grid_out = grid;
+    return LTGNN_OK;
+}
+
 }  // namespace
+
+int ltgnn::functors::linear_gate_sums(int device, int64_t M, int K, const float* G, const float* W,
+                                      const GateSumEpilogue& ep, int* parts, cudaStream_t stream) {
+    LTGNN_REQUIRE(M > 0 && K % 32 == 0 && K > 0 && K <= 128 && (ep.n == 64 || ep.n == 128) && M < (1ll << 31) - 128,
+                  LTGNN_E_SHAPE, "linear_gate_sums: M=%lld K=%d N=%d", static_cast<long long>(M), K, ep.n);
+    return launch_ts(device, M, K, ep.n, G, W, 1, ep, parts, stream);
+}
 
 extern "C" int ltgnn_linear(int device, int64_t M, int32_t K, int32_t N, const float* X, const float* W,
                             int w_transposed, const float* bias, int relu, const float* gate, float gate_scale, float* Y,
@@ -200,27 +256,9 @@ extern "C" int ltgnn_linear(int device, int64_t M, int32_t K, int32_t N, const f
     LTGNN_REQUIRE(aligned16(X) && aligned16(W) && aligned16(Y) && aligned16(gate), LTGNN_E_ALIGN,
                   "linear: 16-byte alignment required");
     StoreEpilogue ep{Y, bias, gate, gate_scale, N, relu};
-    if (K % 32 == 0 && K <= 128 && N % 32 == 0 && N <= 128 && M < (1ll << 31) - 128) {
+    if (K % 32 == 0 && K <= 128 && N % 32 == 0 && N <= 128 && M < (1ll << 31) - 128)
         // the streaming shapes of the GCN layers: A operand in tensor memory (see linear_ts_kernel)
-        const DeviceInfo* di = device_info(device);
-        if (!di) return LTGNN_E_CUDA;
-        LTGNN_REQUIRE(di->cc_major == 10, LTGNN_E_UNSUPPORTED, "linear: device is sm_%d%d, need sm_100", di->cc_major,
-                      di->cc_minor);
-        const size_t wbytes = 2ull * N * K * 4;
-        const int depth = 1024 + wbytes + (lt::kLdWarps * 8 + lt::kEpWarps) * patch::kPatchBytes <= static_cast<size_t>(di->smem_optin) ? 8 : 4;
-        const size_t smem = 1024 + wbytes + (lt::kLdWarps * depth + lt::kEpWarps) * patch::kPatchBytes;
-        LTGNN_REQUIRE(smem <= static_cast<size_t>(di->smem_optin), LTGNN_E_SHAPE, "linear: %zu B of shared memory", smem);
-        LTGNN_USE_DEVICE(device);
-        LTGNN_CUDA_TRY(cudaFuncSetAttribute(lt::linear_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            static_cast<int>(smem)));
-        const int64_t tiles = (M + 127) / 128;
-        const int grid = static_cast<int>(tiles < di->sm_count ? tiles : di->sm_count);
-        lt::linear_ts_kernel<<<grid, lt::kThreads, smem, static_cast<cudaStream_t>(stream_)>>>(
-            reinterpret_cast<const float4*>(X), ep, W, w_transposed ? N : K, w_transposed, static_cast<uint32_t>(M), K, N,
-            depth);
-        LTGNN_CUDA_TRY(cudaGetLastError());
-        return LTGNN_OK;
-    }
+        return launch_ts(device, M, K, N, X, W, w_transposed, ep, nullptr, static_cast<cudaStream_t>(stream_));
     RowLoader ld{reinterpret_cast<const float4*>(X), K / 4};
     rowgemm::BSpec bs{W, w_transposed ? N : K, w_transposed, 1};
     return rowgemm::launch(device, ld, ep, bs, M, K, N, static_cast<cudaStream_t>(stream_), "linear");

@@ -184,6 +184,9 @@ node_init_fwd_direct_kernel(const InitParams p, float* __restrict__ X0, uint32_t
 //     sensor rows of every window, written compactly to dz [B, S, D] (4 % of the bytes);
 // (2) d h_s = dz W[:, :ds] on the row-GEMM skeleton and dW = dz^T [h_s | 1] on the tensor-core weight-gradient
 //     skeleton, both over the B*S sensor rows only.
+// ltgnn_node_init_bwd_from_layer replaces (1) when dx0 is the first GCN layer's input gradient G1 W1: the tensor-core GEMM
+// that would form it does the gate, the column sums and the sensor-row extraction in its epilogue (GateSumEpilogue,
+// functors.cuh) and never stores dx0 -- one read of G1 instead of a write and a read of dx0.
 
 // colsum partial layout: part[cta][D]
 // kBits: the gate comes as 1 bit per element (`live`, layout [b][D/32][N]) instead of the float tensor X0
@@ -307,7 +310,8 @@ extern "C" int ltgnn_node_init_fwd(int device, int64_t B, int32_t N, int32_t S, 
     return LTGNN_OK;
 }
 
-// workspace: dz [B,S,D] | colsum partials [n_stream_ctas][D] | weight-gradient partials
+// workspace (ltgnn_node_init_bwd and ltgnn_node_init_bwd_from_layer):
+//   dz [B,S,D] | colsum partials [n_stream_ctas][D] | weight-gradient partials
 static int stream_ctas(const DeviceInfo* di) { return di->sm_count * 8; }
 static int dw_cols(int ds) { return (ds + 1 + 31) / 32 * 32; }  // [h_s | 1] padded to whole 32-column blocks
 
@@ -316,6 +320,23 @@ extern "C" int64_t ltgnn_node_init_ws_floats(int device, int64_t B, int32_t S, i
     if (!di) return -1;
     return B * S * D + static_cast<int64_t>(stream_ctas(di)) * D +
            static_cast<int64_t>(di->sm_count) * tgrad::kMo * dw_cols(ds);
+}
+
+// (2a) d h_s [M, ds] = dz [M, D] * W[:, :ds]   (W is [D, ds+1] row-major: a [K, N] operand with ld = ds+1)
+// (2b) dW [D, ds+1] = dz^T [h_s | 1]
+static int sensor_row_grads(int device, int64_t M, int32_t ds, int32_t D, const float* hs, const float* W, const float* dz,
+                            float* wpart, float* dhs, float* dW, cudaStream_t stream) {
+    functors::RowLoader ld{reinterpret_cast<const float4*>(dz), D / 4};
+    functors::StoreEpilogue ep{dhs, nullptr, nullptr, 1.f, ds, 0};
+    rowgemm::BSpec bs{W, ds + 1, 1, 1};
+    int rc = rowgemm::launch(device, ld, ep, bs, M, D, ds, stream, "node_init_bwd(dhs)");
+    if (rc) return rc;
+    functors::StackedRows g{reinterpret_cast<const float4*>(dz), nullptr, D / 4, 0};
+    functors::RowsThenOne x{reinterpret_cast<const float4*>(hs), ds / 4};
+    int grid = 0;
+    rc = tgrad::launch(device, g, x, wpart, M, dw_cols(ds), &grid, stream, "node_init_bwd(dW)");
+    if (rc) return rc;
+    return tgrad::gather(wpart, grid, dw_cols(ds), 0, D, 0, ds + 1, dW, ds + 1, 0, stream);
 }
 
 extern "C" int ltgnn_node_init_bwd(int device, int64_t B, int32_t N, int32_t S, int32_t ds, int32_t D, const float* hs,
@@ -361,20 +382,46 @@ extern "C" int ltgnn_node_init_bwd(int device, int64_t B, int32_t N, int32_t S, 
     LTGNN_CUDA_TRY(cudaGetLastError());
     rc = reduce_parts(cpart, D, dbias, static_cast<int>(g1), D, 0, stream);
     if (rc) return rc;
+    return sensor_row_grads(device, B * S, ds, D, hs, W, dz, wpart, dhs, dW, stream);
+}
 
-    // (2a) d h_s [B*S, ds] = dz [B*S, D] * W[:, :ds]   (W is [D, ds+1] row-major: a [K, N] operand with ld = ds+1)
-    const int64_t M = B * S;
-    functors::RowLoader ld{reinterpret_cast<const float4*>(dz), d4};
-    functors::StoreEpilogue ep{dhs, nullptr, nullptr, 1.f, ds, 0};
-    rowgemm::BSpec bs{W, ds + 1, 1, 1};
-    rc = rowgemm::launch(device, ld, ep, bs, M, D, ds, stream, "node_init_bwd(dhs)");
+extern "C" int ltgnn_node_init_bwd_from_layer(int device, int64_t B, int32_t N, int32_t S, int32_t ds, int32_t D,
+                                              int32_t K, const float* hs, const int32_t* slot, const float* W,
+                                              const float* G1, const float* W1, const uint32_t* live_in,
+                                              float gate_scale, float* dhs, float* dW, float* dbias, float* ws,
+                                              void* stream_) {
+    const DeviceInfo* di;
+    int rc = check_common(device, B, N, S, ds, D, &di, "node_init_bwd_from_layer");
     if (rc) return rc;
+    LTGNN_REQUIRE(D == 64 || D == 128, LTGNN_E_SHAPE, "node_init_bwd_from_layer: D=%d must be 64 or 128", D);
+    LTGNN_REQUIRE(ds % 32 == 0 && ds <= 224, LTGNN_E_SHAPE, "node_init_bwd_from_layer: ds=%d must be a multiple of 32",
+                  ds);
+    LTGNN_REQUIRE(K > 0 && K % 32 == 0 && K <= 128, LTGNN_E_SHAPE,
+                  "node_init_bwd_from_layer: K=%d must be a multiple of 32 up to 128", K);
+    LTGNN_REQUIRE(B * N < (1ll << 31) - 128, LTGNN_E_SHAPE, "node_init_bwd_from_layer: B*N=%lld rows",
+                  static_cast<long long>(B * N));
+    LTGNN_REQUIRE(hs && slot && W && G1 && W1 && live_in && dhs && dW && dbias && ws, LTGNN_E_ARG,
+                  "node_init_bwd_from_layer: null tensor");
+    LTGNN_REQUIRE(aligned16(G1) && aligned16(W1) && aligned16(ws) && aligned16(hs) && aligned16(dhs), LTGNN_E_ALIGN,
+                  "node_init_bwd_from_layer: 16-byte alignment required");
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    LTGNN_USE_DEVICE(device);
+    if (B == 0) {
+        LTGNN_CUDA_TRY(cudaMemsetAsync(dW, 0, sizeof(float) * D * (ds + 1), stream));
+        LTGNN_CUDA_TRY(cudaMemsetAsync(dbias, 0, sizeof(float) * D, stream));
+        return LTGNN_OK;
+    }
+    float* dz = ws;
+    float* cpart = dz + B * S * D;  // one row per GEMM CTA: at most sm_count <= stream_ctas rows
+    float* wpart = cpart + static_cast<int64_t>(stream_ctas(di)) * D;
 
-    // (2b) dW [D, ds+1] = dz^T [h_s | 1]
-    functors::StackedRows g{reinterpret_cast<const float4*>(dz), nullptr, d4, 0};
-    functors::RowsThenOne x{reinterpret_cast<const float4*>(hs), ds / 4};
-    int grid = 0;
-    rc = tgrad::launch(device, g, x, wpart, M, dw_cols(ds), &grid, stream, "node_init_bwd(dW)");
+    // (1) dX0 = G1 W1 on the tensor cores; the epilogue keeps only the gated column sums and sensor rows of it
+    functors::GateSumEpilogue ep{dz, cpart, live_in, slot, gate_scale, D, static_cast<uint32_t>(N),
+                                 static_cast<uint32_t>(S)};
+    int parts = 0;
+    rc = functors::linear_gate_sums(device, B * N, K, G1, W1, ep, &parts, stream);
     if (rc) return rc;
-    return tgrad::gather(wpart, grid, dw_cols(ds), 0, D, 0, ds + 1, dW, ds + 1, 0, stream);
+    rc = reduce_parts(cpart, D, dbias, parts, D, 0, stream);
+    if (rc) return rc;
+    return sensor_row_grads(device, B * S, ds, D, hs, W, dz, wpart, dhs, dW, stream);
 }

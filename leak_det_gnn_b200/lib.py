@@ -63,6 +63,9 @@ SIGNATURES = {
     "ltgnn_node_init_bwd": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p,
                                     c_void_p]),
+    "ltgnn_node_init_bwd_from_layer": (c_int, [c_int, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p,
+                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p,
+                                               c_void_p, c_void_p, c_void_p, c_void_p]),
     "ltgnn_gcn_layer_supported": (c_int, [c_void_p, c_int32, c_int32]),
     "ltgnn_gcn_layer_fwd": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int, c_float,
                                     c_uint64, c_void_p, c_void_p, c_void_p]),

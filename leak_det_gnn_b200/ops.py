@@ -415,6 +415,11 @@ def wgrad(g: torch.Tensor, x: torch.Tensor, out: Optional[torch.Tensor] = None) 
 # (ltgnn_linear + ltgnn_spmm_fused), which computes the same bits and stays as the cross-check.
 FUSED_LAYER = True
 
+# Node init's backward straight from the first layer's aggregated gradient (ltgnn_node_init_bwd_from_layer: the input
+# gradient of that layer is never stored) where the shapes allow; False = ltgnn_linear + ltgnn_node_init_bwd, which give
+# d h_s and d sensor_to_node.weight in the same bits and d sensor_to_node.bias up to summation order -- the cross-check.
+FUSED_NODE_INIT_BWD = True
+
 
 def gcn_layer_supported(graph: PipeGraph, x: torch.Tensor, weight: torch.Tensor) -> bool:
     return bool(_lib.load().ltgnn_gcn_layer_supported(graph.handle(x.device), int(weight.shape[1]), int(weight.shape[0])))
@@ -483,6 +488,39 @@ def node_init_bwd(h_s, slot, weight, dx0, x0, gate_scale, live=None):
                                      dx0.data_ptr(), x0.data_ptr(), None if live is None else live.data_ptr(),
                                      float(gate_scale), dhs.data_ptr(), dw.data_ptr(), db.data_ptr(), ws.data_ptr(),
                                      _stream(h_s)))
+    _inst.end(tok)
+    return dhs, dw, db
+
+
+def node_init_bwd_from_layer(h_s, slot, weight, gz, w1, live, gate_scale):
+    """node_init_bwd for dx0 = gz @ w1, the input gradient of the first GCN layer, without forming dx0 (see
+    ltgnn_node_init_bwd_from_layer): gz (B, N, K) the layer's aggregated output gradient, w1 (K, D) its weight,
+    ``live`` node_init_fwd's ``live_out`` (required).  Returns (dh_s, dW, dbias); dh_s and dW carry the bits of
+    ``node_init_bwd(h_s, slot, weight, gz @ w1, x0, gate_scale, live=live)``, dbias differs by summation order."""
+    for t, nm in ((h_s, "h_s"), (weight, "weight"), (gz, "gz"), (w1, "w1")):
+        _check_act(t, nm)
+    b, s, ds = h_s.shape
+    n, k = gz.shape[1], gz.shape[2]
+    d = w1.shape[1]
+    if d not in (64, 128) or ds % 32 or k % 32 or k > 128:
+        raise ValueError(f"node_init_bwd_from_layer: node width {d} / sensor width {ds} / layer width {k} not built (64 or "
+                         "128 / a multiple of 32 / a multiple of 32 up to 128); the sm_100a kernels have no library fallback")
+    if tuple(gz.shape) != (b, n, k) or tuple(w1.shape) != (k, d) or tuple(weight.shape) != (d, ds + 1):
+        raise ValueError(f"gz {tuple(gz.shape)} / w1 {tuple(w1.shape)} / weight {tuple(weight.shape)} do not fit h_s "
+                         f"{tuple(h_s.shape)}")
+    if live is None or live.dtype != torch.int32 or tuple(live.shape) != (b, d // 32, n):
+        raise ValueError(f"live must be int32 of shape {(b, d // 32, n)}")
+    L = _lib.load()
+    dev = _dev_index(h_s)
+    dhs = torch.empty_like(h_s)
+    dw = torch.empty_like(weight)
+    db = torch.empty(d, device=h_s.device, dtype=torch.float32)
+    ws = torch.empty(int(L.ltgnn_node_init_ws_floats(dev, b, s, ds, d)), device=h_s.device, dtype=torch.float32)
+    tok = _inst.begin("node_init_bwd")
+    _lib.check(L.ltgnn_node_init_bwd_from_layer(dev, b, n, s, ds, d, k, h_s.data_ptr(), slot.data_ptr(),
+                                                weight.data_ptr(), gz.data_ptr(), w1.data_ptr(), live.data_ptr(),
+                                                float(gate_scale), dhs.data_ptr(), dw.data_ptr(), db.data_ptr(),
+                                                ws.data_ptr(), _stream(h_s)))
     _inst.end(tok)
     return dhs, dw, db
 
@@ -1275,6 +1313,11 @@ class _GnnBody(torch.autograd.Function):
                 grads[2 * l] = wgrad(gz, x_in)
             if not below[l]:
                 break
+            if l == 0 and FUSED_NODE_INIT_BWD and ctx.lives[0] is not None and w0.shape[0] in (64, 128) \
+                    and h_s.shape[2] % 32 == 0 and w.shape[0] % 32 == 0 and w.shape[0] <= 128:
+                # node init reads only the gated column sums and sensor rows of this layer's input gradient
+                dhs, dw0, db0 = node_init_bwd_from_layer(h_s, slot, w0, gz, w.contiguous(), ctx.lives[0], scale)
+                return (dhs, None, None, None, None, dvals, None, dw0, db0, *grads)
             g = _linear_any(gz, w, transposed=True)
             del gz
         dhs = dw0 = db0 = None
